@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Gibbs sweep path (BASELINE.json metric: "Gibbs sweeps/sec & ESS/sec, nSubj=1M nItem=100").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One "step" = one Gibbs sweep of GibbsRtIrtQuantile (the LatentQr sampler, q = 0.85, F = 3 covariates) over the
@@ -13,11 +13,9 @@ exchange over NVLink peer memory fused into the global draw kernel; ERIRT_EXCHAN
 the total work is fixed: "scaling": "strong".
 
 Keys of the JSON line (DESIGN.md "Measurement"):
-  value         sweeps/s, data resident in HBM, CUDA events on the library's stream, max over ranks; the timed region starts
-                right after one throw-away sweep whose exchange lines the GPUs up.  K sweeps last only milliseconds, so when
-                K x ms_per_step < 0.5 s the region is the K sweeps plus the long run below (`timed_sweeps` sweeps in total);
-                `k_steps` keeps the figure of the K sweeps alone
-  long_run      the continuation of the same chain over >= 0.5 s of sweeps (clocks are sampled over both)
+  value         sweeps/s over exactly K = --steps sweeps, data resident in HBM, CUDA events on the library's stream, max over
+                ranks; the timed region starts right after one throw-away sweep whose exchange lines the GPUs up
+  long_run      the continuation of the same chain over >= 0.5 s of sweeps, timed on its own (clocks are sampled over both)
   e2e           sweeps/s through the public C-ABI calls with HOST (pinned) buffers: erirt_create + erirt_set_data
                 (H2D + ingest) + erirt_set_state + K sweeps + erirt_get_trace/erirt_get_moments (D2H), all timed
   roofline      person-sweep kernel: algorithmic HBM bytes per launch / its mean CUDA-event duration, against the
@@ -30,6 +28,8 @@ Keys of the JSON line (DESIGN.md "Measurement"):
   cpu_baseline  the CPU oracle (a C restatement of the reference; Julia is not installed) on one host core, on a
                 bounded sample of the persons, extrapolated linearly in nSubj
 --impl reference times that same CPU restatement with all host threads (OpenMP over persons/items).
+--dump-outputs DIR writes what the K timed sweeps computed (see dump_outputs) as DIR/<name>.npy; the inputs depend only on
+the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -44,6 +44,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree, which may be read-only
 
 N_SUBJ, N_ITEM, N_FEAT, Q_RT = 1_000_000, 100, 3, 0.85
 N_BLOCKS = 8  # data is generated in 8 seeded person blocks so that every GPU count sees the same data set
@@ -265,6 +266,38 @@ def item_struct_traces(eng, first, n, qw):
         cols.append(eng.get_trace("rt", N, 2 * J)[first:first + n, :, 0])
     cols.append(eng.get_trace("qr", 0, qw)[first:first + n, :, 0])
     return cols
+
+
+DUMP_PERSONS = 1 << 18  # person-level outputs are written for this many persons (fixed sample drawn with SEED)
+
+
+def dump_outputs(eng, out_dir, last, world, rank):
+    """What a caller of the timed path receives after its last sweep (api.sample's MCMC.Para and Post), as out_dir/<name>.npy in
+    float64: theta and zeta (erirt_get_state), the running mean and SD of theta, zeta and nu (erirt_get_moments), and a, b, lambda,
+    sigma2, beta, Sigma_p and logLike from trace row `last`.  The eight person-level arrays are restricted to the same seeded sample
+    of DUMP_PERSONS persons (ascending ids), so that everything stays near 17 MB.  The item statistics are summed with atomics, so
+    two runs of one build agree only up to that rounding as the chain carries it forward (on a B200 in f32: logLike of sweep 1 within
+    1e-10 relative, person draws within 0.1 after 26 sweeps).  Collective when world > 1."""
+    from erirt_b200 import distributed as D
+    J = N_ITEM
+    person = {"theta": eng.get_state("theta"), "zeta": eng.get_state("zeta")}
+    for f in ("theta", "zeta", "nu"):
+        person[f + "_mean"], person[f + "_sd"] = eng.get_moments(f)
+    if world > 1:
+        person = {k: D.gather_person_vector(v, N_SUBJ) for k, v in person.items()}
+    if rank != 0:
+        return
+    idx = np.sort(np.random.default_rng(SEED).choice(N_SUBJ, DUMP_PERSONS, replace=False))
+    out = {k: v[idx] for k, v in person.items()}
+    ra = eng.get_trace("ra", eng.N, 2 * J)[last, :, 0]
+    rt = eng.get_trace("rt", eng.N, 2 * J)[last, :, 0]
+    qr = eng.get_trace("qr", 0, N_FEAT + 6)[last, :, 0]
+    out.update({"a": ra[:J], "b": ra[J:], "lambda": rt[:J], "sigma2": rt[J:], "beta": qr[:N_FEAT + 2],
+                "Sigma_p": qr[N_FEAT + 2:].reshape(2, 2, order="F"), "logLike": eng.get_trace("logLike")[last, :, 0]})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(v, dtype=np.float64))
+    log(f"outputs of sweep {last + 1} written to {out_dir}")
 
 
 def cpu_oracle_rate(tp, n_sample, n_sweeps, nthreads, warm=1):
@@ -506,7 +539,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the sub-records (f64, crossqr, configs, c4_chains, ess)")
     ap.add_argument("--short", action="store_true", help="profiling run: timed sweeps only, no e2e / cpu / roofline / sub-record passes")
     ap.add_argument("--sub", default=None, choices=["f64", "crossqr", "configs"], help="(internal) run one sub-record and print it")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed sweeps computed (state, moments, last trace row) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none")
     if args.impl == "reference":
         return run_reference(args)
     if args.sub:
@@ -588,6 +625,8 @@ def main():
     eng.sample(K)
     ms = max_over_ranks(eng.stats()["last_sample_ms"])
     done = W + 1 + K
+    if args.dump_outputs:
+        dump_outputs(eng, args.dump_outputs, done - 1, world, rank)
     long_run = None
     if not args.short:
         n_long = int(max(1, min(cap - done - 8, max(K, math.ceil(LONG_RUN_SECONDS * 1e3 / (ms / K))))))
@@ -765,20 +804,11 @@ def main():
             cpu = {"value": None, "unit": UNIT, "cores": 1, "kind": "port", "sample": f"failed: {ex}"}
 
     if rank == 0:
-        # K sweeps of this workload last well under a second (13 ms at N = 1, 2 ms at N = 8 for the driver's K = 20): the headline is
-        # taken over the K sweeps PLUS the long run that follows them in the same chain (>= 0.5 s of device time in total), the
-        # K-sweep figure stays in the line as `k_steps`
-        timed_sweeps, timed_ms = K, ms
-        if long_run is not None and ms < LONG_RUN_SECONDS * 1e3:
-            timed_sweeps, timed_ms = K + long_run["sweeps"], ms + long_run["ms_per_step"] * long_run["sweeps"]
-        k_steps = {"sweeps": K, "value": value, "ms_per_step": ms / K}
-        value = timed_sweeps / (timed_ms / 1e3)
-        launches = 2 * timed_sweeps
         line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
-                "ms_per_step": timed_ms / timed_sweeps, "timed_sweeps": timed_sweeps, "k_steps": k_steps,
+                "ms_per_step": ms / K, "timed_sweeps": K,
                 "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
                 "dtype": args.dtype, "data": "synthetic", "config": make_config(world),
-                "clocks": clk, "gpu_launches": launches, "long_run": long_run, "e2e": e2e, "e2e_device_generated_data": e2e_gen,
+                "clocks": clk, "gpu_launches": 2 * K, "long_run": long_run, "e2e": e2e, "e2e_device_generated_data": e2e_gen,
                 "roofline": roofline, "cpu_baseline": cpu, "ess": ess,
                 "sharding_check": {"loglike_sweeps_1_5_" + args.dtype: ll_first, "loglike_sweeps_1_5_f64": ll64,
                                    "note": "the same chain (seed, data, initial state) at every GPU count: Philox counters use global person ids, "
