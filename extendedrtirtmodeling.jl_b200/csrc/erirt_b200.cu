@@ -364,21 +364,17 @@ struct erirt_handle {
   // one-shot peer exchange (NVLink peer memory, CUDA IPC between the per-GPU processes)
   double* xbuf = nullptr;             // this GPU's exchange buffer
   double** dPeerBufs = nullptr;       // device array [world] of every GPU's exchange buffer
-  std::vector<void*> peer_opened;     // mappings opened with cudaIpcOpenMemHandle
   uint32_t* dXseq = nullptr;
   int xstride = 0;
   bool peer_ready = false;
-  int peer_cache_slot = -1;           // >= 0: xbuf / dPeerBufs / dXseq / the peer mappings belong to g_peer_cache[slot], not to the handle
+  int peer_cache_slot = -1;           // the g_peer_cache entry that owns xbuf / dPeerBufs / dXseq and the peer mappings (-1: none yet)
   // graph
   cudaGraphExec_t graph_exec = nullptr;
-  cudaGraphExec_t graph_multi = nullptr;  // ERIRT_GRAPH_SWEEPS sweeps in one graph (experimental)
-  int graph_multi_sweeps = 0;
+  cudaGraphExec_t graph_multi = nullptr;  // GRAPH_SWEEPS sweeps in one graph
 };
 
 static int launch_person(erirt_handle* h, int stage);
 static int launch_global(erirt_handle* h, int stage);
-static bool pdl_enabled();
-static bool global_rehearsal_enabled();
 static int finalize_constants(erirt_handle* h);
 static int pick_device(int32_t device);
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -431,7 +427,6 @@ static const void* person_kernel_ptr(int tpp) {
     default: return (const void*)person_sweep_kernel<R, 8, FAM>;
   }
 }
-// fam 0: the specialised kernel of the one-launch models; fam 1: Cross family and the evaluation stage
 template <int MODEL>
 static const void* person_fast_kernel_ptr_m(int tpp) {
   switch (tpp) {
@@ -450,8 +445,12 @@ static const void* person_fast_kernel_ptr(int tpp, int model) {
     default: return person_fast_kernel_ptr_m<M_LATENTQR>(tpp);
   }
 }
-static const void* person_kernel_for(const erirt_handle* h, int fam) {
-  if (fam == 0) return h->cfg.dtype == ERIRT_F32 ? person_fast_kernel_ptr(h->tpp, h->cfg.model) : person_kernel_ptr<double, 0>(h->tpp);
+// Stage 0 is the sweep of the one-launch models, stages 1 and 2 the two halves of a Cross-family sweep, stage 3 the evaluation.
+// Stage 0 in f32 runs person_sweep_fast_kernel (plan h->S); every other stage runs the generic kernel (plan h->S_gen).
+static bool runs_fast_kernel(const erirt_handle* h, int stage) { return stage == 0 && h->cfg.dtype == ERIRT_F32; }
+static const void* person_kernel_for(const erirt_handle* h, int stage) {
+  if (runs_fast_kernel(h, stage)) return person_fast_kernel_ptr(h->tpp, h->cfg.model);
+  if (stage == 0) return person_kernel_ptr<double, 0>(h->tpp);  // Cross-family and evaluation code compiled out
   return h->cfg.dtype == ERIRT_F32 ? person_kernel_ptr<float, 1>(h->tpp_gen) : person_kernel_ptr<double, 1>(h->tpp_gen);
 }
 
@@ -481,8 +480,8 @@ extern "C" const char* erirt_last_error(void) { return g_err.c_str(); }
 // Exchange buffers and their CUDA IPC mappings are kept for the next handle of the process (same device, rank, world and slot size):
 // opening the seven peer mappings of an 8-GPU chain costs ~40 ms per erirt_create + attach, more than 100 sweeps of the benchmark.
 // The stamps are sequence numbers that simply keep counting (xseq is cached with the buffer), so a reused buffer needs no reset;
-// every rank of a sharded program makes the same calls, hence the same reuse decisions.  ERIRT_PEER_CACHE=0 disables the cache;
-// erirt_trim_pool releases the entries that are not in use.
+// every rank of a sharded program makes the same calls, hence the same reuse decisions.  erirt_trim_pool releases the entries
+// that are not in use.
 struct PeerCacheEntry {
   int device = -1, world = 0, rank = -1, xstride = 0;
   double* xbuf = nullptr;
@@ -494,10 +493,6 @@ struct PeerCacheEntry {
 };
 static std::mutex g_peer_mu;
 static std::vector<PeerCacheEntry> g_peer_cache;
-static bool peer_cache_enabled() {
-  const char* e = getenv("ERIRT_PEER_CACHE");
-  return !(e && atoi(e) == 0);
-}
 static void peer_cache_release_entry(PeerCacheEntry& c) {
   for (void* p : c.opened) cudaIpcCloseMemHandle(p);
   c.opened.clear();
@@ -518,11 +513,6 @@ static int free_handle(erirt_handle* h) {
     if (h->stream) cudaStreamSynchronize(h->stream);
     std::lock_guard<std::mutex> lk(g_peer_mu);
     g_peer_cache[h->peer_cache_slot].in_use = false;
-  } else {
-    for (void* p : h->peer_opened) cudaIpcCloseMemHandle(p);
-    if (h->xbuf) cudaFree(h->xbuf);
-    if (h->dPeerBufs) cudaFree(h->dPeerBufs);
-    if (h->dXseq) cudaFree(h->dXseq);
   }
   if (h->arena && h->stream) {  // all device buffers of the handle: back to the pool
     cudaFreeAsync(h->arena, h->stream);
@@ -586,24 +576,19 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
   const bool is_cross = cfg->model == ERIRT_RTIRT_CROSS || cfg->model == ERIRT_RTIRT_CROSSQR;
   const bool is_cqr = cfg->model == ERIRT_RTIRT_CROSSQR;
   const bool fast_engine = h->rsz == 4 && !is_cross;
-  const char* env_tpp = getenv("ERIRT_TPP");
   const int n_groups = h->L.Jp / 4;
   auto choose = [&](bool fast, int& tpp, SmemPlan& S) -> const char* {
-    if (env_tpp) tpp = atoi(env_tpp);
-    else {
-      for (tpp = 1; tpp < 8; tpp *= 2) {
-        SmemPlan s = make_smem_plan(h->L, tpp, h->rsz, has_rt, is_cqr, is_cross, fast);
-        if (s.total <= 75 * 1024 && n_groups <= 16 * tpp) break;
-      }
-      // Float64 (the generic kernel): a cell costs thousands of instructions, so a problem with fewer tiles than two per SM is
-      // spread over more, smaller tiles (measured at BASELINE configs 1-3: 2x the sweeps/s from TPP 1 -> 8; the f32 kernels, whose
-      // sweep is bound by the per-tile latency chain, gain nothing: profiles/r02_summary.md)
-      // (for a large problem TPP = 8 was 7 % faster while the cell loop was one divergent exact draw per cell; with the branch-free
-      // attempt 0 the 168-register TPP = 4 instantiation wins, 4.0 against 5.3 ms per sweep at 1M x 100)
-      if (!fast && h->rsz == 8)
-        while (tpp < 8 && (int64_t)align_up((size_t)cfg->n_subj, 128) / (CTA_THREADS / tpp) < 2 * (int64_t)h->sm_count) tpp *= 2;
+    for (tpp = 1; tpp < 8; tpp *= 2) {
+      SmemPlan s = make_smem_plan(h->L, tpp, h->rsz, has_rt, is_cqr, is_cross, fast);
+      if (s.total <= 75 * 1024 && n_groups <= 16 * tpp) break;
     }
-    if (tpp != 1 && tpp != 2 && tpp != 4 && tpp != 8) return "ERIRT_TPP must be 1, 2, 4 or 8";
+    // Float64 (the generic kernel): a cell costs thousands of instructions, so a problem with fewer tiles than two per SM is
+    // spread over more, smaller tiles (measured at BASELINE configs 1-3: 2x the sweeps/s from TPP 1 -> 8; the f32 kernels, whose
+    // sweep is bound by the per-tile latency chain, gain nothing: profiles/r02_summary.md)
+    // (for a large problem TPP = 8 was 7 % faster while the cell loop was one divergent exact draw per cell; with the branch-free
+    // attempt 0 the 168-register TPP = 4 instantiation wins, 4.0 against 5.3 ms per sweep at 1M x 100)
+    if (!fast && h->rsz == 8)
+      while (tpp < 8 && (int64_t)align_up((size_t)cfg->n_subj, 128) / (CTA_THREADS / tpp) < 2 * (int64_t)h->sm_count) tpp *= 2;
     if (n_groups > 16 * tpp) return "too many items for this TPP (at most 64*TPP - 4)";
     S = make_smem_plan(h->L, tpp, h->rsz, has_rt, is_cqr, is_cross, fast);
     if (S.total > 227 * 1024) return "n_item needs more shared memory per CTA than an SM has";
@@ -616,7 +601,7 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
     h->tpp_gen = h->tpp;
     h->S_gen = h->S;
   }
-  h->n_pad = (int64_t)align_up((size_t)cfg->n_subj, CTA_THREADS > 128 ? CTA_THREADS : 128);
+  h->n_pad = (int64_t)align_up((size_t)cfg->n_subj, 128);
   h->cap = cfg->n_iter * cfg->n_chain;
   h->qw = qr_small_width(cfg->model, cfg->n_item, cfg->n_feat);
 
@@ -705,13 +690,11 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
   ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kfn, CTA_THREADS, h->S.total);
   if (ce != cudaSuccess || occ < 1) { free_handle(h); return fail(ERIRT_E_CUDA, "person kernel does not fit on an SM: %s", cudaGetErrorString(ce)); }
   const int n_tiles = (int)(h->n_pad / h->S.P);
-  const char* env_occ = getenv("ERIRT_CTAS_PER_SM");
-  if (env_occ && atoi(env_occ) > 0 && atoi(env_occ) < occ) occ = atoi(env_occ);
   h->grid = std::min(n_tiles, h->sm_count * occ);
   // A full grid leaves ONE slot free: with dynamic tile dealing no person CTA exits before the last round, so the global kernel of the
   // sweep (256 threads, 80 registers, ~55 KB) could otherwise not become resident early enough to finish its rehearsal pass
   // (global.cuh) before the person kernel ends; the slot costs 1/444 of the person kernel's throughput
-  if (global_rehearsal_enabled() && h->grid == h->sm_count * occ && h->grid > 1) h->grid -= 1;
+  if (h->grid == h->sm_count * occ && h->grid > 1) h->grid -= 1;
   // test hook: ERIRT_MAX_GRID caps the persistent grid, so that a small problem gives every CTA many tiles (the cross-tile register
   // accumulators and their 16-tile fold are otherwise reached only at benchmark size); results do not depend on the grid
   const char* env_grid = getenv("ERIRT_MAX_GRID");
@@ -1107,8 +1090,7 @@ static PersonArgs<R> make_person_args(erirt_handle* h, int stage) {
   A.n_local = h->cfg.n_subj;
   A.n_pad = h->n_pad;
   A.person_offset = (uint32_t)h->cfg.subj_offset;
-  const bool generic = stage != 0 || h->cfg.dtype != ERIRT_F32;  // which kernel launch_person() picks
-  A.S = generic ? h->S_gen : h->S;
+  A.S = runs_fast_kernel(h, stage) ? h->S : h->S_gen;
   A.n_tiles = (int)(h->n_pad / A.S.P);
   A.L = h->L;
   A.model = h->cfg.model;
@@ -1132,9 +1114,9 @@ static GlobalArgs make_global_args(erirt_handle* h, int stage) {
     // The rehearsal pays when the person launch in front of this kernel is long enough to hide it (about 20 us) and big enough to
     // have flushed the instruction caches: more than one tile per CTA.  Behind a one-round launch (the small problems) it would only
     // delay the real pass.
-    const bool generic = stage != 0 || h->cfg.dtype != ERIRT_F32;
-    const int64_t tiles = h->n_pad / (generic ? h->S_gen.P : h->S.P);
-    A.rehearse = (global_rehearsal_enabled() && tiles > (generic ? h->grid_gen : h->grid)) ? 1 : 0;
+    const bool fast = runs_fast_kernel(h, stage);
+    const int64_t tiles = h->n_pad / (fast ? h->S.P : h->S_gen.P);
+    A.rehearse = tiles > (fast ? h->grid : h->grid_gen) ? 1 : 0;
   }
   A.tile_ctr = h->dTileCtr;
   A.sweep_ctr = h->dSweep;
@@ -1158,7 +1140,7 @@ static GlobalArgs make_global_args(erirt_handle* h, int stage) {
   A.onepl = h->cfg.itemtype_1pl;
   A.cov2one = h->cfg.cov2one;
   A.compat = h->cfg.compat;
-  A.kz_from_stats = (stage == 0 && h->cfg.dtype == ERIRT_F32) ? 1 : 0;  // stage 0 in f32 == person_sweep_fast_kernel (launch_person)
+  A.kz_from_stats = runs_fast_kernel(h, stage) ? 1 : 0;
   const double q = h->cfg.q_rt;
   A.k1 = (1.0 - 2.0 * q) / (q * (1.0 - q));
   A.k2 = 2.0 / (q * (1.0 - q));
@@ -1173,16 +1155,7 @@ static GlobalArgs make_global_args(erirt_handle* h, int stage) {
 
 // Every kernel of the sweep chain is launched with programmatic stream serialization (griddep_wait / griddep_launch in the
 // kernels, layout.cuh): a kernel's CTAs may become resident, and run what does not depend on its predecessor, while the predecessor
-// is still running.  ERIRT_PDL=0 switches the attribute off (plain stream order; the device-side calls are then no-ops).
-static bool pdl_enabled() {
-  static const bool on = [] { const char* e = getenv("ERIRT_PDL"); return !(e && atoi(e) == 0); }();
-  return on;
-}
-// ERIRT_G_REHEARSE=0 switches the instruction-cache rehearsal of the global kernel off (global.cuh); it needs the early residency PDL gives
-static bool global_rehearsal_enabled() {
-  static const bool on = [] { const char* e = getenv("ERIRT_G_REHEARSE"); return pdl_enabled() && !(e && atoi(e) == 0); }();
-  return on;
-}
+// is still running.
 static cudaError_t launch_chain_kernel(const void* kfn, dim3 grid, dim3 block, void** args, size_t smem, cudaStream_t stream) {
   cudaLaunchConfig_t lc{};
   lc.gridDim = grid;
@@ -1193,12 +1166,12 @@ static cudaError_t launch_chain_kernel(const void* kfn, dim3 grid, dim3 block, v
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   lc.attrs = at;
-  lc.numAttrs = pdl_enabled() ? 1 : 0;
+  lc.numAttrs = 1;
   return cudaLaunchKernelExC(&lc, kfn, args);
 }
 
 static int launch_person(erirt_handle* h, int stage) {
-  const void* kfn = person_kernel_for(h, stage == 0 ? 0 : 1);
+  const void* kfn = person_kernel_for(h, stage);
   if (h->cfg.dtype == ERIRT_F32) {
     PersonArgs<float> A = make_person_args<float>(h, stage);
     void* args[] = {&A};
@@ -1240,6 +1213,8 @@ static int enqueue_step(erirt_handle* h, bool prologue) {
   return launch_global(h, cross ? 2 : 0);
 }
 
+constexpr int GRAPH_SWEEPS = 16;  // sweeps of the long CUDA graph of erirt_sample
+
 extern "C" int erirt_sample(erirt_handle* h, int64_t n_sweeps) {
   if (!h) return fail(ERIRT_E_ARG, "null handle");
   if (!h->data_set) return fail(ERIRT_E_STATE, "erirt_set_data has not been called");
@@ -1266,11 +1241,10 @@ extern "C" int erirt_sample(erirt_handle* h, int64_t n_sweeps) {
     }
   }
   const bool graphs = h->cfg.use_graph && !h->cfg.time_kernels && n_sweeps > 0;
-  // The sweeps are replayed from two CUDA graphs: one of `gs` sweeps (ERIRT_GRAPH_SWEEPS, default 16) and one of a single sweep for the
-  // remainder.  Inside a graph the kernels overlap their neighbours through the programmatic-dependent-launch edges; a graph boundary
-  // serialises, so the long graph also keeps the launch-bound small problems busy.  Both are captured on the first call, before the
-  // timed region of this call starts.
-  int gs = 1;
+  // The sweeps are replayed from two CUDA graphs: one of GRAPH_SWEEPS sweeps and one of a single sweep for the remainder.  Inside a
+  // graph the kernels overlap their neighbours through the programmatic-dependent-launch edges; a graph boundary serialises, so the
+  // long graph also keeps the launch-bound small problems busy.  Both are captured on the first call, before the timed region of this
+  // call starts.
   if (graphs) {
     auto capture = [&](int sweeps, cudaGraphExec_t* exec) -> int {
       cudaGraph_t graph;
@@ -1286,21 +1260,12 @@ extern "C" int erirt_sample(erirt_handle* h, int64_t n_sweeps) {
       return 0;
     };
     if (!h->graph_exec && (rc = capture(1, &h->graph_exec))) return rc;
-    const char* env_gs = getenv("ERIRT_GRAPH_SWEEPS");
-    gs = env_gs ? std::max(1, std::min(64, atoi(env_gs))) : 16;
-    if (gs > 1) {
-      if (h->graph_multi && h->graph_multi_sweeps != gs) { cudaGraphExecDestroy(h->graph_multi); h->graph_multi = nullptr; }
-      if (!h->graph_multi) {
-        if ((rc = capture(gs, &h->graph_multi))) return rc;
-        h->graph_multi_sweeps = gs;
-      }
-    }
+    if (!h->graph_multi && (rc = capture(GRAPH_SWEEPS, &h->graph_multi))) return rc;
   }
   CU(cudaEventRecord(h->ev0, h->stream));
   if (graphs) {
     int64_t left = n_sweeps;
-    if (gs > 1)
-      for (; left >= gs; left -= gs) CU(cudaGraphLaunch(h->graph_multi, h->stream));
+    for (; left >= GRAPH_SWEEPS; left -= GRAPH_SWEEPS) CU(cudaGraphLaunch(h->graph_multi, h->stream));
     for (; left > 0; --left) CU(cudaGraphLaunch(h->graph_exec, h->stream));
   } else {
     for (int64_t t = 0; t < n_sweeps; ++t) {
@@ -1731,35 +1696,41 @@ extern "C" int erirt_peer_export(erirt_handle* h, void* ipc_handle64) {
   CU(cudaSetDevice(h->cfg.device));
   if (!h->xbuf) {
     h->xstride = (int)align_up((size_t)std::max(h->L.s_count, h->c_count), 16);  // the statistics per sweep, the ingest constants once
-    if (peer_cache_enabled()) {
-      std::lock_guard<std::mutex> lk(g_peer_mu);
-      for (size_t t = 0; t < g_peer_cache.size(); ++t) {
-        PeerCacheEntry& c = g_peer_cache[t];
-        if (!c.in_use && c.device == h->cfg.device && c.world == h->world && c.rank == h->rank && c.xstride == h->xstride && c.xbuf) {
-          c.in_use = true;
-          h->peer_cache_slot = (int)t;
-          h->xbuf = c.xbuf; h->dPeerBufs = c.dPeerBufs; h->dXseq = c.dXseq;
-          break;
-        }
+    std::lock_guard<std::mutex> lk(g_peer_mu);
+    for (size_t t = 0; t < g_peer_cache.size(); ++t) {
+      PeerCacheEntry& c = g_peer_cache[t];
+      if (!c.in_use && c.device == h->cfg.device && c.world == h->world && c.rank == h->rank && c.xstride == h->xstride && c.xbuf) {
+        c.in_use = true;
+        h->peer_cache_slot = (int)t;
+        h->xbuf = c.xbuf; h->dPeerBufs = c.dPeerBufs; h->dXseq = c.dXseq;
+        break;
       }
     }
   }
   if (!h->xbuf) {
     const size_t bytes = (size_t)2 * h->world * h->xstride * 16 + 256;  // [2 parities][world][xstride] 16-byte packets (global.cuh)
-    CU(cudaMalloc((void**)&h->xbuf, bytes));
-    CU(cudaMemset(h->xbuf, 0, bytes));
-    CU(cudaMalloc((void**)&h->dPeerBufs, h->world * sizeof(double*)));
-    CU(cudaMalloc((void**)&h->dXseq, sizeof(uint32_t)));
-    CU(cudaMemset(h->dXseq, 0, sizeof(uint32_t)));
-    CU(cudaDeviceSynchronize());
-    if (peer_cache_enabled()) {
-      std::lock_guard<std::mutex> lk(g_peer_mu);
-      PeerCacheEntry c;
-      c.device = h->cfg.device; c.world = h->world; c.rank = h->rank; c.xstride = h->xstride;
-      c.xbuf = h->xbuf; c.dPeerBufs = h->dPeerBufs; c.dXseq = h->dXseq; c.in_use = true;
-      g_peer_cache.push_back(c);
-      h->peer_cache_slot = (int)g_peer_cache.size() - 1;
+    auto alloc = [&]() -> int {
+      CU(cudaMalloc((void**)&h->xbuf, bytes));
+      CU(cudaMemset(h->xbuf, 0, bytes));
+      CU(cudaMalloc((void**)&h->dPeerBufs, h->world * sizeof(double*)));
+      CU(cudaMalloc((void**)&h->dXseq, sizeof(uint32_t)));
+      CU(cudaMemset(h->dXseq, 0, sizeof(uint32_t)));
+      CU(cudaDeviceSynchronize());
+      return 0;
+    };
+    if (int rc = alloc()) {  // the buffers belong to no cache entry yet: free what was allocated
+      if (h->xbuf) cudaFree(h->xbuf);
+      if (h->dPeerBufs) cudaFree(h->dPeerBufs);
+      if (h->dXseq) cudaFree(h->dXseq);
+      h->xbuf = nullptr; h->dPeerBufs = nullptr; h->dXseq = nullptr;
+      return rc;
     }
+    std::lock_guard<std::mutex> lk(g_peer_mu);
+    PeerCacheEntry c;
+    c.device = h->cfg.device; c.world = h->world; c.rank = h->rank; c.xstride = h->xstride;
+    c.xbuf = h->xbuf; c.dPeerBufs = h->dPeerBufs; c.dXseq = h->dXseq; c.in_use = true;
+    g_peer_cache.push_back(c);
+    h->peer_cache_slot = (int)g_peer_cache.size() - 1;
   }
   cudaIpcMemHandle_t hd;
   CU(cudaIpcGetMemHandle(&hd, h->xbuf));
@@ -1771,7 +1742,7 @@ extern "C" int erirt_peer_attach(erirt_handle* h, const void* ipc_handles) {
   if (!h->xbuf) return fail(ERIRT_E_STATE, "erirt_peer_export has not been called");
   if (h->prologue_done) return fail(ERIRT_E_STATE, "erirt_peer_attach must precede erirt_sample");
   CU(cudaSetDevice(h->cfg.device));
-  if (h->peer_cache_slot >= 0) {
+  {
     std::lock_guard<std::mutex> lk(g_peer_mu);
     PeerCacheEntry& c = g_peer_cache[h->peer_cache_slot];
     if (c.handles.size() == (size_t)64 * h->world && memcmp(c.handles.data(), ipc_handles, c.handles.size()) == 0) {
@@ -1797,13 +1768,11 @@ extern "C" int erirt_peer_attach(erirt_handle* h, const void* ipc_handles) {
     opened.push_back(p);
     ptrs[r] = (double*)p;
   }
-  if (h->peer_cache_slot >= 0) {
+  {
     std::lock_guard<std::mutex> lk(g_peer_mu);
     PeerCacheEntry& c = g_peer_cache[h->peer_cache_slot];
     c.opened = opened;
     c.handles.assign((const char*)ipc_handles, (const char*)ipc_handles + (size_t)64 * h->world);
-  } else {
-    h->peer_opened = opened;
   }
   CU(cudaMemcpy(h->dPeerBufs, ptrs.data(), h->world * sizeof(double*), cudaMemcpyHostToDevice));
   h->peer_ready = true;
@@ -1813,16 +1782,14 @@ extern "C" int erirt_peer_attach(erirt_handle* h, const void* ipc_handles) {
 extern "C" int erirt_peer_detach(erirt_handle* h) {
   if (!h) return fail(ERIRT_E_ARG, "null handle");
   CU(cudaSetDevice(h->cfg.device));
-  CU(cudaStreamSynchronize(h->stream));
-  for (void* p : h->peer_opened) cudaIpcCloseMemHandle(p);  // (mappings of a cached exchange buffer stay open for the next handle)
-  h->peer_opened.clear();
+  CU(cudaStreamSynchronize(h->stream));  // (the peer mappings stay open with the cached exchange buffer, for the next handle)
   // Later sweeps go through ncclAllReduce when the chain has an NCCL communicator; a chain created with
   // erirt_comm_init(..., NULL) has no exchange left and launch_global refuses to run (ERIRT_E_STATE) instead of drawing
   // the item / structural parameters from the local shard's statistics only.
   h->peer_ready = false;
-  // both captured graphs carry GlobalArgs.peer_bufs of the mappings just closed
+  // both captured graphs carry GlobalArgs.peer_bufs, the exchange just detached
   if (h->graph_exec) { cudaGraphExecDestroy(h->graph_exec); h->graph_exec = nullptr; }
-  if (h->graph_multi) { cudaGraphExecDestroy(h->graph_multi); h->graph_multi = nullptr; h->graph_multi_sweeps = 0; }
+  if (h->graph_multi) { cudaGraphExecDestroy(h->graph_multi); h->graph_multi = nullptr; }
   return 0;
 }
 

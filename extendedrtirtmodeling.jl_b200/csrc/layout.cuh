@@ -5,10 +5,7 @@
 
 namespace erirt {
 
-#ifndef ERIRT_CTA_THREADS
-#define ERIRT_CTA_THREADS 128
-#endif
-constexpr int CTA_THREADS = ERIRT_CTA_THREADS;  // person-sweep CTA; tile = CTA_THREADS / TPP persons
+constexpr int CTA_THREADS = 128;  // person-sweep CTA; tile = CTA_THREADS / TPP persons
 constexpr int MAXD = 32;          // largest dense system solved in the global kernel (2*(nFeat+1) <= 32)
 constexpr int QCAP = 1024;        // PG fast-retry queue capacity per tile (overflow is handled inline)
 

@@ -120,30 +120,21 @@ __device__ __noinline__ double pg_draw_cell_f64(PhiloxKey key, uint32_t gid, uin
   return pg_draw_exact<double>(key, gid, sweep, j, z, 0, na);
 }
 
-#ifndef ERIRT_DIAG
-#define ERIRT_DIAG 0  // diagnostic builds only (tools/gpu_diag.sh): bit0 no PG math, bit1 no statistics pass, bit2 no row sums
-#endif
 constexpr int STAT_FLUSH_TILES = 8;  // item statistics live in registers and are folded into f64 every 8 tiles
 
 // resident CTAs per SM the register allocation is tuned for: the tile of TPP=2 leaves room for 3 CTAs, TPP=4 for 5, TPP=8 for 7.
 // TPP = 4 is compiled for four (128 registers, no spills): measured against five (102 registers) CrossQr 1M x 100 runs 1.77 -> 1.70 ms
 // per sweep and the fast kernel forced to TPP = 4 0.80 -> 0.75 ms (gpurun_out/ab_r02i.log, cqr_r02i.log); three (144 registers) is slower
-#ifndef ERIRT_MINCTAS_TPP4  // experiment hook (tools/gpu_ab2.sh)
-#define ERIRT_MINCTAS_TPP4 (ERIRT_CTA_THREADS == 128 ? 4 : 3)
-#endif
 template <int TPP>
 constexpr int min_ctas_per_sm() {
-  return CTA_THREADS == 128 ? (TPP >= 8 ? 7 : (TPP == 4 ? ERIRT_MINCTAS_TPP4 : 3)) : (TPP >= 8 ? 4 : (TPP == 4 ? ERIRT_MINCTAS_TPP4 : 1));
+  return TPP >= 8 ? 7 : (TPP == 4 ? 4 : 3);
 }
 
 // Float64: a tile row costs 17 bytes per cell, so shared memory holds three CTAs at most where TPP = 4 is chosen (J = 100: 54 KB);
 // compiled for five the kernel had 96 registers and 684 bytes of spills in its cell loop
-#ifndef ERIRT_MINCTAS_F64
-#define ERIRT_MINCTAS_F64 3
-#endif
 template <int TPP>
 constexpr int min_ctas_f64() {
-  return CTA_THREADS == 128 ? (TPP >= 8 ? 4 : ERIRT_MINCTAS_F64) : 1;
+  return TPP >= 8 ? 4 : 3;
 }
 
 // FAM = 0: the one-launch-per-sweep models (MlIrt, RtIrt, RtIrtNull, Latent, LatentQr) -- the hot configuration, with the
@@ -341,7 +332,7 @@ __global__ void __launch_bounds__(CTA_THREADS, (sizeof(R) == 8 ? min_ctas_f64<TP
       // ---- row sums over items (Draw.pl.jl:55-56, 137-138), TPP threads per person ----
       R sA2 = 0, sAB = 0, sAK = 0, sLT = 0;
       constexpr int CHUNK = 8 / TPP;  // consecutive groups owned by this thread inside each block of 8
-      for (int g0 = q * CHUNK; g0 < ((ERIRT_DIAG & 4) ? 0 : G); g0 += 8) {
+      for (int g0 = q * CHUNK; g0 < G; g0 += 8) {
 #pragma unroll
       for (int cc = 0; cc < CHUNK; ++cc) {
         const int g = g0 + cc;
@@ -622,11 +613,7 @@ __global__ void __launch_bounds__(CTA_THREADS, (sizeof(R) == 8 ? min_ctas_f64<TP
           // Float64: attempt 0 of every cell without a branch (pg_attempt0_f64: both envelope pieces, first term of the series); the
           // cells it does not accept (4 %) go to the tile's work queue and are drawn by the exact loop, dealt over the whole CTA
           uint32_t dm = 0;
-#ifndef ERIRT_F64_UNROLL
-#define ERIRT_F64_UNROLL 1
-#endif
-          constexpr int f64_unroll = ERIRT_F64_UNROLL;  // 1: one cell pair in flight (one copy of the code), 2: both pairs of the group
-  #pragma unroll f64_unroll
+#pragma unroll 1
           for (int h = 0; h < 2; ++h) {  // one Philox block = the cell pair (4g + 2h, 4g + 2h + 1); rolled: one copy of the code
             const uint4 w = philox(A.sched, gid, k + 1, make_site(DOM_PERSON, PK_PG, (uint32_t)(2 * g + h)), 0);
             const R a0 = h ? pA.v[2] : pA.v[0], a1 = h ? pA.v[3] : pA.v[1];
@@ -744,7 +731,7 @@ __global__ void __launch_bounds__(CTA_THREADS, (sizeof(R) == 8 ? min_ctas_f64<TP
     }
 
     // ---- per-item statistics: thread per (item group, person class), tile read transposed, sums kept in registers ----
-    if (e_active && !(ERIRT_DIAG & 2)) {
+    if (e_active) {
       for (int pp = er; pp < P; pp += Rc) {
         const R tp = s_u[pp * Dgp + F + 1], zp = s_u[pp * Dgp + F + 2];
         if (do_pg) {

@@ -23,19 +23,6 @@ static_assert(FMD_ABMAX < MD_COUNT, "misc block too small");
 
 constexpr int TAB_PITCH = 20;  // floats per item group in the response tables: groups g and g+4 fall on disjoint banks
 constexpr int FAST_FLUSH_TILES = 16;  // item statistics live in f32 registers and are folded into the f64 accumulators every 16 tiles
-// ERIRT_QUEUE_MODE 0 (default): one two-ended work queue per tile (CTA), [0, QSTD) certainly-rejected cells, [QSTD, QCAP) undecided /
-// Method-B cells, filled with one shared-memory atomic per warp and drained by all four warps after a CTA barrier.
-// ERIRT_QUEUE_MODE 1 (experiment, measured 7 % slower at C5: the per-warp remainders cost more than the two barriers save):
-// work queues of the cells that leave the fast path are WARP-LOCAL: a warp serves its own persons from the row sums to the
-// drain, so nothing between the tile load and the transposed statistics pass needs a CTA barrier.  Region of a warp:
-// QW entries, [0, QSTDW) certainly-rejected cells (standard), [QSTDW, QW) undecided / Method-B cells (special).
-#ifndef ERIRT_QUEUE_MODE
-#define ERIRT_QUEUE_MODE 0
-#endif
-constexpr int QSTD = 768;
-constexpr int QW = QCAP / (CTA_THREADS / 32);
-constexpr int QSTDW = (QW * 3) / 4;
-
 // Phase timers of the diagnostic build (tools/make_tick_build.py, -DERIRT_TICKS): clock64() per warp at the phase boundaries.
 #ifdef ERIRT_TICKS
 #define PF_NTICK 16
@@ -537,7 +524,6 @@ __global__ void __launch_bounds__(CTA_THREADS, min_ctas_per_sm<TPP>()) person_sw
       }
     }
     PF_TICK(6);  // PG main pass
-#if ERIRT_QUEUE_MODE == 0
     {
       // ---- hand the cells that left the fast path to the tile's work queues: one shared-memory atomic per WARP reserves the
       //      slots of all its lanes in both queues (packed counts, warp prefix sum), then every lane writes its entries ----
@@ -636,93 +622,6 @@ __global__ void __launch_bounds__(CTA_THREADS, min_ctas_per_sm<TPP>()) person_sw
     __syncthreads();  // the whole tile (omega_{k+1}, u rows) is final: the transposed passes below read across warps
     if (tid == 0) s_qctl[0] = 0;  // next written by the push of the next tile, two barriers from here
     PF_TICK(10);  // barrier
-#else
-    uint32_t wq_counts;  // packed entry counts of this warp's queues (low 16 bits standard, high 16 bits special)
-    uint32_t* const wq = s_queue + (tid >> 5) * QW;
-    {
-      // ---- hand the cells that left the fast path to the WARP's work queues: a warp prefix sum over the packed counts gives every
-      //      lane its slots in both queues (no atomic, no CTA barrier), then every lane writes its entries ----
-      const u64 smask = dmask & rmask, umask = dmask & ~rmask;  // standard (certainly rejected) / special (undecided)
-      const uint32_t n_std = (uint32_t)__popcll(smask), n_spc = (uint32_t)__popcll(umask);
-      acc_defer += n_std + n_spc;
-      uint32_t pre = n_std | (n_spc << 16);
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t t = __shfl_up_sync(0xffffffffu, pre, o);
-        if ((tid & 31) >= o) pre += t;
-      }
-      wq_counts = __shfl_sync(0xffffffffu, pre, 31);
-      uint32_t slot_s = (pre & 0xffffu) - n_std;
-      uint32_t slot_u = (pre >> 16) - n_spc;
-      // bit 4*kk+e of a mask -> item index: the thread owns 32/TPP consecutive items in every block of 32
-      constexpr int BPB = 32 / TPP;
-      auto push = [&](uint32_t m, int bit0, uint32_t& slot, const uint32_t cap, const uint32_t qbase, const uint32_t flag) {
-        while (m) {
-          const int bit = bit0 + __ffs((int)m) - 1;
-          m &= m - 1u;
-          const int j = ((bit / BPB) << 5) + q * BPB + (bit % BPB);
-          if (slot < cap) wq[qbase + slot] = ((uint32_t)p << 16) | (uint32_t)j | flag;
-          else {  // queue overflow: finish the cell here
-            const float z = fmaf(s_par[PAR_A * Jp + j], thp, s_par[PAR_AB * Jp + j]);
-            my_om[j] = pg_resolve_f32(A.key, gid, k + 1, j, z, flag != 0u);
-          }
-          ++slot;
-        }
-      };
-      if (wq_counts) {
-        push((uint32_t)smask, 0, slot_s, (uint32_t)QSTDW, 0u, 0u);
-        push((uint32_t)(smask >> 32), 32, slot_s, (uint32_t)QSTDW, 0u, 0u);
-        push((uint32_t)umask, 0, slot_u, (uint32_t)(QW - QSTDW), (uint32_t)QSTDW, 0x80000000u);
-        push((uint32_t)(umask >> 32), 32, slot_u, (uint32_t)(QW - QSTDW), (uint32_t)QSTDW, 0x80000000u);
-      }
-    }
-    PF_TICK(7);  // queue push
-    __syncwarp();  // the warp's queue entries and the theta_k of its persons (s_u) are visible to its lanes
-    PF_TICK(8);
-
-    if (wq_counts) {
-      // ---- drain, one phase per warp: standard entries (Method-A retry rounds, two cells in flight per lane) are dealt from lane 0
-      //      upwards, special entries (undecided attempt 0: replay it with the a_1 term) from the last lane downwards ----
-      const int lane = tid & 31;
-      const uint32_t qn = min(wq_counts & 0xffffu, (uint32_t)QSTDW), qu = min(wq_counts >> 16, (uint32_t)(QW - QSTDW));
-      for (uint32_t idx = lane; idx < qn; idx += 64) {
-        const bool has2 = idx + 32 < qn;
-        const uint32_t e1 = wq[idx], e2 = wq[has2 ? idx + 32 : idx];
-        const int j1 = (int)(e1 & 0xffffu), p1 = (int)(e1 >> 16), j2 = (int)(e2 & 0xffffu), p2 = (int)(e2 >> 16);
-        const float z1 = fmaf(s_par[PAR_A * Jp + j1], s_u[p1 * Dgp + F + 1], s_par[PAR_AB * Jp + j1]);
-        const float z2 = fmaf(s_par[PAR_A * Jp + j2], s_u[p2 * Dgp + F + 1], s_par[PAR_AB * Jp + j2]);
-        const uint32_t g1 = A.person_offset + (uint32_t)(row0 + p1), g2 = A.person_offset + (uint32_t)(row0 + p2);
-        const bool b1 = !(0.5f * fabsf(z1) <= (float)PG_CSWITCH), b2 = !(0.5f * fabsf(z2) <= (float)PG_CSWITCH);  // Method B or NaN
-        float om1 = b1 ? 0.0f : -2.0f, om2 = (has2 && !b2) ? -2.0f : 0.0f;
-#pragma unroll 1
-        for (uint32_t r = 1; r < PG_MAX_ATTEMPTS && (om1 < 0.f || om2 < 0.f); ++r) {
-          const uint4 w1 = philox(A.sched, g1, k + 1, make_site(DOM_PERSON, PK_PG_RETRY, (uint32_t)j1), r);
-          const uint4 w2 = philox(A.sched, g2, k + 1, make_site(DOM_PERSON, PK_PG_RETRY, (uint32_t)j2), r);
-          const float o1 = pg_exact_pair(z1, w1.x, w1.y, w1.z, w1.w);
-          const float o2 = pg_exact_pair(z2, w2.x, w2.y, w2.z, w2.w);
-          if (om1 < 0.f) om1 = o1;
-          if (om2 < 0.f) om2 = o2;
-        }
-        if (om1 < 0.f) om1 = 0.25f * (float)PG_T;
-        if (om2 < 0.f) om2 = 0.25f * (float)PG_T;
-        if (b1) om1 = pg_resolve_f32(A.key, g1, k + 1, j1, z1, false);  // rare: Method-B regime (or NaN state)
-        if (has2 && b2) om2 = pg_resolve_f32(A.key, g2, k + 1, j2, z2, false);
-        s_om[p1 * Jp + j1] = om1;
-        if (has2) s_om[p2 * Jp + j2] = om2;
-      }
-      for (uint32_t idx = (uint32_t)(31 - lane); idx < qu; idx += 32) {
-        const uint32_t e1 = wq[QSTDW + idx];
-        const int j1 = (int)(e1 & 0xffffu), p1 = (int)((e1 >> 16) & 0x7fffu);
-        const float z1 = fmaf(s_par[PAR_A * Jp + j1], s_u[p1 * Dgp + F + 1], s_par[PAR_AB * Jp + j1]);
-        s_om[p1 * Jp + j1] = pg_resolve_f32(A.key, A.person_offset + (uint32_t)(row0 + p1), k + 1, j1, z1, true);
-      }
-    }
-    PF_TICK(9);  // drain
-    __syncthreads();  // the whole tile (omega_{k+1}, u rows) is final: the transposed passes below read across warps
-    PF_TICK(10);  // barrier
-    const int next_tile = (int)s_qctl[1];
-    if (next_tile >= A.n_tiles - 2 * (int)gridDim.x) griddep_launch();
-#endif
 
     // ---- per-item statistics: thread per (item group, person class), tile read transposed, sums kept in registers ----
     if (e_active) {

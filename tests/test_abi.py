@@ -78,6 +78,34 @@ def test_product_does_not_import_oracle():
                 assert "oracle_py" not in txt and "liberirt_oracle" not in txt and "import oracle" not in txt, f
 
 
+def test_environment_and_build_switches_are_the_documented_ones():
+    """The ERIRT_* environment variables the product reads are exactly those of the table in INTEGRATION.md section 5, and the only
+    ERIRT_* macros the kernels test with #if / #ifdef / #ifndef are the three diagnostic builds: no tuning switch selects a path
+    that the benchmark does not run."""
+    pkg = os.path.join(ROOT, "extendedrtirtmodeling.jl_b200")
+    sources = [os.path.join(ROOT, "bench.py")]
+    sources += [os.path.join(ROOT, "julia", f) for f in os.listdir(os.path.join(ROOT, "julia")) if f.endswith(".jl")]
+    for dirpath, _, files in os.walk(pkg):
+        sources += [os.path.join(dirpath, f) for f in files if f.endswith((".py", ".cu", ".cuh", ".h"))]
+    read = set()
+    for path in sources:
+        txt = open(path, encoding="utf-8", errors="ignore").read()
+        read |= set(re.findall(r'(?:getenv\(|os\.environ\.get\(|get\(ENV,\s*)"(ERIRT_[A-Z0-9_]+)"', txt))
+    doc = open(os.path.join(ROOT, "INTEGRATION.md"), encoding="utf-8").read()
+    table = doc[doc.index("## 5. Environment switches"):]
+    table = table[:table.index("\n## ")] if "\n## " in table else table
+    documented = set(re.findall(r"^\|\s*`(ERIRT_[A-Z0-9_]+)`\s*\|", table, flags=re.M))
+    assert read == documented, f"read but not documented: {sorted(read - documented)}; documented but not read: {sorted(documented - read)}"
+
+    tested = set()
+    for dirpath, _, files in os.walk(os.path.join(pkg, "csrc")):
+        for f in files:
+            for line in open(os.path.join(dirpath, f), encoding="utf-8", errors="ignore"):
+                if re.match(r"\s*#\s*(?:if|ifdef|ifndef)\b", line):
+                    tested |= set(re.findall(r"\b(ERIRT_[A-Z0-9_]+)\b", line))
+    assert tested == {"ERIRT_TICKS", "ERIRT_TIMELINE", "ERIRT_CHECKS"}, sorted(tested)
+
+
 def test_julia_stub_matches_the_header(lib):
     """julia/ErirtB200.jl cannot be executed here (no Julia): check statically that its ErirtConfig mirrors erirt_config field by field
     (names, order, widths) and that every C symbol it ccalls is declared in include/erirt_b200.h."""

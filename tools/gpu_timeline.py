@@ -62,7 +62,7 @@ if TICKS:
         if v: print(f"  {nm:28s} {v / K:14.0f} warp-cycles per sweep  {100 * v / tot:5.1f} %")
     sys.exit(0)
 eng.sample(K)
-print(which, "ms per sweep", eng.stats()["last_sample_ms"] / K, "PDL", os.environ.get("ERIRT_PDL", "1"), "REHEARSE", os.environ.get("ERIRT_G_REHEARSE", "1"))
+print(which, "ms per sweep", eng.stats()["last_sample_ms"] / K)
 buf = (ctypes.c_ulonglong * (256 * 16))()
 eng.lib.erirt_diag_timeline(buf)
 t = np.array(list(buf), dtype=np.float64).reshape(256, 16)
