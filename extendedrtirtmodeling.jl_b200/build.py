@@ -1,4 +1,5 @@
 """Build the CUDA shared library in-tree with nvcc for sm_100a (no JIT cache, the .so travels with the repo)."""
+import glob
 import os
 import shutil
 import subprocess
@@ -7,7 +8,6 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "liberirt_b200.so")
 SOURCES = ["erirt_b200.cu"]
-HEADERS = ["rng.cuh", "pg.cuh", "pg_fast.cuh", "pg_coeffs.h", "layout.cuh", "person.cuh", "person_fast.cuh", "global.cuh"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
               "-shared"]
 
@@ -23,7 +23,8 @@ def is_stale():
     if not os.path.exists(LIB):
         return True
     t = os.path.getmtime(LIB)
-    deps = [os.path.join(CSRC, f) for f in SOURCES + HEADERS] + [os.path.join(HERE, "..", "include", "erirt_b200.h")]
+    # every file of csrc/ (the sources and every header they include) and the ABI header
+    deps = glob.glob(os.path.join(CSRC, "*")) + [os.path.join(HERE, "..", "include", "erirt_b200.h")]
     return any(os.path.getmtime(d) > t for d in deps if os.path.exists(d))
 
 

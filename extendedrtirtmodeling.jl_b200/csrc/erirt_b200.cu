@@ -56,6 +56,24 @@ static int fail(int code, const char* fmt, ...) {
     cudaError_t _e = (expr);                                                                             \
     if (_e != cudaSuccess) return fail(ERIRT_E_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__); \
   } while (0)
+// CU for a function that holds stream-ordered staging buffers: its lambda `cleanup` frees them before the error is returned
+#define CUX(expr)                                                                                        \
+  do {                                                                                                   \
+    cudaError_t _e = (expr);                                                                             \
+    if (_e != cudaSuccess) {                                                                             \
+      cleanup();                                                                                         \
+      return fail(ERIRT_E_CUDA, "%s failed: %s", #expr, cudaGetErrorString(_e));                        \
+    }                                                                                                    \
+  } while (0)
+
+static int pick_device(int device) {
+  int ndev = 0;
+  cudaError_t e = cudaGetDeviceCount(&ndev);
+  if (e != cudaSuccess || ndev == 0) return fail(ERIRT_E_CUDA, "no CUDA device available (%s); this engine has no CPU fallback", cudaGetErrorString(e));
+  if (device < 0 || device >= ndev) return fail(ERIRT_E_ARG, "device %d out of range [0,%d)", device, ndev);
+  CU(cudaSetDevice(device));
+  return 0;
+}
 
 // ------------------------------------------------------------------------------------------------
 // NCCL through dlopen (no link-time dependency; single-GPU use never touches it)
@@ -130,15 +148,7 @@ __global__ void pack_transpose_kernel(const SrcT* __restrict__ src, int64_t ld, 
     }
   }
 }
-template <typename R>
-__global__ void pack_vec_kernel(const double* __restrict__ src, int64_t n, R* __restrict__ dst) {
-  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) dst[i] = (R)src[i];
-}
-template <typename R>
-__global__ void unpack_vec_kernel(const R* __restrict__ src, int64_t n, double* __restrict__ dst) {
-  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) dst[i] = (double)src[i];
-}
-// row-major padded [n][Jp] <-> column-major [n][J] float64 (state get/set of omega)
+// row-major padded [n][Jp] <-> column-major [n][J] float64 (data and state get/set; a person vector or one column of X is J = Jp = 1)
 template <typename R>
 __global__ void tile_to_colmajor_kernel(const R* __restrict__ src, int64_t n, int J, int Jp, double* __restrict__ dst) {
   const int64_t total = n * J;
@@ -186,7 +196,8 @@ __global__ void colsum_finish_kernel(const double* __restrict__ part, int J, dou
   for (int p = 0; p < parts; ++p) acc += part[(int64_t)j * parts + p];
   out[j] = acc;
 }
-// the same for the N x J cell weights of CrossQr: sums tiled [n_pad][Jp], results column-major [n][J]
+// post-burn-in mean and SD from the running sums: tiled [n_pad][Jp] (the N x J cell weights of CrossQr), results column-major [n][J];
+// a person vector is J = Jp = 1.  No FMA contraction: same bits as the host formula
 __global__ void tile_moments_kernel(const double* __restrict__ s1, const double* __restrict__ s2, int64_t n, int J, int Jp, double cnt,
                                     double* __restrict__ mean, double* __restrict__ sd) {
   const int64_t total = n * J;
@@ -197,16 +208,6 @@ __global__ void tile_moments_kernel(const double* __restrict__ s1, const double*
     const double a = s1[i * Jp + j], b = s2[i * Jp + j], m = a / cnt;
     mean[t] = m;
     sd[t] = cnt > 1.0 ? sqrt(fmax(0.0, __dsub_rn(b, __dmul_rn(__dmul_rn(cnt, m), m)) / (cnt - 1.0))) : 0.0;
-  }
-}
-// post-burn-in mean and SD of a person vector from its running sums (erirt_get_moments)
-__global__ void moments_finish_kernel(const double* __restrict__ s1, const double* __restrict__ s2, int64_t n, double cnt,
-                                      double* __restrict__ mean, double* __restrict__ sd) {
-  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-    if (cnt <= 0.0) { mean[i] = sd[i] = __longlong_as_double(0x7ff8000000000000LL); continue; }
-    const double m = s1[i] / cnt;
-    mean[i] = m;
-    sd[i] = cnt > 1.0 ? sqrt(fmax(0.0, __dsub_rn(s2[i], __dmul_rn(__dmul_rn(cnt, m), m)) / (cnt - 1.0))) : 0.0;  // no FMA contraction: same bits as the host formula
   }
 }
 // column sums of the packed tiles (erirt_generate_data: the data never existed in column-major form), same two-stage scheme with
@@ -333,6 +334,8 @@ struct erirt_handle {
   int sm_count = 0;
   int grid = 0;
   size_t rsz = 4;
+  double k1 = 0.0, k2 = 0.0;  // (1 - 2q) / (q (1 - q)) and 2 / (q (1 - q)) of q = cfg.q_rt
+  PhiloxKey key{};            // make_key(cfg.seed, cfg.chain)
   int64_t n_pad = 0;
   int cap = 0, qw = 0;
   cudaStream_t stream = nullptr;
@@ -376,7 +379,9 @@ struct erirt_handle {
 static int launch_person(erirt_handle* h, int stage);
 static int launch_global(erirt_handle* h, int stage);
 static int finalize_constants(erirt_handle* h);
-static int pick_device(int32_t device);
+// fn(float{}) or fn(double{}): the real type R of the handle's device state, for launches of a kernel template over R
+template <typename Fn>
+static auto with_real(const erirt_handle* h, Fn&& fn) { return h->cfg.dtype == ERIRT_F32 ? fn(float{}) : fn(double{}); }
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 // `fast`: plan of person_sweep_fast_kernel (f32, one-launch models): the generic plan plus the response tables
@@ -543,11 +548,7 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
   if (!(cfg->q_rt > 0.0 && cfg->q_rt < 1.0)) return fail(ERIRT_E_ARG, "qRt must be between 0 and 1");  // Draw.pl.jl:476
 
   HostTimer tm;
-  int ndev = 0;
-  cudaError_t e = cudaGetDeviceCount(&ndev);
-  if (e != cudaSuccess || ndev == 0) return fail(ERIRT_E_CUDA, "no CUDA device available (%s); this engine has no CPU fallback", cudaGetErrorString(e));
-  if (cfg->device < 0 || cfg->device >= ndev) return fail(ERIRT_E_ARG, "device %d out of range [0,%d)", cfg->device, ndev);
-  CU(cudaSetDevice(cfg->device));
+  if (int rc = pick_device(cfg->device)) return rc;
   // three attributes, not cudaGetDeviceProperties: that call was measured at 3-260 ms per erirt_create on this box
   struct { int major, minor, multiProcessorCount; } prop;
   CU(cudaDeviceGetAttribute(&prop.major, cudaDevAttrComputeCapabilityMajor, cfg->device));
@@ -570,12 +571,15 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
   h->cfg = *cfg;
   h->sm_count = prop.multiProcessorCount;
   h->rsz = cfg->dtype == ERIRT_F32 ? 4 : 8;
+  h->k1 = (1.0 - 2.0 * cfg->q_rt) / (cfg->q_rt * (1.0 - cfg->q_rt));
+  h->k2 = 2.0 / (cfg->q_rt * (1.0 - cfg->q_rt));
+  h->key = make_key(cfg->seed, cfg->chain);
   h->L = make_layout(cfg->n_item, cfg->n_feat);
   const bool has_rt = cfg->model != ERIRT_MLIRT;
   // threads per person: smallest TPP whose shared-memory plan leaves room for >= 3 CTAs per SM (75 KB + 1 KB reserved each)
   const bool is_cross = cfg->model == ERIRT_RTIRT_CROSS || cfg->model == ERIRT_RTIRT_CROSSQR;
   const bool is_cqr = cfg->model == ERIRT_RTIRT_CROSSQR;
-  const bool fast_engine = h->rsz == 4 && !is_cross;
+  const bool fast_engine = cfg->dtype == ERIRT_F32 && !is_cross;
   const int n_groups = h->L.Jp / 4;
   auto choose = [&](bool fast, int& tpp, SmemPlan& S) -> const char* {
     for (tpp = 1; tpp < 8; tpp *= 2) {
@@ -587,7 +591,7 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
     // sweep is bound by the per-tile latency chain, gain nothing: profiles/r02_summary.md)
     // (for a large problem TPP = 8 was 7 % faster while the cell loop was one divergent exact draw per cell; with the branch-free
     // attempt 0 the 168-register TPP = 4 instantiation wins, 4.0 against 5.3 ms per sweep at 1M x 100)
-    if (!fast && h->rsz == 8)
+    if (!fast && cfg->dtype == ERIRT_F64)
       while (tpp < 8 && (int64_t)align_up((size_t)cfg->n_subj, 128) / (CTA_THREADS / tpp) < 2 * (int64_t)h->sm_count) tpp *= 2;
     if (n_groups > 16 * tpp) return "too many items for this TPP (at most 64*TPP - 4)";
     S = make_smem_plan(h->L, tpp, h->rsz, has_rt, is_cqr, is_cross, fast);
@@ -750,6 +754,45 @@ static void pack_columns(erirt_handle* h, const YT* dYc, int64_t ldY, const doub
   }
 }
 
+// The start of every ingest: zero the packed Y / logT (the padding cells stay zero) and the constants the ingest adds up
+static int clear_data(erirt_handle* h) {
+  const size_t cells = (size_t)h->n_pad * h->L.Jp;
+  CU(cudaMemsetAsync(h->dY, 0, cells, h->stream));
+  if (h->cfg.model != ERIRT_MLIRT) CU(cudaMemsetAsync(h->dLogT, 0, cells * h->rsz, h->stream));
+  CU(cudaMemsetAsync(h->dConstsLocal, 0, h->c_count * sizeof(double), h->stream));
+  return 0;
+}
+
+// The end of every ingest, after Y / logT are packed: X (column-major float64 [n][F], leading dimension ldX; a host buffer unless
+// x_on_device) into dX, the constants in f64 (T1, T2, K0 are consecutive Jp-blocks of the consts vector, finished from `part`:
+// [3 Jp][parts] partial column sums; X'X), then a synchronisation, after which the data set is in place.
+static int finish_ingest(erirt_handle* h, const double* X, int64_t ldX, bool x_on_device, const double* part, int parts) {
+  const int64_t n = h->cfg.n_subj;
+  const int Jp = h->L.Jp, F = h->cfg.n_feat, pb = F + 1;
+  double* staged = nullptr;
+  auto cleanup = [&]() { if (staged) cudaFreeAsync(staged, h->stream); };
+  if (F > 0 && !x_on_device) {
+    CUX(cudaMallocAsync((void**)&staged, (size_t)n * F * sizeof(double), h->stream));
+    CUX(cudaMemcpy2DAsync(staged, n * sizeof(double), X, ldX * sizeof(double), n * sizeof(double), F, cudaMemcpyHostToDevice, h->stream));
+    X = staged;
+    ldX = n;
+  }
+  for (int f = 0; f < F; ++f)
+    with_real(h, [&](auto r) {
+      using R = decltype(r);
+      colmajor_to_tile_kernel<R><<<1024, 256, 0, h->stream>>>(X + ldX * f, n, 1, 1, (R*)h->dX + (int64_t)f * h->n_pad);
+    });
+  colsum_finish_kernel<<<(3 * Jp + 127) / 128, 128, 0, h->stream>>>(part, 3 * Jp, h->dConstsLocal + h->c_T1, parts);
+  xtx_kernel<<<pb * pb, 256, 0, h->stream>>>(X, ldX, n, pb, h->dConstsLocal + h->c_XtX);
+  CUX(cudaGetLastError());
+  cleanup();
+  staged = nullptr;
+  CUX(cudaStreamSynchronize(h->stream));
+  h->data_set = true;
+  h->consts_final = false;
+  return 0;
+}
+
 // Ingest (K8).  on_device: the three matrices are device buffers and are packed in place.  Otherwise they are host buffers and are
 // streamed through one bounded staging buffer in chunks of whole columns (H2D copy, pack, next chunk: the staging memory stays at
 // <= 64 MB instead of a second copy of the data set, and the packed tiles are the only full-size device copy).
@@ -761,59 +804,32 @@ static int ingest(erirt_handle* h, const YT* Y, int64_t ldY, const double* T, in
   if (h->cfg.n_feat > 0 && !X) return fail(ERIRT_E_ARG, "X is required when n_feat > 0");
   CU(cudaSetDevice(h->cfg.device));
   const int64_t n = h->cfg.n_subj;
-  const int J = h->cfg.n_item, Jp = h->L.Jp, F = h->cfg.n_feat, pb = F + 1;
-  const bool f32 = h->cfg.dtype == ERIRT_F32;
+  const int J = h->cfg.n_item, Jp = h->L.Jp, F = h->cfg.n_feat;
   if (ldY < n || (has_rt && ldT < n) || (F > 0 && ldX < n)) return fail(ERIRT_E_ARG, "leading dimension smaller than n_subj");
   if (!has_rt) T = nullptr;
-  const size_t cells = (size_t)h->n_pad * Jp;
-  CU(cudaMemsetAsync(h->dY, 0, cells, h->stream));
-  if (has_rt) CU(cudaMemsetAsync(h->dLogT, 0, cells * h->rsz, h->stream));
-  CU(cudaMemsetAsync(h->dConstsLocal, 0, h->c_count * sizeof(double), h->stream));
+  if (int rc = clear_data(h)) return rc;
   CU(cudaMemsetAsync(h->dColPart, 0, (size_t)3 * Jp * COLSUM_PARTS * sizeof(double), h->stream));
-  char* stage = nullptr;
-  double* dXc = nullptr;
-  auto cleanup = [&]() { if (stage) cudaFreeAsync(stage, h->stream); if (dXc && !on_device) cudaFreeAsync(dXc, h->stream); };
-#define CUX(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) { cleanup(); return fail(ERIRT_E_CUDA, "%s failed: %s", #expr, cudaGetErrorString(_e)); } } while (0)
   if (on_device) {
-    if (f32) pack_columns<float, YT>(h, Y, ldY, T, ldT, 0, J);
-    else pack_columns<double, YT>(h, Y, ldY, T, ldT, 0, J);
-    dXc = const_cast<double*>(X);
-  } else {
-    // stream-ordered allocations: cudaFree of large blocks is a device-wide synchronisation (measured up to 0.9 s for GB-sized blocks)
-    const size_t col_bytes = (size_t)n * (sizeof(YT) + (has_rt ? sizeof(double) : 0));
-    int cc = (int)std::max<size_t>(1, std::min<size_t>((size_t)J, ((size_t)64 << 20) / col_bytes));
-    const size_t y_bytes = align_up((size_t)n * cc * sizeof(YT), 256);
-    CUX(cudaMallocAsync((void**)&stage, y_bytes + (has_rt ? (size_t)n * cc * sizeof(double) : 0), h->stream));
-    YT* sY = (YT*)stage;
-    double* sT = has_rt ? (double*)(stage + y_bytes) : nullptr;
-    for (int c0 = 0; c0 < J; c0 += cc) {
-      const int nc = std::min(cc, J - c0);
-      CUX(cudaMemcpy2DAsync(sY, n * sizeof(YT), Y + ldY * c0, ldY * sizeof(YT), n * sizeof(YT), nc, cudaMemcpyHostToDevice, h->stream));
-      if (has_rt) CUX(cudaMemcpy2DAsync(sT, n * sizeof(double), T + ldT * c0, ldT * sizeof(double), n * sizeof(double), nc, cudaMemcpyHostToDevice, h->stream));
-      if (f32) pack_columns<float, YT>(h, sY, n, sT, n, c0, nc);
-      else pack_columns<double, YT>(h, sY, n, sT, n, c0, nc);
-    }
-    if (F > 0) {
-      CUX(cudaMallocAsync((void**)&dXc, (size_t)n * F * sizeof(double), h->stream));
-      CUX(cudaMemcpy2DAsync(dXc, n * sizeof(double), X, ldX * sizeof(double), n * sizeof(double), F, cudaMemcpyHostToDevice, h->stream));
-      ldX = n;
-    }
+    with_real(h, [&](auto r) { pack_columns<decltype(r), YT>(h, Y, ldY, T, ldT, 0, J); });
+    return finish_ingest(h, X, ldX, true, h->dColPart, COLSUM_PARTS);
   }
-  for (int f = 0; f < F; ++f) {
-    if (f32) pack_vec_kernel<float><<<256, 256, 0, h->stream>>>(dXc + ldX * f, n, (float*)h->dX + (int64_t)f * h->n_pad);
-    else pack_vec_kernel<double><<<256, 256, 0, h->stream>>>(dXc + ldX * f, n, (double*)h->dX + (int64_t)f * h->n_pad);
+  // stream-ordered allocations: cudaFree of large blocks is a device-wide synchronisation (measured up to 0.9 s for GB-sized blocks)
+  char* stage = nullptr;
+  auto cleanup = [&]() { if (stage) cudaFreeAsync(stage, h->stream); };
+  const size_t col_bytes = (size_t)n * (sizeof(YT) + (has_rt ? sizeof(double) : 0));
+  int cc = (int)std::max<size_t>(1, std::min<size_t>((size_t)J, ((size_t)64 << 20) / col_bytes));
+  const size_t y_bytes = align_up((size_t)n * cc * sizeof(YT), 256);
+  CUX(cudaMallocAsync((void**)&stage, y_bytes + (has_rt ? (size_t)n * cc * sizeof(double) : 0), h->stream));
+  YT* sY = (YT*)stage;
+  double* sT = has_rt ? (double*)(stage + y_bytes) : nullptr;
+  for (int c0 = 0; c0 < J; c0 += cc) {
+    const int nc = std::min(cc, J - c0);
+    CUX(cudaMemcpy2DAsync(sY, n * sizeof(YT), Y + ldY * c0, ldY * sizeof(YT), n * sizeof(YT), nc, cudaMemcpyHostToDevice, h->stream));
+    if (has_rt) CUX(cudaMemcpy2DAsync(sT, n * sizeof(double), T + ldT * c0, ldT * sizeof(double), n * sizeof(double), nc, cudaMemcpyHostToDevice, h->stream));
+    with_real(h, [&](auto r) { pack_columns<decltype(r), YT>(h, sY, n, sT, n, c0, nc); });
   }
-  // constants in f64 straight from the caller's data: T1, T2, K0 are consecutive Jp-blocks of the consts vector
-  colsum_finish_kernel<<<(3 * Jp + 127) / 128, 128, 0, h->stream>>>(h->dColPart, 3 * Jp, h->dConstsLocal + h->c_T1);
-  xtx_kernel<<<pb * pb, 256, 0, h->stream>>>(dXc, ldX, n, pb, h->dConstsLocal + h->c_XtX);
-  CUX(cudaGetLastError());
   cleanup();
-  stage = nullptr; dXc = nullptr;
-  CUX(cudaStreamSynchronize(h->stream));
-#undef CUX
-  h->data_set = true;
-  h->consts_final = false;
-  return 0;
+  return finish_ingest(h, X, ldX, false, h->dColPart, COLSUM_PARTS);
 }
 
 // ---- data generated on the device (SURVEY 8f-1) ----
@@ -826,11 +842,11 @@ extern "C" int erirt_generate_data(erirt_handle* h, const double* theta, const d
   if (error_type < 0 || error_type > 4) return fail(ERIRT_E_ARG, "error_type must be 0 (truncated normal), 1 (unit normal), 2 (norm), 3 (tail) or 4 (skew)");
   if (has_rt && error_type == 0 && !sigma2) return fail(ERIRT_E_ARG, "sigma2 is required for error_type 0");
   const int64_t n = h->cfg.n_subj;
-  const int J = h->cfg.n_item, Jp = h->L.Jp, F = h->cfg.n_feat, pb = F + 1;
+  const int J = h->cfg.n_item, Jp = h->L.Jp, F = h->cfg.n_feat;
   if (F > 0 && (!X || ldX < n)) return fail(ERIRT_E_ARG, "X (leading dimension >= n_subj) is required when n_feat > 0");
   CU(cudaSetDevice(h->cfg.device));
-  const bool f32 = h->cfg.dtype == ERIRT_F32;
   HostTimer tm;
+  if (int rc = clear_data(h)) return rc;
   // device copy of the small inputs: [theta n][zeta n][a Jp][b Jp][lambda Jp][sd Jp][rho Jp]; the person vectors go straight from
   // the caller's buffers, the item vectors through a small host block
   std::vector<double> hit((size_t)5 * Jp, 0.0);
@@ -842,19 +858,13 @@ extern "C" int erirt_generate_data(erirt_handle* h, const double* theta, const d
     it[3 * Jp + j] = sigma2 ? std::sqrt(sigma2[j]) : 1.0;
     it[4 * Jp + j] = rho ? rho[j] : 0.0;
   }
-  double *dbuf = nullptr, *dXc = nullptr, *dpart_alloc = nullptr;
-  auto cleanup = [&]() { if (dbuf) cudaFreeAsync(dbuf, h->stream); if (dXc) cudaFreeAsync(dXc, h->stream); if (dpart_alloc) cudaFreeAsync(dpart_alloc, h->stream); };
-#define CUX(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) { cleanup(); return fail(ERIRT_E_CUDA, "%s failed: %s", #expr, cudaGetErrorString(_e)); } } while (0)
+  double *dbuf = nullptr, *dpart = nullptr;  // dpart: [3][Jp][TILE_COLSUM_PARTS]
+  auto cleanup = [&]() { if (dbuf) cudaFreeAsync(dbuf, h->stream); if (dpart) cudaFreeAsync(dpart, h->stream); };
   CUX(cudaMallocAsync((void**)&dbuf, ((size_t)2 * n + 5 * Jp) * sizeof(double), h->stream));
   CUX(cudaMemcpyAsync(dbuf, theta, n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
   if (has_rt) CUX(cudaMemcpyAsync(dbuf + n, zeta, n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
   CUX(cudaMemcpyAsync(dbuf + 2 * n, hit.data(), hit.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
   tm.mark("generate: host staging, H2D");
-  const size_t cells = (size_t)h->n_pad * Jp;
-  CUX(cudaMemsetAsync(h->dY, 0, cells, h->stream));
-  if (has_rt) CUX(cudaMemsetAsync(h->dLogT, 0, cells * h->rsz, h->stream));
-  CUX(cudaMemsetAsync(h->dConstsLocal, 0, h->c_count * sizeof(double), h->stream));
-  double* dpart = nullptr;  // [3][Jp][TILE_COLSUM_PARTS]
   GenArgs A{};
   A.Y = h->dY; A.logT = h->dLogT;
   A.theta = dbuf; A.zeta = has_rt ? dbuf + n : nullptr;
@@ -862,33 +872,16 @@ extern "C" int erirt_generate_data(erirt_handle* h, const double* theta, const d
   A.n = n; A.J = J; A.Jp = Jp; A.err = error_type; A.has_rt = has_rt ? 1 : 0;
   A.person_offset = (uint32_t)h->cfg.subj_offset;
   A.key = make_key(seed, 0xDA7Au);
-  const int grid = h->sm_count * 8;
-  if (f32) generate_data_kernel<float><<<grid, 256, 0, h->stream>>>(A);
-  else generate_data_kernel<double><<<grid, 256, 0, h->stream>>>(A);
-  CUX(cudaMallocAsync((void**)&dpart_alloc, (size_t)3 * Jp * TILE_COLSUM_PARTS * sizeof(double), h->stream));
-  dpart = dpart_alloc;
-  if (f32) tile_colsum_part_kernel<float><<<TILE_COLSUM_PARTS, Jp, 0, h->stream>>>(h->dY, has_rt ? (const float*)h->dLogT : nullptr, n, Jp, dpart);
-  else tile_colsum_part_kernel<double><<<TILE_COLSUM_PARTS, Jp, 0, h->stream>>>(h->dY, has_rt ? (const double*)h->dLogT : nullptr, n, Jp, dpart);
-  if (F > 0) {
-    CUX(cudaMallocAsync((void**)&dXc, (size_t)n * F * sizeof(double), h->stream));
-    CUX(cudaMemcpy2DAsync(dXc, n * sizeof(double), X, ldX * sizeof(double), n * sizeof(double), F, cudaMemcpyHostToDevice, h->stream));
-  }
-  for (int f = 0; f < F; ++f) {
-    if (f32) pack_vec_kernel<float><<<256, 256, 0, h->stream>>>(dXc + (int64_t)n * f, n, (float*)h->dX + (int64_t)f * h->n_pad);
-    else pack_vec_kernel<double><<<256, 256, 0, h->stream>>>(dXc + (int64_t)n * f, n, (double*)h->dX + (int64_t)f * h->n_pad);
-  }
-  colsum_finish_kernel<<<(3 * Jp + 127) / 128, 128, 0, h->stream>>>(dpart, 3 * Jp, h->dConstsLocal + h->c_T1, TILE_COLSUM_PARTS);
-  xtx_kernel<<<pb * pb, 256, 0, h->stream>>>(dXc, n, n, pb, h->dConstsLocal + h->c_XtX);
-  CUX(cudaGetLastError());
+  with_real(h, [&](auto r) { generate_data_kernel<decltype(r)><<<h->sm_count * 8, 256, 0, h->stream>>>(A); });
+  CUX(cudaMallocAsync((void**)&dpart, (size_t)3 * Jp * TILE_COLSUM_PARTS * sizeof(double), h->stream));
+  with_real(h, [&](auto r) {
+    using R = decltype(r);
+    tile_colsum_part_kernel<R><<<TILE_COLSUM_PARTS, Jp, 0, h->stream>>>(h->dY, has_rt ? (const R*)h->dLogT : nullptr, n, Jp, dpart);
+  });
+  const int rc = finish_ingest(h, X, ldX, false, dpart, TILE_COLSUM_PARTS);
   cleanup();
-  dbuf = dXc = dpart_alloc = nullptr;
-  tm.mark("generate: launches, X H2D");
-  CUX(cudaStreamSynchronize(h->stream));
-  tm.mark("generate: device work");
-#undef CUX
-  h->data_set = true;
-  h->consts_final = false;
-  return 0;
+  tm.mark("generate: launches, device work");
+  return rc;
 }
 
 // The data set held by the handle (ingested or generated), back in Julia's column-major Float64 (logT as stored: f32-rounded in f32 mode)
@@ -909,8 +902,10 @@ extern "C" int erirt_get_data(erirt_handle* h, double* Y, int64_t ldY, double* l
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
   }
   if (logT && e == cudaSuccess) {
-    if (h->cfg.dtype == ERIRT_F32) tile_to_colmajor_kernel<float><<<1024, 256, 0, h->stream>>>((const float*)h->dLogT, n, J, Jp, tmp);
-    else tile_to_colmajor_kernel<double><<<1024, 256, 0, h->stream>>>((const double*)h->dLogT, n, J, Jp, tmp);
+    with_real(h, [&](auto r) {
+      using R = decltype(r);
+      tile_to_colmajor_kernel<R><<<1024, 256, 0, h->stream>>>((const R*)h->dLogT, n, J, Jp, tmp);
+    });
     e = cudaMemcpy2DAsync(logT, ldT * sizeof(double), tmp, n * sizeof(double), n * sizeof(double), J, cudaMemcpyDeviceToHost, h->stream);
   }
   cudaFreeAsync(tmp, h->stream);
@@ -964,13 +959,19 @@ static int finalize_constants(erirt_handle* h) {
 // ------------------------------------------------------------------------------------------------
 // state
 // ------------------------------------------------------------------------------------------------
-static int person_vec(erirt_handle* h, int field, void** p) {
+// Device storage [n_subj][Jp] of R of a person field, seen by the caller as column-major [n_subj][J] float64: the person vectors
+// theta / zeta / nu are J = Jp = 1; omega and the N x J nu of CrossQr are the tiles.  CrossQr's nu is drawn before it is read (no
+// initial value is needed); setting it serves erirt_loglik_current (D-hat at Post.mean, GibbsRtIrtCross.pl.jl:344-352)
+struct PersonField { void* p; int J, Jp; };
+static bool person_field(const erirt_handle* h, int field, PersonField* f) {
+  const int J = h->cfg.n_item, Jp = h->L.Jp;
   switch (field) {
-    case ERIRT_THETA: *p = h->dTheta; return 0;
-    case ERIRT_ZETA: *p = h->dZeta; return 0;
-    case ERIRT_NU: *p = h->dNu; return 0;
+    case ERIRT_THETA: *f = {h->dTheta, 1, 1}; return true;
+    case ERIRT_ZETA: *f = {h->dZeta, 1, 1}; return true;
+    case ERIRT_NU: *f = h->cfg.model == ERIRT_RTIRT_CROSSQR ? PersonField{h->dNuCell, J, Jp} : PersonField{h->dNu, 1, 1}; return true;
+    case ERIRT_OMEGA: *f = {h->dOmega, J, Jp}; return true;
   }
-  return -1;
+  return false;
 }
 static int param_slot(erirt_handle* h, int field, int* off, int* len) {
   const Layout& L = h->L;
@@ -990,32 +991,18 @@ static int param_slot(erirt_handle* h, int field, int* off, int* len) {
 extern "C" int erirt_set_state(erirt_handle* h, int32_t field, const double* v, int64_t n) {
   if (!h || !v) return fail(ERIRT_E_ARG, "null argument");
   CU(cudaSetDevice(h->cfg.device));
-  void* pv;
+  PersonField pf;
   int off, len;
-  // CrossQr: nu is N x J.  The sampler draws it before reading it (no initial value is needed); setting it serves
-  // erirt_loglik_current (D-hat at Post.mean, GibbsRtIrtCross.pl.jl:344-352)
-  const bool nu_cell = field == ERIRT_NU && h->cfg.model == ERIRT_RTIRT_CROSSQR;
-  if (!nu_cell && person_vec(h, field, &pv) == 0) {
-    if (n != h->cfg.n_subj) return fail(ERIRT_E_ARG, "field %d expects %lld values, got %lld", field, (long long)h->cfg.n_subj, (long long)n);
-    double* tmp;
-    CU(cudaMallocAsync((void**)&tmp, n * sizeof(double), h->stream));
-    cudaMemcpyAsync(tmp, v, n * sizeof(double), cudaMemcpyHostToDevice, h->stream);
-    if (h->cfg.dtype == ERIRT_F32) pack_vec_kernel<float><<<256, 256, 0, h->stream>>>(tmp, n, (float*)pv);
-    else pack_vec_kernel<double><<<256, 256, 0, h->stream>>>(tmp, n, (double*)pv);
-    cudaFreeAsync(tmp, h->stream);
-    cudaError_t e = cudaStreamSynchronize(h->stream);
-    if (e != cudaSuccess) return fail(ERIRT_E_CUDA, "set_state: %s", cudaGetErrorString(e));
-    return 0;
-  }
-  if (field == ERIRT_OMEGA || nu_cell) {
-    const int64_t want = h->cfg.n_subj * h->cfg.n_item;
+  if (person_field(h, field, &pf)) {
+    const int64_t want = h->cfg.n_subj * pf.J;
     if (n != want) return fail(ERIRT_E_ARG, "field %d expects %lld values, got %lld", field, (long long)want, (long long)n);
-    void* dst = nu_cell ? h->dNuCell : h->dOmega;
     double* tmp;
     CU(cudaMallocAsync((void**)&tmp, n * sizeof(double), h->stream));
     cudaMemcpyAsync(tmp, v, n * sizeof(double), cudaMemcpyHostToDevice, h->stream);
-    if (h->cfg.dtype == ERIRT_F32) colmajor_to_tile_kernel<float><<<1024, 256, 0, h->stream>>>(tmp, h->cfg.n_subj, h->cfg.n_item, h->L.Jp, (float*)dst);
-    else colmajor_to_tile_kernel<double><<<1024, 256, 0, h->stream>>>(tmp, h->cfg.n_subj, h->cfg.n_item, h->L.Jp, (double*)dst);
+    with_real(h, [&](auto r) {
+      using R = decltype(r);
+      colmajor_to_tile_kernel<R><<<1024, 256, 0, h->stream>>>(tmp, h->cfg.n_subj, pf.J, pf.Jp, (R*)pf.p);
+    });
     cudaFreeAsync(tmp, h->stream);
     cudaError_t e = cudaStreamSynchronize(h->stream);
     if (e != cudaSuccess) return fail(ERIRT_E_CUDA, "set_state: %s", cudaGetErrorString(e));
@@ -1032,23 +1019,17 @@ extern "C" int erirt_set_state(erirt_handle* h, int32_t field, const double* v, 
 extern "C" int erirt_get_state(erirt_handle* h, int32_t field, double* out, int64_t n) {
   if (!h || !out) return fail(ERIRT_E_ARG, "null argument");
   CU(cudaSetDevice(h->cfg.device));
-  void* pv;
+  PersonField pf;
   int off, len;
-  const bool nu_cell = field == ERIRT_NU && h->cfg.model == ERIRT_RTIRT_CROSSQR;
-  if (person_vec(h, field, &pv) == 0 || field == ERIRT_OMEGA) {
-    const bool om = field == ERIRT_OMEGA || nu_cell;
-    const void* tile_src = nu_cell ? h->dNuCell : h->dOmega;
-    const int64_t want = om ? h->cfg.n_subj * h->cfg.n_item : h->cfg.n_subj;
+  if (person_field(h, field, &pf)) {
+    const int64_t want = h->cfg.n_subj * pf.J;
     if (n != want) return fail(ERIRT_E_ARG, "field %d expects %lld values, got %lld", field, (long long)want, (long long)n);
     double* tmp;
     CU(cudaMallocAsync((void**)&tmp, n * sizeof(double), h->stream));
-    if (om) {
-      if (h->cfg.dtype == ERIRT_F32) tile_to_colmajor_kernel<float><<<1024, 256, 0, h->stream>>>((const float*)tile_src, h->cfg.n_subj, h->cfg.n_item, h->L.Jp, tmp);
-      else tile_to_colmajor_kernel<double><<<1024, 256, 0, h->stream>>>((const double*)tile_src, h->cfg.n_subj, h->cfg.n_item, h->L.Jp, tmp);
-    } else {
-      if (h->cfg.dtype == ERIRT_F32) unpack_vec_kernel<float><<<256, 256, 0, h->stream>>>((const float*)pv, n, tmp);
-      else unpack_vec_kernel<double><<<256, 256, 0, h->stream>>>((const double*)pv, n, tmp);
-    }
+    with_real(h, [&](auto r) {
+      using R = decltype(r);
+      tile_to_colmajor_kernel<R><<<1024, 256, 0, h->stream>>>((const R*)pf.p, h->cfg.n_subj, pf.J, pf.Jp, tmp);
+    });
     cudaMemcpyAsync(out, tmp, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
     cudaFreeAsync(tmp, h->stream);
     cudaError_t e = cudaStreamSynchronize(h->stream);
@@ -1096,11 +1077,10 @@ static PersonArgs<R> make_person_args(erirt_handle* h, int stage) {
   A.model = h->cfg.model;
   A.n_chain = h->cfg.n_chain;
   A.n_burnin = h->cfg.n_burnin;
-  const double q = h->cfg.q_rt;
-  A.k1 = (1.0 - 2.0 * q) / (q * (1.0 - q));
-  A.k2 = 2.0 / (q * (1.0 - q));
-  A.key = make_key(h->cfg.seed, h->cfg.chain);
-  A.sched = make_sched(A.key);
+  A.k1 = h->k1;
+  A.k2 = h->k2;
+  A.key = h->key;
+  A.sched = make_sched(h->key);
   return A;
 }
 
@@ -1141,10 +1121,9 @@ static GlobalArgs make_global_args(erirt_handle* h, int stage) {
   A.cov2one = h->cfg.cov2one;
   A.compat = h->cfg.compat;
   A.kz_from_stats = runs_fast_kernel(h, stage) ? 1 : 0;
-  const double q = h->cfg.q_rt;
-  A.k1 = (1.0 - 2.0 * q) / (q * (1.0 - q));
-  A.k2 = 2.0 / (q * (1.0 - q));
-  A.key = make_key(h->cfg.seed, h->cfg.chain);
+  A.k1 = h->k1;
+  A.k2 = h->k2;
+  A.key = h->key;
   A.peer_bufs = h->peer_ready ? h->dPeerBufs : nullptr;
   A.xseq = h->dXseq;
   A.world = h->world;
@@ -1172,16 +1151,12 @@ static cudaError_t launch_chain_kernel(const void* kfn, dim3 grid, dim3 block, v
 
 static int launch_person(erirt_handle* h, int stage) {
   const void* kfn = person_kernel_for(h, stage);
-  if (h->cfg.dtype == ERIRT_F32) {
-    PersonArgs<float> A = make_person_args<float>(h, stage);
+  return with_real(h, [&](auto r) -> int {
+    PersonArgs<decltype(r)> A = make_person_args<decltype(r)>(h, stage);
     void* args[] = {&A};
     CU(launch_chain_kernel(kfn, dim3(stage == 0 ? h->grid : h->grid_gen), dim3(CTA_THREADS), args, A.S.total, h->stream));
-  } else {
-    PersonArgs<double> A = make_person_args<double>(h, stage);
-    void* args[] = {&A};
-    CU(launch_chain_kernel(kfn, dim3(stage == 0 ? h->grid : h->grid_gen), dim3(CTA_THREADS), args, A.S.total, h->stream));
-  }
-  return 0;
+    return 0;
+  });
 }
 static int launch_global(erirt_handle* h, int stage) {
   if (h->world > 1 && !h->peer_ready && !h->comm)
@@ -1330,23 +1305,54 @@ __global__ void trace_gather_kernel(double* __restrict__ dst, int64_t n_iter, in
   }
 }
 
-extern "C" int erirt_get_trace(erirt_handle* h, int32_t which, int64_t first_col, int64_t n_cols, double* out) {
-  if (!h || !out) return fail(ERIRT_E_ARG, "null argument");
+// Where the columns of trace `which` come from: columns [small0, small0 + small_w) from the sweep-major trace small [s][small_w],
+// columns [pcol0, pcol0 + pn) from field pfield of the person trace (pn = 0: the trace has no person columns).
+struct TraceSource {
+  const double* small;
+  int64_t small0, small_w;
+  int pfield;
+  int64_t pcol0, pn;
+  bool person_cols;  // [first_col, first_col + n_cols) includes person columns
+};
+// Checks [first_col, first_col + n_cols) against the trace's width and resolves `which`.  Whether person columns may be read without
+// a person trace is each caller's rule: erirt_get_trace refuses them only once a sweep has run (before that every value it returns
+// is NaN), erirt_trace_ess_rhat refuses them always.
+static int trace_source(const erirt_handle* h, int which, int64_t first_col, int64_t n_cols, TraceSource* src) {
   const int64_t W = full_width(h, which);
   if (W <= 0) return fail(ERIRT_E_ARG, "trace %d does not exist for this model", which);
   if (first_col < 0 || n_cols < 0 || first_col + n_cols > W) return fail(ERIRT_E_ARG, "columns [%lld,%lld) outside [0,%lld)", (long long)first_col, (long long)(first_col + n_cols), (long long)W);
-  CU(cudaSetDevice(h->cfg.device));
-  const int64_t N = h->cfg.n_subj, J = h->cfg.n_item, nIter = h->cfg.n_iter, nChain = h->cfg.n_chain;
-  const int64_t done = h->sweeps_done;
+  const int64_t N = h->cfg.n_subj, J = h->cfg.n_item;
   // column ranges: person block [0,N) for ra/rt, trailing nu block for LatentQr qr
-  int pfield = -1;
-  int64_t pcol0 = 0, small0 = 0, small_w = 0;
-  const double* dsmall = nullptr;
-  if (which == ERIRT_TRACE_RA) { pfield = 0; small0 = N; dsmall = h->dTrRa; small_w = 2 * J; }
-  else if (which == ERIRT_TRACE_RT) { pfield = 1; small0 = N; dsmall = h->dTrRt; small_w = 2 * J; }
-  else if (which == ERIRT_TRACE_QR) { dsmall = h->dTrQr; small_w = h->qw; if (h->cfg.model == ERIRT_RTIRT_LATENTQR) { pfield = 2; pcol0 = h->qw; } }
-  else { dsmall = h->dTrLl; small_w = 1; }
-  if (pfield >= 0 && first_col < pcol0 + N && first_col + n_cols > pcol0 && done > 0 && !h->dPtrace)
+  TraceSource s{nullptr, 0, 0, 0, -1, 0, false};
+  if (which == ERIRT_TRACE_RA) { s.small = h->dTrRa; s.small0 = N; s.small_w = 2 * J; s.pfield = 0; s.pcol0 = 0; s.pn = N; }
+  else if (which == ERIRT_TRACE_RT) { s.small = h->dTrRt; s.small0 = N; s.small_w = 2 * J; s.pfield = 1; s.pcol0 = 0; s.pn = N; }
+  else if (which == ERIRT_TRACE_QR) {
+    s.small = h->dTrQr; s.small_w = h->qw;
+    if (h->cfg.model == ERIRT_RTIRT_LATENTQR) { s.pfield = 2; s.pcol0 = h->qw; s.pn = N; }
+  } else { s.small = h->dTrLl; s.small_w = 1; }
+  s.person_cols = first_col < s.pcol0 + s.pn && first_col + n_cols > s.pcol0;
+  *src = s;
+  return 0;
+}
+
+// Columns [col0, col0 + nc) of chain l into dst [nc][n_iter] (trace_gather_kernel)
+static void gather_trace(erirt_handle* h, const TraceSource& s, double* dst, int64_t col0, int64_t nc, int64_t l) {
+  const int64_t nIter = h->cfg.n_iter;
+  const int grid = (int)std::min<int64_t>((nIter * nc + 255) / 256, (int64_t)h->sm_count * 16);
+  with_real(h, [&](auto r) {
+    using R = decltype(r);
+    trace_gather_kernel<R><<<grid, 256, 0, h->stream>>>(dst, nIter, nc, col0, l, h->cfg.n_chain, h->sweeps_done, s.small, s.small0, s.small_w,
+                                                         (const R*)h->dPtrace, s.pfield, s.pcol0, s.pn, h->n_pad);
+  });
+}
+
+extern "C" int erirt_get_trace(erirt_handle* h, int32_t which, int64_t first_col, int64_t n_cols, double* out) {
+  if (!h || !out) return fail(ERIRT_E_ARG, "null argument");
+  TraceSource src;
+  if (int rc = trace_source(h, which, first_col, n_cols, &src)) return rc;
+  CU(cudaSetDevice(h->cfg.device));
+  const int64_t nIter = h->cfg.n_iter, nChain = h->cfg.n_chain;
+  if (src.person_cols && h->sweeps_done > 0 && !h->dPtrace)
     return fail(ERIRT_E_STATE, "person columns requested but person_trace = 0 (use erirt_get_moments)");
   if (n_cols == 0) return 0;
   // assembled on the device in column chunks of <= 64 MB per chain (Julia's layout makes such a chunk contiguous in `out`), one D2H copy each
@@ -1357,13 +1363,7 @@ extern "C" int erirt_get_trace(erirt_handle* h, int32_t which, int64_t first_col
   for (int64_t l = 0; l < nChain && e == cudaSuccess; ++l)
     for (int64_t c0 = 0; c0 < n_cols && e == cudaSuccess; c0 += chunk_cols) {
       const int64_t nc = std::min(chunk_cols, n_cols - c0);
-      const int grid = (int)std::min<int64_t>((nIter * nc + 255) / 256, (int64_t)h->sm_count * 16);
-      if (h->rsz == 4)
-        trace_gather_kernel<float><<<grid, 256, 0, h->stream>>>(tmp, nIter, nc, first_col + c0, l, nChain, done, dsmall, small0, small_w,
-                                                                (const float*)h->dPtrace, pfield < 0 ? 0 : pfield, pfield < 0 ? -1 : pcol0, pfield < 0 ? 0 : N, h->n_pad);
-      else
-        trace_gather_kernel<double><<<grid, 256, 0, h->stream>>>(tmp, nIter, nc, first_col + c0, l, nChain, done, dsmall, small0, small_w,
-                                                                 (const double*)h->dPtrace, pfield < 0 ? 0 : pfield, pfield < 0 ? -1 : pcol0, pfield < 0 ? 0 : N, h->n_pad);
+      gather_trace(h, src, tmp, first_col + c0, nc, l);
       e = cudaMemcpyAsync(out + nIter * (c0 + n_cols * l), tmp, (size_t)nIter * nc * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
       if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);  // tmp is reused by the next chunk
     }
@@ -1431,23 +1431,14 @@ extern "C" int erirt_ess_rhat(const double* x, int64_t n_iter, int64_t n_cols, i
 
 extern "C" int erirt_trace_ess_rhat(erirt_handle* h, int32_t which, int64_t first_col, int64_t n_cols, int64_t skip, double* ess, double* rhat) {
   if (!h || !ess || !rhat) return fail(ERIRT_E_ARG, "null argument");
-  const int64_t W = full_width(h, which);
-  if (W <= 0) return fail(ERIRT_E_ARG, "trace %d does not exist for this model", which);
-  if (first_col < 0 || n_cols < 0 || first_col + n_cols > W) return fail(ERIRT_E_ARG, "columns [%lld,%lld) outside [0,%lld)", (long long)first_col, (long long)(first_col + n_cols), (long long)W);
+  TraceSource src;
+  if (int rc = trace_source(h, which, first_col, n_cols, &src)) return rc;
   CU(cudaSetDevice(h->cfg.device));
-  const int64_t N = h->cfg.n_subj, J = h->cfg.n_item, nIter = h->cfg.n_iter, nChain = h->cfg.n_chain;
-  const int64_t done = h->sweeps_done, done_iter = done / nChain;  // complete iterations (every chain has drawn)
+  const int64_t nIter = h->cfg.n_iter, nChain = h->cfg.n_chain;
+  const int64_t done_iter = h->sweeps_done / nChain;  // complete iterations (every chain has drawn)
   if (nChain > 32) return fail(ERIRT_E_ARG, "ess_rhat: at most 32 chains");
   if (skip < 0 || skip > done_iter) return fail(ERIRT_E_ARG, "skip %lld outside [0, %lld] completed iterations", (long long)skip, (long long)done_iter);
-  int pfield = -1;
-  int64_t pcol0 = 0, small0 = 0, small_w = 0;
-  const double* dsmall = nullptr;
-  if (which == ERIRT_TRACE_RA) { pfield = 0; small0 = N; dsmall = h->dTrRa; small_w = 2 * J; }
-  else if (which == ERIRT_TRACE_RT) { pfield = 1; small0 = N; dsmall = h->dTrRt; small_w = 2 * J; }
-  else if (which == ERIRT_TRACE_QR) { dsmall = h->dTrQr; small_w = h->qw; if (h->cfg.model == ERIRT_RTIRT_LATENTQR) { pfield = 2; pcol0 = h->qw; } }
-  else { dsmall = h->dTrLl; small_w = 1; }
-  if (pfield >= 0 && first_col < pcol0 + N && first_col + n_cols > pcol0 && !h->dPtrace)
-    return fail(ERIRT_E_STATE, "person columns requested but person_trace = 0");
+  if (src.person_cols && !h->dPtrace) return fail(ERIRT_E_STATE, "person columns requested but person_trace = 0");
   if (n_cols == 0) return 0;
   // the columns are gathered into [chain][column][iteration] in chunks of <= 256 MB and never leave the device
   const int64_t chunk_cols = std::max<int64_t>(1, std::min<int64_t>(n_cols, ((int64_t)256 << 20) / (nIter * nChain * (int64_t)sizeof(double))));
@@ -1456,15 +1447,7 @@ extern "C" int erirt_trace_ess_rhat(erirt_handle* h, int32_t which, int64_t firs
   int rc = 0;
   for (int64_t c0 = 0; c0 < n_cols && rc == 0; c0 += chunk_cols) {
     const int64_t nc = std::min(chunk_cols, n_cols - c0);
-    const int grid = (int)std::min<int64_t>((nIter * nc + 255) / 256, (int64_t)h->sm_count * 16);
-    for (int64_t l = 0; l < nChain; ++l) {
-      if (h->rsz == 4)
-        trace_gather_kernel<float><<<grid, 256, 0, h->stream>>>(tmp + nIter * nc * l, nIter, nc, first_col + c0, l, nChain, done, dsmall, small0, small_w,
-                                                                (const float*)h->dPtrace, pfield < 0 ? 0 : pfield, pfield < 0 ? -1 : pcol0, pfield < 0 ? 0 : N, h->n_pad);
-      else
-        trace_gather_kernel<double><<<grid, 256, 0, h->stream>>>(tmp + nIter * nc * l, nIter, nc, first_col + c0, l, nChain, done, dsmall, small0, small_w,
-                                                                 (const double*)h->dPtrace, pfield < 0 ? 0 : pfield, pfield < 0 ? -1 : pcol0, pfield < 0 ? 0 : N, h->n_pad);
-    }
+    for (int64_t l = 0; l < nChain; ++l) gather_trace(h, src, tmp + nIter * nc * l, first_col + c0, nc, l);
     rc = run_ess_rhat(tmp, nIter, nc, nChain, skip, done_iter - skip, h->stream, ess + c0, rhat + c0);
   }
   cudaFreeAsync(tmp, h->stream);
@@ -1478,27 +1461,20 @@ extern "C" int erirt_get_moments(erirt_handle* h, int32_t field, double* mean, d
   if (slot < 0) return fail(ERIRT_E_ARG, "moments exist for THETA, ZETA and NU only");
   const bool nu_cell = field == ERIRT_NU && h->cfg.model == ERIRT_RTIRT_CROSSQR;
   if (nu_cell && !h->dNuMom) return fail(ERIRT_E_STATE, "the running moments of the N x J weights of CrossQr need erirt_config.nu_cell_moments = 1");
-  if (n != (nu_cell ? h->cfg.n_subj * h->cfg.n_item : h->cfg.n_subj)) return fail(ERIRT_E_ARG, nu_cell ? "expects n_subj * n_item values" : "expects n_subj values");
+  PersonField pf;
+  person_field(h, field, &pf);
+  if (n != h->cfg.n_subj * pf.J) return fail(ERIRT_E_ARG, nu_cell ? "expects n_subj * n_item values" : "expects n_subj values");
   CU(cudaSetDevice(h->cfg.device));
   CU(cudaStreamSynchronize(h->stream));
   const int64_t nChain = h->cfg.n_chain;
   const int64_t first = (int64_t)h->cfg.n_burnin * nChain;  // sweeps with m > n_burnin
   const int64_t cnt = h->sweeps_done > first ? h->sweeps_done - first : 0;
-  if (nu_cell) {  // column-major N x J out of the tiled sums
-    double* tmp = nullptr;
-    CU(cudaMallocAsync((void**)&tmp, (size_t)2 * n * sizeof(double), h->stream));
-    tile_moments_kernel<<<1024, 256, 0, h->stream>>>(h->dNuMom, h->dNuMom + (size_t)h->n_pad * h->L.Jp, h->cfg.n_subj, h->cfg.n_item, h->L.Jp, (double)cnt, tmp, tmp + n);
-    cudaError_t e = cudaMemcpyAsync(mean, tmp, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess && sd) e = cudaMemcpyAsync(sd, tmp + n, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-    cudaFreeAsync(tmp, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    if (e != cudaSuccess) return fail(ERIRT_E_CUDA, "get_moments: %s", cudaGetErrorString(e));
-    return 0;
-  }
+  // running sum and sum of squares of the field, laid out like it: [2][n_pad][Jp]
+  const double* s1 = nu_cell ? h->dNuMom : h->dMom + (size_t)(2 * slot) * h->n_pad;
   // mean and SD are finished on the device and copied straight into the caller's buffers (pinned buffers make this a plain DMA)
   double* tmp = nullptr;
   CU(cudaMallocAsync((void**)&tmp, (size_t)2 * n * sizeof(double), h->stream));
-  moments_finish_kernel<<<592, 256, 0, h->stream>>>(h->dMom + (size_t)(2 * slot) * h->n_pad, h->dMom + (size_t)(2 * slot + 1) * h->n_pad, n, (double)cnt, tmp, tmp + n);
+  tile_moments_kernel<<<1024, 256, 0, h->stream>>>(s1, s1 + (size_t)h->n_pad * pf.Jp, h->cfg.n_subj, pf.J, pf.Jp, (double)cnt, tmp, tmp + n);
   cudaError_t e = cudaMemcpyAsync(mean, tmp, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
   if (e == cudaSuccess && sd) e = cudaMemcpyAsync(sd, tmp + n, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
   cudaFreeAsync(tmp, h->stream);
@@ -1796,58 +1772,42 @@ extern "C" int erirt_peer_detach(erirt_handle* h) {
 // ------------------------------------------------------------------------------------------------
 // parity entry points
 // ------------------------------------------------------------------------------------------------
-static int pick_device(int device) {
-  int ndev = 0;
-  cudaError_t e = cudaGetDeviceCount(&ndev);
-  if (e != cudaSuccess || ndev == 0) return fail(ERIRT_E_CUDA, "no CUDA device available (%s); this engine has no CPU fallback", cudaGetErrorString(e));
-  if (device < 0 || device >= ndev) return fail(ERIRT_E_ARG, "device out of range");
-  CU(cudaSetDevice(device));
+// n float64 inputs to the device, `launch(grid, din, dout)` enqueues the kernel on the default stream, n float64 results back
+template <typename Launch>
+static int run_parity_kernel(const char* name, int32_t device, const double* in, int64_t n, double* out, Launch launch) {
+  if (int rc = pick_device(device)) return rc;
+  if (n == 0) return 0;
+  double *din = nullptr, *dout = nullptr;
+  CU(cudaMalloc((void**)&din, n * sizeof(double)));
+  CU(cudaMalloc((void**)&dout, n * sizeof(double)));
+  CU(cudaMemcpy(din, in, n * sizeof(double), cudaMemcpyHostToDevice));
+  launch((int)std::min<int64_t>((n + 255) / 256, 148 * 8), din, dout);
+  cudaError_t e = cudaDeviceSynchronize();
+  if (e == cudaSuccess) e = cudaMemcpy(out, dout, n * sizeof(double), cudaMemcpyDeviceToHost);
+  cudaFree(din);
+  cudaFree(dout);
+  if (e != cudaSuccess) return fail(ERIRT_E_CUDA, "%s: %s", name, cudaGetErrorString(e));
   return 0;
 }
 
 extern "C" int erirt_k_pg(const double* z, int64_t rows, int32_t cols, int64_t row0, uint64_t seed, uint32_t chain,
                           uint32_t sweep, int32_t dtype, int32_t device, double* out) {
   if (!z || !out || rows < 0 || cols < 1) return fail(ERIRT_E_ARG, "bad argument");
-  int rc = pick_device(device);
-  if (rc) return rc;
-  const int64_t n = rows * cols;
-  if (n == 0) return 0;
-  double *dz = nullptr, *dout = nullptr;
-  CU(cudaMalloc((void**)&dz, n * sizeof(double)));
-  CU(cudaMalloc((void**)&dout, n * sizeof(double)));
-  CU(cudaMemcpy(dz, z, n * sizeof(double), cudaMemcpyHostToDevice));
   const PhiloxKey key = make_key(seed, chain);
-  const int grid = (int)std::min<int64_t>((n + 255) / 256, 148 * 8);
-  if (dtype == ERIRT_F32) k_pg_fast_kernel<<<grid, 256>>>(dz, rows, cols, row0, key, sweep, dout);
-  else k_pg_kernel<double><<<grid, 256>>>(dz, rows, cols, row0, key, sweep, dout);
-  cudaError_t e = cudaDeviceSynchronize();
-  if (e == cudaSuccess) e = cudaMemcpy(out, dout, n * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(dz);
-  cudaFree(dout);
-  if (e != cudaSuccess) return fail(ERIRT_E_CUDA, "erirt_k_pg: %s", cudaGetErrorString(e));
-  return 0;
+  return run_parity_kernel("erirt_k_pg", device, z, rows * cols, out, [&](int grid, const double* dz, double* dout) {
+    if (dtype == ERIRT_F32) k_pg_fast_kernel<<<grid, 256>>>(dz, rows, cols, row0, key, sweep, dout);
+    else k_pg_kernel<double><<<grid, 256>>>(dz, rows, cols, row0, key, sweep, dout);
+  });
 }
 
 extern "C" int erirt_k_nu_person(const double* mu, double lam, int64_t n, int64_t row0, uint64_t seed, uint32_t chain,
                                  uint32_t sweep, int32_t dtype, int32_t device, double* out) {
   if (!mu || !out || n < 0) return fail(ERIRT_E_ARG, "bad argument");
-  int rc = pick_device(device);
-  if (rc) return rc;
-  if (n == 0) return 0;
-  double *dm = nullptr, *dout = nullptr;
-  CU(cudaMalloc((void**)&dm, n * sizeof(double)));
-  CU(cudaMalloc((void**)&dout, n * sizeof(double)));
-  CU(cudaMemcpy(dm, mu, n * sizeof(double), cudaMemcpyHostToDevice));
   const PhiloxKey key = make_key(seed, chain);
-  const int grid = (int)std::min<int64_t>((n + 255) / 256, 148 * 8);
-  if (dtype == ERIRT_F32) k_nu_person_kernel<float><<<grid, 256>>>(dm, lam, n, row0, key, sweep, dout);
-  else k_nu_person_kernel<double><<<grid, 256>>>(dm, lam, n, row0, key, sweep, dout);
-  cudaError_t e = cudaDeviceSynchronize();
-  if (e == cudaSuccess) e = cudaMemcpy(out, dout, n * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(dm);
-  cudaFree(dout);
-  if (e != cudaSuccess) return fail(ERIRT_E_CUDA, "erirt_k_nu_person: %s", cudaGetErrorString(e));
-  return 0;
+  return run_parity_kernel("erirt_k_nu_person", device, mu, n, out, [&](int grid, const double* dm, double* dout) {
+    if (dtype == ERIRT_F32) k_nu_person_kernel<float><<<grid, 256>>>(dm, lam, n, row0, key, sweep, dout);
+    else k_nu_person_kernel<double><<<grid, 256>>>(dm, lam, n, row0, key, sweep, dout);
+  });
 }
 
 extern "C" int erirt_k_philox(const uint32_t ctr[4], const uint32_t key[2], int32_t device, uint32_t out[4]) {
