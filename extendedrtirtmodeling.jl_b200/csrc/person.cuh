@@ -137,6 +137,137 @@ constexpr int min_ctas_f64() {
   return TPP >= 8 ? 4 : 3;
 }
 
+// ---------------- per-person conditionals, shared by person_sweep_kernel and person_sweep_fast_kernel ----------------
+// The callers differ only in their inputs; every expression keeps the operand order and association of the sampler it states.
+
+// quantile weights are kept in [1e-10, 1e10]
+template <typename R>
+__device__ __forceinline__ R clamp_nu(R x) {
+  return x < R(1e-10) ? R(1e-10) : (x > R(1e10) ? R(1e10) : x);
+}
+
+// theta_k from the row sums sum a^2 omega, sum a^2 b omega, sum a kappa (drawSubjAbility / ...Null, Draw.pl.jl:49-80)
+template <typename R>
+__device__ __forceinline__ R theta_draw(int model, R xb1, R S11, R d_a2, R d_ab, R d_ak, R zn) {
+  const R mu0 = (model == M_MLIRT || model == M_RTIRT) ? xb1 : R(0);
+  const R var0 = (model == M_MLIRT) ? R(1) : S11;
+  const R iv0 = rdiv(R(1), var0);
+  const R parV = rdiv(R(1), iv0 + d_a2);
+  const R parM = parV * (mu0 * iv0 + d_ak + d_ab);
+  return parM + sqrt_of(parV) * zn;
+}
+
+// prior mean and variance of zeta_k given theta_k and nu_k (Draw.pl.jl:119-174); mu = 0, var = 1 for MlIrt, which has no zeta.
+// has_rt, latent and qr are the kernel's flags of `model`: derived here again, they cost the Float64 kernel two selects.
+template <typename R>
+__device__ __forceinline__ void zeta_prior(int model, bool has_rt, bool latent, bool qr, R th, R nu, R xb1, R xb2, R beta_th, R S22, R k1,
+                                           R k2, R& mu, R& var) {
+  mu = R(0);
+  var = R(1);
+  if (has_rt) {
+    if (model == M_RTIRT) { mu = xb2; var = S22; }
+    else if (latent) {
+      mu = fma(th, beta_th, xb1);
+      var = S22;
+      if (qr) { mu = fma(k1, nu, mu); var = S22 * (k2 * nu); }
+    } else if (model == M_NULL) { mu = R(0); var = R(1); }  // Draw.pl.jl:120-121
+    else { mu = R(0); var = S22; }
+  }
+}
+
+// zeta_k from its prior and the likelihood's precision and numerator (the row sums of the model's response-time part)
+template <typename R>
+__device__ __forceinline__ R zeta_draw(R mu_z, R var_z, R prec, R num, R zn) {
+  const R ivz = rdiv(R(1), var_z);
+  const R parV = rdiv(R(1), ivz + prec);
+  const R parM = parV * (mu_z * ivz + num);
+  return parM + sqrt_of(parV) * zn;
+}
+
+// structural log-density of (theta_k, zeta_k) (getLogLikelihood*, GibbsRtIrt.pl.jl:195-272)
+template <typename R>
+__device__ __forceinline__ R struct_log_density(int model, R th, R ze, R xb1, R xb2, R mu_z, R var_z, R S11, R S12, R S22) {
+  const R LOG2PI = R(1.8378770664093454835606594728112);
+  if (model == M_MLIRT) {
+    const R r = th - xb1;
+    return R(-0.5) * LOG2PI - R(0.5) * r * r;
+  } else if (model == M_LATENT || model == M_LATENTQR) {
+    const R r = ze - mu_z;
+    return R(-0.5) * (LOG2PI + rlog(var_z)) - R(0.5) * r * rdiv(r, var_z);
+  } else {
+    const R e1 = th - (model == M_RTIRT ? xb1 : R(0));
+    const R e2 = ze - (model == M_RTIRT ? xb2 : R(0));
+    const R det = S11 * S22 - S12 * S12;
+    return -LOG2PI - R(0.5) * rlog(det) - R(0.5) * rdiv(S22 * e1 * e1 - R(2) * S12 * e1 * e2 + S11 * e2 * e2, det);
+  }
+}
+
+// running moments (post burn-in) and the person trace of row pi at sweep k
+template <typename R>
+__device__ __forceinline__ void record_person(const PersonArgs<R>& A, int64_t pi, uint32_t k, bool moments, bool trace, bool has_rt, bool qr,
+                                              R th, R ze, R nu) {
+  if (moments) {
+    double* m = A.mom + pi;  // fire-and-forget reductions (RED.ADD.F64): no round trip on the critical path
+    atomicAdd(&m[0], (double)th);
+    atomicAdd(&m[A.n_pad], (double)th * (double)th);
+    if (has_rt) {
+      atomicAdd(&m[2 * A.n_pad], (double)ze);
+      atomicAdd(&m[3 * A.n_pad], (double)ze * (double)ze);
+    }
+    if (qr) {
+      atomicAdd(&m[4 * A.n_pad], (double)nu);
+      atomicAdd(&m[5 * A.n_pad], (double)nu * (double)nu);
+    }
+  }
+  if (trace) {
+    R* t = A.ptrace + ((int64_t)(k - 1) * 3) * A.n_pad + pi;
+    t[0] = th;
+    t[A.n_pad] = ze;
+    t[2 * A.n_pad] = nu;
+  }
+}
+
+// nu_{k+1} | zeta_k, theta_k, beta_k, Sigma_k (LatentQr, drawQrWeightsLatentQr, Draw.pl.jl:325-343)
+template <typename R>
+__device__ __forceinline__ R draw_nu_person(R th, R ze, R xb1, R beta_th, R S22, R k1, R k2, R zn, R un) {
+  const R xb = fma(th, beta_th, xb1);
+  const R isc = rdiv(R(1), sqrt_of(S22 * k2));
+  const R parA = fabs(ze - xb) * isc;
+  const R parB = sqrt_of(R(2) * k2 + k1 * k1) * isc;
+  R mu = rdiv(parB, parA);
+  if (!(mu >= R(1e-10))) mu = R(1e-10);
+  const R ig = ig_msh<R>(mu, parB * parB, zn, un);
+  return clamp_nu(rdiv(R(1), ig));
+}
+
+// the person's row u = [1 X theta zeta nu 1/nu] of the Gram (X is written in part 1); zero for a padding row
+template <typename R>
+__device__ __forceinline__ void write_u_row(R* u, bool pvalid, bool qr, int F, R th, R ze, R nu) {
+  u[0] = pvalid ? R(1) : R(0);
+  u[F + 1] = pvalid ? th : R(0);
+  u[F + 2] = pvalid ? ze : R(0);
+  u[F + 3] = (pvalid && qr) ? nu : R(0);
+  u[F + 4] = (pvalid && qr) ? rdiv(R(1), nu) : R(0);  // weight of the nu-weighted Gram
+}
+
+// end of the kernel, called by every thread once its shared-memory atomics on s_scal are issued: add the CTA's accumulators (n_blocks
+// per-item blocks, the Gram and, for LatentQr, its 1/nu-weighted twin, the scalars) to A.stats and let the last omega store drain.
+// J and Jp are the kernel's copies: read from A.L in here, the item loop is no longer unrolled.
+template <typename R>
+__device__ __forceinline__ void flush_to_stats(const PersonArgs<R>& A, int J, int Jp, const double* s_acc_item, int n_blocks,
+                                               const double* s_acc_gram, bool qr, const double* s_scal, int tid) {
+  const Layout& L = A.L;
+  __syncthreads();
+  for (int t = tid; t < n_blocks * Jp; t += CTA_THREADS) {
+    const int j = t % Jp;
+    if (j < J) atomicAdd(&A.stats[L.s_S0 + t], s_acc_item[t]);
+  }
+  for (int t = tid; t < 2 * L.ntri; t += CTA_THREADS)
+    if (t < L.ntri || qr) atomicAdd(&A.stats[L.s_gram + t], s_acc_gram[t]);
+  if (tid < SC_COUNT) atomicAdd(&A.stats[L.s_scal + tid], s_scal[tid]);
+  if (tid == 0) tma_store_wait_all();
+}
+
 // FAM = 0: the one-launch-per-sweep models (MlIrt, RtIrt, RtIrtNull, Latent, LatentQr) -- the hot configuration, with the
 // Cross-family / evaluation code compiled out; FAM = 1: everything (Cross, CrossQr stages 1/2, stage 3 evaluation).
 template <typename R, int TPP, int FAM>
@@ -389,94 +520,30 @@ __global__ void __launch_bounds__(CTA_THREADS, (sizeof(R) == 8 ? min_ctas_f64<TP
       // ---- person phase, part 2: theta_k, zeta_k, structural log-density, moments ----
       if (tid < P) {
         const R* d = s_sum + 4 * tid;
-        if (do_theta) {
-          const R mu0 = (model == M_MLIRT || model == M_RTIRT) ? xb1 : R(0);
-          const R var0 = (model == M_MLIRT) ? R(1) : S11;
-          const R iv0 = rdiv(R(1), var0);
-          const R parV = rdiv(R(1), iv0 + d[0]);
-          const R parM = parV * (mu0 * iv0 + d[2] + d[1]);
-          th = parM + sqrt_of(parV) * zn_theta;
-        }
-        R mu_z = R(0), var_z = R(1);
-        if (has_rt) {
-          if (model == M_RTIRT) { mu_z = xb2; var_z = S22; }
-          else if (latent) {
-            mu_z = fma(th, s_beta[F + 1], xb1);
-            var_z = S22;
-            if (qr) { mu_z = fma(k1, nu, mu_z); var_z = S22 * (k2 * nu); }
-          } else if (model == M_NULL) { mu_z = R(0); var_z = R(1); }  // Draw.pl.jl:120-121
-          else { mu_z = R(0); var_z = S22; }
-        }
+        if (do_theta) th = theta_draw(model, xb1, S11, d[0], d[1], d[2], zn_theta);
+        R mu_z, var_z;
+        zeta_prior(model, has_rt, latent, qr, th, nu, xb1, xb2, s_beta[F + 1], S22, k1, k2, mu_z, var_z);
         if (do_zeta) {
-          const R ivz = rdiv(R(1), var_z);
           // Cross: sum_j (lambda - logT - theta rho_j)/sigma2;  CrossQr: the same weighted by 1/(k2 nu_ij), plus k1 sum_j 1/(sigma2 k2)
           const R prec = cqr ? d[0] : sum_is2;
           const R num = cqr ? d[3] - th * d[1] + k1 * sum_is2 : (cross ? d[3] - th * sum_rho_is2 : d[3]);
-          const R parV = rdiv(R(1), ivz + prec);
-          const R parM = parV * (mu_z * ivz + num);
-          ze = parM + sqrt_of(parV) * zn_zeta;
+          ze = zeta_draw(mu_z, var_z, prec, num, zn_zeta);
         }
         if (pvalid && stage == 1) A.theta[pi] = th;  // K_a: theta_k only; everything else happens in K_b
         if (pvalid && stage != 1) {
-          const R LOG2PI = R(1.8378770664093454835606594728112);
-          R ls;
-          if (model == M_MLIRT) {
-            const R r = th - xb1;
-            ls = R(-0.5) * LOG2PI - R(0.5) * r * r;
-          } else if (latent) {
-            const R r = ze - mu_z;
-            ls = R(-0.5) * (LOG2PI + rlog(var_z)) - R(0.5) * r * rdiv(r, var_z);
-          } else {
-            const R e1 = th - (model == M_RTIRT ? xb1 : R(0));
-            const R e2 = ze - (model == M_RTIRT ? xb2 : R(0));
-            const R det = S11 * S22 - S12 * S12;
-            ls = -LOG2PI - R(0.5) * rlog(det) - R(0.5) * rdiv(S22 * e1 * e1 - R(2) * S12 * e1 * e2 + S11 * e2 * e2, det);
-          }
-          acc_ll_struct += (double)ls;
+          acc_ll_struct += (double)struct_log_density(model, th, ze, xb1, xb2, mu_z, var_z, S11, S12, S22);
           if (do_theta) A.theta[pi] = th;
           if (do_zeta) A.zeta[pi] = ze;
-          if (post_burnin && !eval) {
-            double* m = A.mom + pi;  // fire-and-forget reductions (RED.ADD.F64): no round trip on the critical path
-            atomicAdd(&m[0], (double)th);
-            atomicAdd(&m[A.n_pad], (double)th * (double)th);
-            if (has_rt) {
-              atomicAdd(&m[2 * A.n_pad], (double)ze);
-              atomicAdd(&m[3 * A.n_pad], (double)ze * (double)ze);
-            }
-            if (qr) {
-              atomicAdd(&m[4 * A.n_pad], (double)nu);
-              atomicAdd(&m[5 * A.n_pad], (double)nu * (double)nu);
-            }
-          }
-          if (A.ptrace && !eval) {
-            R* t = A.ptrace + ((int64_t)(k - 1) * 3) * A.n_pad + pi;
-            t[0] = th;
-            t[A.n_pad] = ze;
-            t[2 * A.n_pad] = nu;
-          }
+          record_person(A, pi, k, post_burnin && !eval, A.ptrace && !eval, has_rt, qr, th, ze, nu);
         }
       }
     }
     if (tid < P) {
-      // ---- nu_{k+1} (LatentQr), Draw.pl.jl:325-343 ----
       if (qr && !eval) {
-        const R xb = fma(th, s_beta[F + 1], xb1);
-        const R isc = rdiv(R(1), sqrt_of(S22 * k2));
-        const R parA = fabs(ze - xb) * isc;
-        const R parB = sqrt_of(R(2) * k2 + k1 * k1) * isc;
-        R mu = rdiv(parB, parA);
-        if (!(mu >= R(1e-10))) mu = R(1e-10);
-        const R ig = ig_msh<R>(mu, parB * parB, zn_nu, un_nu);
-        nu = rdiv(R(1), ig);
-        nu = nu < R(1e-10) ? R(1e-10) : (nu > R(1e10) ? R(1e10) : nu);
+        nu = draw_nu_person(th, ze, xb1, s_beta[F + 1], S22, k1, k2, zn_nu, un_nu);
         if (pvalid) A.nu[pi] = nu;
       }
-      R* u = s_u + tid * Dgp;
-      u[0] = pvalid ? R(1) : R(0);
-      u[F + 1] = pvalid ? th : R(0);
-      u[F + 2] = pvalid ? ze : R(0);
-      u[F + 3] = (pvalid && qr) ? nu : R(0);
-      u[F + 4] = (pvalid && qr) ? rdiv(R(1), nu) : R(0);  // weight of the nu-weighted Gram
+      write_u_row(s_u + tid * Dgp, pvalid, qr, F, th, ze, nu);
       if (pvalid && do_pg) acc_cells += (uint32_t)J;
     }
     __syncthreads();
@@ -543,8 +610,7 @@ __global__ void __launch_bounds__(CTA_THREADS, (sizeof(R) == 8 ? min_ctas_f64<TP
               R mu = rdiv(parB, parA);
               if (!(mu >= R(1e-10))) mu = R(1e-10);
               const R ig = ig_msh<R>(mu, parB * parB, zn[e], un[e]);
-              nun = rdiv(R(1), ig);
-              nun = nun < R(1e-10) ? R(1e-10) : (nun > R(1e10) ? R(1e10) : nun);
+              nun = clamp_nu(rdiv(R(1), ig));
             }
           }
           out.v[e] = nun;
@@ -824,15 +890,7 @@ __global__ void __launch_bounds__(CTA_THREADS, (sizeof(R) == 8 ? min_ctas_f64<TP
   if (cqr) atomicAdd(&s_scal[SC_LL_RT], acc_ll_rt);
   atomicAdd(&s_scal[SC_PG_DEFER], (double)acc_defer);
   if (tid < P) atomicAdd(&s_scal[SC_PG_CELLS], (double)acc_cells);
-  __syncthreads();
-  for (int t = tid; t < n_stat_blocks * Jp; t += CTA_THREADS) {
-    const int j = t % Jp;
-    if (j < J) atomicAdd(&A.stats[L.s_S0 + t], s_acc_item[t]);
-  }
-  for (int t = tid; t < 2 * L.ntri; t += CTA_THREADS)
-    if (t < L.ntri || qr) atomicAdd(&A.stats[L.s_gram + t], s_acc_gram[t]);
-  if (tid < SC_COUNT) atomicAdd(&A.stats[L.s_scal + tid], s_scal[tid]);
-  if (tid == 0) tma_store_wait_all();
+  flush_to_stats(A, J, Jp, s_acc_item, n_stat_blocks, s_acc_gram, qr, s_scal, tid);
 }
 
 // ---------------- parity / distribution-test kernels ----------------

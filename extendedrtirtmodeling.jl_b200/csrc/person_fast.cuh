@@ -1,7 +1,7 @@
 // person_fast.cuh -- the f32 person-sweep kernel of the one-launch models (MlIrt, RtIrt, RtIrtNull, Latent, LatentQr):
 // the hot configuration (BASELINE config 5 = LatentQr, 1M x 100, f32).  Same statement, data layout, Philox stream and
-// statistics as person_sweep_kernel<float, TPP, 0> (person.cuh, which remains the f64 / Cross-family kernel); what differs
-// is the instruction schedule of the per-cell loops:
+// statistics as person_sweep_kernel<float, TPP, 0> (person.cuh, which remains the f64 / Cross-family kernel), and the same
+// per-person conditionals (the helpers in person.cuh); what differs is the instruction schedule of the per-cell loops:
 //   * all per-cell arithmetic runs two cells per instruction on the packed FP32 pipe (FFMA2/FMUL2/FADD2, pg_fast.cuh);
 //   * attempt 0 of the PG draw decides only "certainly accepted" / "certainly rejected" with constant bounds of a_1/a_0
 //     (6 MUFU per cell instead of 10); undecided cells (0.5 %) are replayed with the a_1 term from a second work queue;
@@ -363,87 +363,24 @@ __global__ void __launch_bounds__(CTA_THREADS, min_ctas_per_sm<TPP>()) person_sw
       PF_TICK(2);  // row sums
       // ---- person phase, part 2: theta_k, zeta_k, structural log-density, moments ----
       if (lead) {
-        {
-          const R mu0 = (model == M_MLIRT || model == M_RTIRT) ? xb1 : R(0);
-          const R var0 = (model == M_MLIRT) ? R(1) : S11;
-          const R iv0 = rdiv(R(1), var0);
-          const R parV = rdiv(R(1), iv0 + d.x);
-          const R parM = parV * (mu0 * iv0 + d.z + d.y);
-          th = parM + sqrt_of(parV) * zn_theta;
-        }
-        R mu_z = R(0), var_z = R(1);
-        if (has_rt) {
-          if (model == M_RTIRT) { mu_z = xb2; var_z = S22; }
-          else if (latent) {
-            mu_z = fmaf(th, s_beta[F + 1], xb1);
-            var_z = S22;
-            if (qr) { mu_z = fmaf(k1, nu, mu_z); var_z = S22 * (k2 * nu); }
-          } else { mu_z = R(0); var_z = R(1); }  // RtIrtNull, Draw.pl.jl:120-121
-          const R ivz = rdiv(R(1), var_z);
-          const R parV = rdiv(R(1), ivz + sum_is2);
-          const R parM = parV * (mu_z * ivz + d.w);
-          ze = parM + sqrt_of(parV) * zn_zeta;
-        }
+        th = theta_draw(model, xb1, S11, d.x, d.y, d.z, zn_theta);
+        R mu_z, var_z;
+        zeta_prior(model, has_rt, latent, qr, th, nu, xb1, xb2, s_beta[F + 1], S22, k1, k2, mu_z, var_z);
+        if (has_rt) ze = zeta_draw(mu_z, var_z, sum_is2, d.w, zn_zeta);
         if (pvalid) {
-          const R LOG2PI = R(1.8378770664093454835606594728112);
-          R ls;
-          if (model == M_MLIRT) {
-            const R r = th - xb1;
-            ls = R(-0.5) * LOG2PI - R(0.5) * r * r;
-          } else if (latent) {
-            const R r = ze - mu_z;
-            ls = R(-0.5) * (LOG2PI + rlog(var_z)) - R(0.5) * r * rdiv(r, var_z);
-          } else {
-            const R e1 = th - (model == M_RTIRT ? xb1 : R(0));
-            const R e2 = ze - (model == M_RTIRT ? xb2 : R(0));
-            const R det = S11 * S22 - S12 * S12;
-            ls = -LOG2PI - R(0.5) * rlog(det) - R(0.5) * rdiv(S22 * e1 * e1 - R(2) * S12 * e1 * e2 + S11 * e2 * e2, det);
-          }
-          acc_ll_struct += (double)ls;
+          acc_ll_struct += (double)struct_log_density(model, th, ze, xb1, xb2, mu_z, var_z, S11, S12, S22);
           A.theta[pi] = th;
           if (has_rt) A.zeta[pi] = ze;
-          if (post_burnin) {
-            double* m = A.mom + pi;  // fire-and-forget reductions (RED.ADD.F64): no round trip on the critical path
-            atomicAdd(&m[0], (double)th);
-            atomicAdd(&m[A.n_pad], (double)th * (double)th);
-            if (has_rt) {
-              atomicAdd(&m[2 * A.n_pad], (double)ze);
-              atomicAdd(&m[3 * A.n_pad], (double)ze * (double)ze);
-            }
-            if (qr) {
-              atomicAdd(&m[4 * A.n_pad], (double)nu);
-              atomicAdd(&m[5 * A.n_pad], (double)nu * (double)nu);
-            }
-          }
-          if (A.ptrace) {
-            R* t = A.ptrace + ((int64_t)(k - 1) * 3) * A.n_pad + pi;
-            t[0] = th;
-            t[A.n_pad] = ze;
-            t[2 * A.n_pad] = nu;
-          }
+          record_person(A, pi, k, post_burnin, A.ptrace != nullptr, has_rt, qr, th, ze, nu);
         }
       }
     }
     if (lead) {
-      // ---- nu_{k+1} (LatentQr), Draw.pl.jl:325-343 ----
       if (qr) {
-        const R xb = fmaf(th, s_beta[F + 1], xb1);
-        const R isc = rdiv(R(1), sqrt_of(S22 * k2));
-        const R parA = fabsf(ze - xb) * isc;
-        const R parB = sqrt_of(R(2) * k2 + k1 * k1) * isc;
-        R mu = rdiv(parB, parA);
-        if (!(mu >= R(1e-10))) mu = R(1e-10);
-        const R ig = ig_msh<R>(mu, parB * parB, zn_nu, un_nu);
-        nu = rdiv(R(1), ig);
-        nu = nu < R(1e-10) ? R(1e-10) : (nu > R(1e10) ? R(1e10) : nu);
+        nu = draw_nu_person(th, ze, xb1, s_beta[F + 1], S22, k1, k2, zn_nu, un_nu);
         if (pvalid) A.nu[pi] = nu;
       }
-      R* u = s_u + p * Dgp;
-      u[0] = pvalid ? R(1) : R(0);
-      u[F + 1] = pvalid ? th : R(0);
-      u[F + 2] = pvalid ? ze : R(0);
-      u[F + 3] = (pvalid && qr) ? nu : R(0);
-      u[F + 4] = (pvalid && qr) ? rdiv(R(1), nu) : R(0);  // weight of the nu-weighted Gram
+      write_u_row(s_u + p * Dgp, pvalid, qr, F, th, ze, nu);
       if (pvalid) acc_cells += (uint32_t)J;
     }
     PF_TICK(4);  // person part 2, nu, u rows
@@ -711,15 +648,7 @@ __global__ void __launch_bounds__(CTA_THREADS, min_ctas_per_sm<TPP>()) person_sw
       atomicAdd(&s_scal[SC_PG_CELLS], (double)c1);
     }
   }
-  __syncthreads();
-  for (int t = tid; t < 5 * Jp; t += CTA_THREADS) {
-    const int j = t % Jp;
-    if (j < J) atomicAdd(&A.stats[L.s_S0 + t], s_acc_item[t]);
-  }
-  for (int t = tid; t < 2 * L.ntri; t += CTA_THREADS)
-    if (t < L.ntri || qr) atomicAdd(&A.stats[L.s_gram + t], s_acc_gram[t]);
-  if (tid < SC_COUNT) atomicAdd(&A.stats[L.s_scal + tid], s_scal[tid]);
-  if (tid == 0) tma_store_wait_all();
+  flush_to_stats(A, J, Jp, s_acc_item, 5, s_acc_gram, qr, s_scal, tid);
 #ifdef ERIRT_TIMELINE
   __syncthreads();
   if (tid == 0) {
