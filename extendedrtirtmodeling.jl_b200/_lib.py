@@ -17,7 +17,7 @@ ERROR_TYPES = {"tnorm": 0, "unit": 1, "norm": 2, "tail": 3, "skew": 4}
 COMPAT_BETA_PRIOR_DIAG = 1
 COMPAT_LATENTQR_SCALE_ELEMENTWISE = 2
 
-EXPORTED = ["erirt_version", "erirt_last_error", "erirt_create", "erirt_destroy", "erirt_set_data",
+EXPORTED = ["erirt_version", "erirt_last_error", "erirt_create", "erirt_create_batch", "erirt_destroy", "erirt_set_data",
             "erirt_set_data_device", "erirt_trim_pool", "erirt_generate_data", "erirt_get_data", "erirt_set_data_y8", "erirt_checkpoint_size", "erirt_checkpoint_save", "erirt_checkpoint_load", "erirt_set_state", "erirt_get_state", "erirt_sample", "erirt_get_trace",
             "erirt_trace_width", "erirt_get_moments", "erirt_trace_ess_rhat", "erirt_ess_rhat", "erirt_loglik_current", "erirt_get_stats", "erirt_debug_check_guards",
             "erirt_nccl_unique_id", "erirt_comm_init", "erirt_peer_export", "erirt_peer_attach", "erirt_peer_detach", "erirt_k_pg", "erirt_k_nu_person", "erirt_k_philox"]
@@ -60,6 +60,7 @@ def load():
     L.erirt_version.restype = C.c_int
     L.erirt_last_error.restype = C.c_char_p
     L.erirt_create.argtypes = [C.POINTER(Config), C.POINTER(vp)]
+    L.erirt_create_batch.argtypes = [C.POINTER(Config), C.c_int32, C.POINTER(vp)]
     L.erirt_destroy.argtypes = [vp]
     L.erirt_trim_pool.argtypes = [C.c_int32]
     L.erirt_set_data.argtypes = [vp, vp, C.c_int64, vp, C.c_int64, vp, C.c_int64]

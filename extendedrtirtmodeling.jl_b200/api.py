@@ -247,6 +247,111 @@ def _collect(MCMC, eng, person_trace):
 sample_bang = sample  # `sample!` is not a Python identifier
 
 
+class _ReplicaView:
+    """Replica r of a batched engine seen through the getters _collect uses; each batched read is made once and shared by the views."""
+
+    def __init__(self, eng, r, cache):
+        self.eng, self.r, self.cache = eng, r, cache
+
+    def _get(self, *key):
+        if key not in self.cache:
+            self.cache[key] = getattr(self.eng, key[0])(*key[1:])
+        return self.cache[key]
+
+    def _at(self, v):
+        return v[self.r] if self.eng.B > 1 else v  # a batch of one has the standalone shapes
+
+    def trace_width(self, which):
+        return self.eng.trace_width(which)
+
+    def get_trace(self, which, first_col=0, n_cols=None):
+        return self._at(self._get("get_trace", which, first_col, n_cols))
+
+    def get_moments(self, name):
+        m, s = self._get("get_moments", name)
+        return self._at(m), self._at(s)
+
+    def get_state(self, name):
+        return self._at(self._get("get_state", name))
+
+
+def _check_batch(MCMCs, person_trace=False):
+    """ValueError (before any GPU work) unless MCMCs can share one replica batch."""
+    if len(MCMCs) == 0:
+        raise ValueError("sampleBatch needs at least one model object")
+    M0 = MCMCs[0]
+    if any(type(M) is not type(M0) for M in MCMCs):
+        raise ValueError("sampleBatch: all model objects must be of one type")
+    if any(M.Cond != M0.Cond for M in MCMCs):
+        raise ValueError("sampleBatch: all model objects must have equal Cond")
+    if M0.model in ("RtIrtCross", "RtIrtCrossQr"):
+        raise ValueError("sampleBatch: the Cross family is not supported (two-stage sweep)")
+    if person_trace:
+        raise ValueError("sampleBatch keeps no person trace (person_trace=True is not supported)")
+    dev = [isinstance(M.Data, DeviceData) for M in MCMCs]
+    if any(dev) and not all(dev):
+        raise ValueError("sampleBatch: mixed host and device data")
+    if all(dev):
+        D0 = M0.Data
+        if any(M.Data.error != D0.error or M.Data.seed != D0.seed + r or (M.Data.X is None) != (D0.X is None) for r, M in enumerate(MCMCs)):
+            raise ValueError("sampleBatch: device data of a batch must share the error type, and replica r must have data seed seed_0 + r")
+
+
+def _batch_data(eng, MCMCs):
+    M0, F = MCMCs[0], MCMCs[0].Cond.nFeat
+    if isinstance(M0.Data, DeviceData):  # one call: replica r generates with data seed D_0.seed + r
+        P = [M.Data.truePara for M in MCMCs]
+        cat = lambda f: np.concatenate([np.asarray(f(p), dtype=np.float64).ravel() for p in P])  # noqa: E731
+        has_rt = M0.has_rt
+        eng.generate_data(cat(lambda p: p.theta), cat(lambda p: p.a), cat(lambda p: p.b), cat(lambda p: p.zeta) if has_rt else None,
+                          cat(lambda p: p.lambda_) if has_rt else None,
+                          cat(lambda p: p.sigma2t) if (has_rt and np.size(P[0].sigma2t)) else None,
+                          cat(lambda p: p.rho) if np.size(P[0].rho) else None,
+                          None if M0.Data.X is None else np.concatenate([M.Data.X for M in MCMCs], axis=0),
+                          error=M0.Data.error, seed=M0.Data.seed)
+    else:
+        eng.set_data(np.concatenate([np.asarray(M.Data.Y) for M in MCMCs], axis=0),
+                     np.concatenate([M.Data.logT for M in MCMCs], axis=0) if M0.has_rt else None,
+                     np.concatenate([M.Data.X for M in MCMCs], axis=0) if F > 0 else None)
+
+
+def sampleBatch(MCMCs, intercept=False, itemtype="2pl", cov2one=None, *, seed=1234, dtype="f64", chain=0, device=0,
+                person_trace=False, compat=0, use_graph=True):
+    """sample(MCMC_r, seed=seed + r, person_trace=False) for every MCMC_r of `MCMCs`, as ONE replica batch on one GPU
+    (erirt_create_batch, DESIGN.md 6.6): one person launch and one global launch per sweep for all of them.  The model objects
+    must be of one type (not the Cross family) with equal Cond; each brings its own Data (all host InputData, or all DeviceData with
+    consecutive data seeds) and initial Para.  Fills every MCMC.Post and MCMC.Para exactly as the sequential calls would.
+    Returns MCMCs."""
+    if itemtype not in ("1pl", "2pl"):
+        raise ValueError("Invalid input: the item type must be '1pl' or '2pl'.")
+    MCMCs = list(MCMCs)
+    _check_batch(MCMCs, person_trace)
+    M0 = MCMCs[0]
+    C = M0.Cond
+    if cov2one is None:
+        cov2one = M0.default_cov2one
+    eng = Engine(M0.model, C.nSubj, C.nItem, C.nFeat, n_iter=C.nIter, n_chain=C.nChain, n_burnin=C.nBurnin, q_rt=C.qRt,
+                 intercept=intercept, itemtype=itemtype, cov2one=cov2one, dtype=dtype, seed=seed, chain=chain, compat=compat,
+                 person_trace=False, device=device, use_graph=use_graph, n_batch=len(MCMCs))
+    try:
+        _batch_data(eng, MCMCs)
+        P = [M.Para for M in MCMCs]
+        init = dict(theta=[p.theta for p in P], a=[p.a for p in P], b=[p.b for p in P])
+        if M0.has_rt:
+            init.update(zeta=[p.zeta for p in P], lambda_=[p.lambda_ for p in P], sigma2=[p.sigma2t for p in P], Sigma=[p.Sigma_p for p in P])
+        if P[0].beta.size:
+            init["beta"] = [p.beta for p in P]
+        eng.set_state(**init)
+        eng.sample(C.nIter * C.nChain)
+        cache = {}
+        for r, M in enumerate(MCMCs):
+            M.nu_cell_moments = False
+            _collect(M, _ReplicaView(eng, r, cache), False)
+    finally:
+        eng.close()
+    return MCMCs
+
+
 def sampleIndependentChains(MCMC, n_chains, group=None, rng=0, **kw):
     """BASELINE configs[3] / SURVEY 8e "independent chains": n_chains truly independent chains of MCMC's model on MCMC's data -- distinct
     Philox keys (chain id c) and distinct initial values (constructor seeded rng + c) -- dealt to the ranks of the torch.distributed
@@ -323,6 +428,40 @@ def getDic(MCMC, dtype="f64", device=0):
     dic.pD = Dbar - Dhat
     dic.DIC = Dbar + dic.pD
     return dic
+
+
+def getDicBatch(MCMCs, dtype="f64", device=0):
+    """getDic(MCMC_r) for every MCMC_r of `MCMCs` (one type, equal Cond, sampled), with ONE batched evaluation engine: one
+    loglik_current call evaluates every replica's Post.mean on its own data."""
+    MCMCs = list(MCMCs)
+    _check_batch(MCMCs)
+    M0 = MCMCs[0]
+    C = M0.Cond
+    eng = Engine(M0.model, C.nSubj, C.nItem, C.nFeat, n_iter=1, n_chain=1, q_rt=C.qRt, dtype=dtype, device=device,
+                 person_trace=False, use_graph=False, n_batch=len(MCMCs))
+    try:
+        _batch_data(eng, MCMCs)
+        P = [M.Post.mean for M in MCMCs]
+        st = dict(theta=[p.theta for p in P], a=[p.a for p in P], b=[p.b for p in P])
+        if M0.has_rt:
+            st.update(zeta=[p.zeta for p in P], lambda_=[p.lambda_ for p in P], sigma2=[p.sigma2t for p in P],
+                      Sigma=[np.asarray(p.Sigma_p).reshape(4) for p in P])
+        if P[0].beta.size:
+            st["beta"] = [p.beta for p in P]
+        if M0.model == "RtIrtLatentQr":
+            st["nu"] = [p.nu for p in P]
+        eng.set_state(**st)
+        ll = np.atleast_1d(eng.loglik_current())
+    finally:
+        eng.close()
+    out = []
+    for M, l in zip(MCMCs, ll):
+        Dhat, Dbar = -2.0 * float(l), -2.0 * float(np.mean(M.Post.logLike))
+        dic = OutputDic()
+        dic.pD = Dbar - Dhat
+        dic.DIC = Dbar + dic.pD
+        out.append(dic)
+    return out
 
 
 def _param_names(MCMC):

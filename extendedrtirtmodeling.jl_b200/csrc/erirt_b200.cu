@@ -338,6 +338,8 @@ struct erirt_handle {
   PhiloxKey key{};            // make_key(cfg.seed, cfg.chain)
   int64_t n_pad = 0;
   int cap = 0, qw = 0;
+  int nb = 1;        // replicas of a batched handle (erirt_create_batch): every per-replica buffer below holds nb copies
+  ReplicaSizes z{};  // lengths of one copy
   cudaStream_t stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   // device buffers
@@ -423,40 +425,53 @@ static SmemPlan make_smem_plan(const Layout& L, int tpp, size_t rsz, bool has_rt
   return S;
 }
 
+// batch: the replica-batch instantiation of the kernel (BATCH = true)
+template <typename R, int TPP, int FAM>
+static const void* person_kernel_ptr_t(bool batch) {
+  return batch ? (const void*)person_sweep_kernel<R, TPP, FAM, true> : (const void*)person_sweep_kernel<R, TPP, FAM>;
+}
 template <typename R, int FAM>
-static const void* person_kernel_ptr(int tpp) {
+static const void* person_kernel_ptr(int tpp, bool batch) {
   switch (tpp) {
-    case 1: return (const void*)person_sweep_kernel<R, 1, FAM>;
-    case 2: return (const void*)person_sweep_kernel<R, 2, FAM>;
-    case 4: return (const void*)person_sweep_kernel<R, 4, FAM>;
-    default: return (const void*)person_sweep_kernel<R, 8, FAM>;
+    case 1: return person_kernel_ptr_t<R, 1, FAM>(batch);
+    case 2: return person_kernel_ptr_t<R, 2, FAM>(batch);
+    case 4: return person_kernel_ptr_t<R, 4, FAM>(batch);
+    default: return person_kernel_ptr_t<R, 8, FAM>(batch);
   }
+}
+template <int TPP, int MODEL>
+static const void* person_fast_kernel_ptr_t(bool batch) {
+  return batch ? (const void*)person_sweep_fast_kernel<TPP, MODEL, true> : (const void*)person_sweep_fast_kernel<TPP, MODEL>;
 }
 template <int MODEL>
-static const void* person_fast_kernel_ptr_m(int tpp) {
+static const void* person_fast_kernel_ptr_m(int tpp, bool batch) {
   switch (tpp) {
-    case 1: return (const void*)person_sweep_fast_kernel<1, MODEL>;
-    case 2: return (const void*)person_sweep_fast_kernel<2, MODEL>;
-    case 4: return (const void*)person_sweep_fast_kernel<4, MODEL>;
-    default: return (const void*)person_sweep_fast_kernel<8, MODEL>;
+    case 1: return person_fast_kernel_ptr_t<1, MODEL>(batch);
+    case 2: return person_fast_kernel_ptr_t<2, MODEL>(batch);
+    case 4: return person_fast_kernel_ptr_t<4, MODEL>(batch);
+    default: return person_fast_kernel_ptr_t<8, MODEL>(batch);
   }
 }
-static const void* person_fast_kernel_ptr(int tpp, int model) {
+static const void* person_fast_kernel_ptr(int tpp, int model, bool batch) {
   switch (model) {
-    case M_MLIRT: return person_fast_kernel_ptr_m<M_MLIRT>(tpp);
-    case M_RTIRT: return person_fast_kernel_ptr_m<M_RTIRT>(tpp);
-    case M_NULL: return person_fast_kernel_ptr_m<M_NULL>(tpp);
-    case M_LATENT: return person_fast_kernel_ptr_m<M_LATENT>(tpp);
-    default: return person_fast_kernel_ptr_m<M_LATENTQR>(tpp);
+    case M_MLIRT: return person_fast_kernel_ptr_m<M_MLIRT>(tpp, batch);
+    case M_RTIRT: return person_fast_kernel_ptr_m<M_RTIRT>(tpp, batch);
+    case M_NULL: return person_fast_kernel_ptr_m<M_NULL>(tpp, batch);
+    case M_LATENT: return person_fast_kernel_ptr_m<M_LATENT>(tpp, batch);
+    default: return person_fast_kernel_ptr_m<M_LATENTQR>(tpp, batch);
   }
 }
 // Stage 0 is the sweep of the one-launch models, stages 1 and 2 the two halves of a Cross-family sweep, stage 3 the evaluation.
 // Stage 0 in f32 runs person_sweep_fast_kernel (plan h->S); every other stage runs the generic kernel (plan h->S_gen).
 static bool runs_fast_kernel(const erirt_handle* h, int stage) { return stage == 0 && h->cfg.dtype == ERIRT_F32; }
 static const void* person_kernel_for(const erirt_handle* h, int stage) {
-  if (runs_fast_kernel(h, stage)) return person_fast_kernel_ptr(h->tpp, h->cfg.model);
-  if (stage == 0) return person_kernel_ptr<double, 0>(h->tpp);  // Cross-family and evaluation code compiled out
-  return h->cfg.dtype == ERIRT_F32 ? person_kernel_ptr<float, 1>(h->tpp_gen) : person_kernel_ptr<double, 1>(h->tpp_gen);
+  const bool batch = h->nb > 1;
+  if (runs_fast_kernel(h, stage)) return person_fast_kernel_ptr(h->tpp, h->cfg.model, batch);
+  if (stage == 0) return person_kernel_ptr<double, 0>(h->tpp, batch);  // Cross-family and evaluation code compiled out
+  return h->cfg.dtype == ERIRT_F32 ? person_kernel_ptr<float, 1>(h->tpp_gen, batch) : person_kernel_ptr<double, 1>(h->tpp_gen, batch);
+}
+static const void* global_kernel_for(const erirt_handle* h) {
+  return h->nb > 1 ? (const void*)global_draw_kernel<true> : (const void*)global_draw_kernel<>;
 }
 
 static int qr_small_width(int model, int J, int F) {
@@ -531,9 +546,15 @@ static int free_handle(erirt_handle* h) {
   return 0;
 }
 
-extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
+extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) { return erirt_create_batch(cfg, 1, out); }
+
+extern "C" int erirt_create_batch(const erirt_config* cfg, int32_t n_batch, erirt_handle** out) {
   if (!cfg || !out) return fail(ERIRT_E_ARG, "null argument");
   *out = nullptr;
+  if (n_batch < 1 || n_batch > 65535) return fail(ERIRT_E_ARG, "n_batch %d outside [1, 65535]", n_batch);
+  if (n_batch > 1 && (cfg->model == ERIRT_RTIRT_CROSS || cfg->model == ERIRT_RTIRT_CROSSQR))
+    return fail(ERIRT_E_UNSUPPORTED, "replica batches of the Cross family are not supported (two-stage sweep)");
+  if (n_batch > 1 && cfg->person_trace) return fail(ERIRT_E_UNSUPPORTED, "replica batches keep no person trace (person_trace = 1)");
   if (cfg->abi_version != ERIRT_ABI_VERSION) return fail(ERIRT_E_ARG, "abi_version %d != %d", cfg->abi_version, ERIRT_ABI_VERSION);
   if (cfg->model < 0 || cfg->model > 6) return fail(ERIRT_E_ARG, "unknown model %d", cfg->model);
   if (cfg->n_subj < 1 || cfg->n_item < 1 || cfg->n_feat < 0) return fail(ERIRT_E_ARG, "bad dimensions");
@@ -569,6 +590,7 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
   }
   erirt_handle* h = new erirt_handle();
   h->cfg = *cfg;
+  h->nb = n_batch;
   h->sm_count = prop.multiProcessorCount;
   h->rsz = cfg->dtype == ERIRT_F32 ? 4 : 8;
   h->k1 = (1.0 - 2.0 * cfg->q_rt) / (cfg->q_rt * (1.0 - cfg->q_rt));
@@ -591,8 +613,9 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
     // sweep is bound by the per-tile latency chain, gain nothing: profiles/r02_summary.md)
     // (for a large problem TPP = 8 was 7 % faster while the cell loop was one divergent exact draw per cell; with the branch-free
     // attempt 0 the 168-register TPP = 4 instantiation wins, 4.0 against 5.3 ms per sweep at 1M x 100)
+    // (a replica batch counts the tiles of all its replicas)
     if (!fast && cfg->dtype == ERIRT_F64)
-      while (tpp < 8 && (int64_t)align_up((size_t)cfg->n_subj, 128) / (CTA_THREADS / tpp) < 2 * (int64_t)h->sm_count) tpp *= 2;
+      while (tpp < 8 && (int64_t)align_up((size_t)cfg->n_subj, 128) * n_batch / (CTA_THREADS / tpp) < 2 * (int64_t)h->sm_count) tpp *= 2;
     if (n_groups > 16 * tpp) return "too many items for this TPP (at most 64*TPP - 4)";
     S = make_smem_plan(h->L, tpp, h->rsz, has_rt, is_cqr, is_cross, fast);
     if (S.total > 227 * 1024) return "n_item needs more shared memory per CTA than an SM has";
@@ -608,6 +631,7 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
   h->n_pad = (int64_t)align_up((size_t)cfg->n_subj, 128);
   h->cap = cfg->n_iter * cfg->n_chain;
   h->qw = qr_small_width(cfg->model, cfg->n_item, cfg->n_feat);
+  h->z = replica_sizes(h->n_pad, h->L, h->cap, h->qw);
 
   {
     tm.mark("create: pool attr, plans");
@@ -622,11 +646,15 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
   // the pool again.
   const size_t cells = (size_t)h->n_pad * h->L.Jp;
   h->c_T1 = 0; h->c_T2 = h->L.Jp; h->c_K0 = 2 * h->L.Jp; h->c_XtX = 3 * h->L.Jp; h->c_sums = h->c_XtX + MAXD * MAXD / 4;
-  h->c_count = h->c_sums + 2;
+  h->c_count = consts_count(h->L);
   {
     struct Req { void** p; size_t bytes; };
     std::vector<Req> reqs;
-    auto want = [&](void** p, size_t bytes) { reqs.push_back({p, align_up(bytes > 0 ? bytes : 16, 256)}); };
+    // every buffer but the ingest scratch dColPart holds one copy per replica (ReplicaSizes)
+    auto want = [&](void** p, size_t bytes) {
+      if (p != (void**)&h->dColPart) bytes *= (size_t)n_batch;
+      reqs.push_back({p, align_up(bytes > 0 ? bytes : 16, 256)});
+    };
     const size_t vec = (size_t)h->n_pad * h->rsz, D = sizeof(double);
     want((void**)&h->dY, cells);
     want(&h->dOmega, cells * h->rsz);
@@ -681,6 +709,8 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
     std::vector<double> p(h->L.p_count, 0.0);
     for (int j = 0; j < cfg->n_item; ++j) { p[h->L.p_a + j] = 1.0; p[h->L.p_sigma2 + j] = 1.0; }
     p[h->L.p_Sigma + 0] = 1.0; p[h->L.p_Sigma + 3] = 1.0;
+    const std::vector<double> one = p;
+    for (int r = 1; r < n_batch; ++r) p.insert(p.end(), one.begin(), one.end());
     cudaMemcpyAsync(h->dParams, p.data(), p.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream);
     cudaStreamSynchronize(h->stream);  // p is a local; also orders the zero-fill before any default-stream access below
   }
@@ -694,11 +724,13 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
   ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kfn, CTA_THREADS, h->S.total);
   if (ce != cudaSuccess || occ < 1) { free_handle(h); return fail(ERIRT_E_CUDA, "person kernel does not fit on an SM: %s", cudaGetErrorString(ce)); }
   const int n_tiles = (int)(h->n_pad / h->S.P);
-  h->grid = std::min(n_tiles, h->sm_count * occ);
+  // A replica batch launches grid x n_batch CTAs: the grid of a replica is sized so that the whole launch stays within the resident
+  // slots where it can (one CTA per replica at least)
+  h->grid = std::max(1, std::min(n_tiles, h->sm_count * occ / n_batch));
   // A full grid leaves ONE slot free: with dynamic tile dealing no person CTA exits before the last round, so the global kernel of the
   // sweep (256 threads, 80 registers, ~55 KB) could otherwise not become resident early enough to finish its rehearsal pass
   // (global.cuh) before the person kernel ends; the slot costs 1/444 of the person kernel's throughput
-  if (h->grid == h->sm_count * occ && h->grid > 1) h->grid -= 1;
+  if (h->grid * n_batch == h->sm_count * occ && h->grid > 1) h->grid -= 1;
   // test hook: ERIRT_MAX_GRID caps the persistent grid, so that a small problem gives every CTA many tiles (the cross-tile register
   // accumulators and their 16-tile fold are otherwise reached only at benchmark size); results do not depend on the grid
   const char* env_grid = getenv("ERIRT_MAX_GRID");
@@ -706,14 +738,14 @@ extern "C" int erirt_create(const erirt_config* cfg, erirt_handle** out) {
   h->grid = std::min(h->grid, max_grid);
   {  // the global kernel stages the statistics in dynamic shared memory on top of its ~42 KB of static scratch
     const size_t gsm = (size_t)(h->L.s_count + 2 + (h->L.F + 1) * (h->L.F + 1) + 5 * h->L.Jp) * sizeof(double);
-    ce = cudaFuncSetAttribute((const void*)global_draw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gsm);
+    ce = cudaFuncSetAttribute(global_kernel_for(h), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gsm);
     if (ce != cudaSuccess) { free_handle(h); return fail(ERIRT_E_CUDA, "cudaFuncSetAttribute(global_draw_kernel, %zu bytes): %s", gsm, cudaGetErrorString(ce)); }
   }
   {
     int occ_gen = 0;
     ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_gen, person_kernel_for(h, 1), CTA_THREADS, h->S_gen.total);
     if (ce != cudaSuccess || occ_gen < 1) { free_handle(h); return fail(ERIRT_E_CUDA, "generic person kernel does not fit on an SM: %s", cudaGetErrorString(ce)); }
-    h->grid_gen = std::min(std::min((int)(h->n_pad / h->S_gen.P), h->sm_count * occ_gen), max_grid);
+    h->grid_gen = std::min(std::min((int)(h->n_pad / h->S_gen.P), std::max(1, h->sm_count * occ_gen / n_batch)), max_grid);
   }
   tm.mark("create: func attrs, occupancy");
   *out = h;
@@ -738,35 +770,36 @@ extern "C" int erirt_trim_pool(int32_t device) {
 // ------------------------------------------------------------------------------------------------
 // data
 // ------------------------------------------------------------------------------------------------
-// Pack columns [c0, c0+nc) of Y / logT (column-major, on the device) into the person-major tiles and add their partial column sums.
+// Pack columns [c0, c0+nc) of replica r's Y / logT (column-major, on the device) into its person-major tiles and add their partial
+// column sums.
 template <typename R, typename YT>
-static void pack_columns(erirt_handle* h, const YT* dYc, int64_t ldY, const double* dTc, int64_t ldT, int c0, int nc) {
+static void pack_columns(erirt_handle* h, int r, const YT* dYc, int64_t ldY, const double* dTc, int64_t ldT, int c0, int nc) {
   const int64_t n = h->cfg.n_subj;
   const int Jp = h->L.Jp;
   dim3 blk(32, 8), grd((unsigned)((n + 31) / 32), (unsigned)((nc + 31) / 32));
   dim3 cg((unsigned)nc, COLSUM_PARTS);
-  pack_transpose_kernel<YT, uint8_t, true><<<grd, blk, 0, h->stream>>>(dYc, ldY, n, nc, h->dY + c0, Jp);
+  pack_transpose_kernel<YT, uint8_t, true><<<grd, blk, 0, h->stream>>>(dYc, ldY, n, nc, h->dY + r * h->z.cells + c0, Jp);
   colsum_part_kernel<YT><<<cg, 256, 0, h->stream>>>(dYc, ldY, n, 2, h->dColPart + (size_t)(2 * Jp + c0) * COLSUM_PARTS);
   if (dTc) {
-    pack_transpose_kernel<double, R, false><<<grd, blk, 0, h->stream>>>(dTc, ldT, n, nc, (R*)h->dLogT + c0, Jp);
+    pack_transpose_kernel<double, R, false><<<grd, blk, 0, h->stream>>>(dTc, ldT, n, nc, (R*)h->dLogT + r * h->z.cells + c0, Jp);
     colsum_part_kernel<double><<<cg, 256, 0, h->stream>>>(dTc, ldT, n, 0, h->dColPart + (size_t)(0 * Jp + c0) * COLSUM_PARTS);
     colsum_part_kernel<double><<<cg, 256, 0, h->stream>>>(dTc, ldT, n, 1, h->dColPart + (size_t)(1 * Jp + c0) * COLSUM_PARTS);
   }
 }
 
-// The start of every ingest: zero the packed Y / logT (the padding cells stay zero) and the constants the ingest adds up
+// The start of every ingest: zero the packed Y / logT of every replica (the padding cells stay zero) and the constants the ingest adds up
 static int clear_data(erirt_handle* h) {
-  const size_t cells = (size_t)h->n_pad * h->L.Jp;
+  const size_t cells = (size_t)h->z.cells * h->nb;
   CU(cudaMemsetAsync(h->dY, 0, cells, h->stream));
   if (h->cfg.model != ERIRT_MLIRT) CU(cudaMemsetAsync(h->dLogT, 0, cells * h->rsz, h->stream));
-  CU(cudaMemsetAsync(h->dConstsLocal, 0, h->c_count * sizeof(double), h->stream));
+  CU(cudaMemsetAsync(h->dConstsLocal, 0, (size_t)h->z.consts * h->nb * sizeof(double), h->stream));
   return 0;
 }
 
-// The end of every ingest, after Y / logT are packed: X (column-major float64 [n][F], leading dimension ldX; a host buffer unless
-// x_on_device) into dX, the constants in f64 (T1, T2, K0 are consecutive Jp-blocks of the consts vector, finished from `part`:
-// [3 Jp][parts] partial column sums; X'X), then a synchronisation, after which the data set is in place.
-static int finish_ingest(erirt_handle* h, const double* X, int64_t ldX, bool x_on_device, const double* part, int parts) {
+// The end of every ingest of replica r, after its Y / logT are packed: X (column-major float64 [n][F], leading dimension ldX; a host
+// buffer unless x_on_device) into dX, the constants in f64 (T1, T2, K0 are consecutive Jp-blocks of the consts vector, finished from
+// `part`: [3 Jp][parts] partial column sums; X'X), then a synchronisation, after which the replica's data is in place.
+static int finish_ingest(erirt_handle* h, int r, const double* X, int64_t ldX, bool x_on_device, const double* part, int parts) {
   const int64_t n = h->cfg.n_subj;
   const int Jp = h->L.Jp, F = h->cfg.n_feat, pb = F + 1;
   double* staged = nullptr;
@@ -778,12 +811,13 @@ static int finish_ingest(erirt_handle* h, const double* X, int64_t ldX, bool x_o
     ldX = n;
   }
   for (int f = 0; f < F; ++f)
-    with_real(h, [&](auto r) {
-      using R = decltype(r);
-      colmajor_to_tile_kernel<R><<<1024, 256, 0, h->stream>>>(X + ldX * f, n, 1, 1, (R*)h->dX + (int64_t)f * h->n_pad);
+    with_real(h, [&](auto rr) {
+      using R = decltype(rr);
+      colmajor_to_tile_kernel<R><<<1024, 256, 0, h->stream>>>(X + ldX * f, n, 1, 1, (R*)h->dX + r * h->z.x + (int64_t)f * h->n_pad);
     });
-  colsum_finish_kernel<<<(3 * Jp + 127) / 128, 128, 0, h->stream>>>(part, 3 * Jp, h->dConstsLocal + h->c_T1, parts);
-  xtx_kernel<<<pb * pb, 256, 0, h->stream>>>(X, ldX, n, pb, h->dConstsLocal + h->c_XtX);
+  double* consts = h->dConstsLocal + r * h->z.consts;
+  colsum_finish_kernel<<<(3 * Jp + 127) / 128, 128, 0, h->stream>>>(part, 3 * Jp, consts + h->c_T1, parts);
+  xtx_kernel<<<pb * pb, 256, 0, h->stream>>>(X, ldX, n, pb, consts + h->c_XtX);
   CUX(cudaGetLastError());
   cleanup();
   staged = nullptr;
@@ -793,25 +827,23 @@ static int finish_ingest(erirt_handle* h, const double* X, int64_t ldX, bool x_o
   return 0;
 }
 
-// Ingest (K8).  on_device: the three matrices are device buffers and are packed in place.  Otherwise they are host buffers and are
-// streamed through one bounded staging buffer in chunks of whole columns (H2D copy, pack, next chunk: the staging memory stays at
-// <= 64 MB instead of a second copy of the data set, and the packed tiles are the only full-size device copy).
+// Ingest (K8) of replica r: rows [r n_subj, (r+1) n_subj) of the caller's matrices.  on_device: the three matrices are device buffers
+// and are packed in place.  Otherwise they are host buffers and are streamed through one bounded staging buffer in chunks of whole
+// columns (H2D copy, pack, next chunk: the staging memory stays at <= 64 MB instead of a second copy of the data set, and the packed
+// tiles are the only full-size device copy).
 template <typename YT>
-static int ingest(erirt_handle* h, const YT* Y, int64_t ldY, const double* T, int64_t ldT, const double* X, int64_t ldX, bool on_device) {
-  if (!h || !Y) return fail(ERIRT_E_ARG, "null argument");
+static int ingest_replica(erirt_handle* h, int r, const YT* Y, int64_t ldY, const double* T, int64_t ldT, const double* X, int64_t ldX,
+                          bool on_device) {
   const bool has_rt = h->cfg.model != ERIRT_MLIRT;
-  if (has_rt && !T) return fail(ERIRT_E_ARG, "logT is required for this model");
-  if (h->cfg.n_feat > 0 && !X) return fail(ERIRT_E_ARG, "X is required when n_feat > 0");
-  CU(cudaSetDevice(h->cfg.device));
   const int64_t n = h->cfg.n_subj;
-  const int J = h->cfg.n_item, Jp = h->L.Jp, F = h->cfg.n_feat;
-  if (ldY < n || (has_rt && ldT < n) || (F > 0 && ldX < n)) return fail(ERIRT_E_ARG, "leading dimension smaller than n_subj");
-  if (!has_rt) T = nullptr;
-  if (int rc = clear_data(h)) return rc;
+  const int J = h->cfg.n_item, Jp = h->L.Jp;
+  Y += r * n;
+  if (T) T += r * n;
+  if (X) X += r * n;
   CU(cudaMemsetAsync(h->dColPart, 0, (size_t)3 * Jp * COLSUM_PARTS * sizeof(double), h->stream));
   if (on_device) {
-    with_real(h, [&](auto r) { pack_columns<decltype(r), YT>(h, Y, ldY, T, ldT, 0, J); });
-    return finish_ingest(h, X, ldX, true, h->dColPart, COLSUM_PARTS);
+    with_real(h, [&](auto rr) { pack_columns<decltype(rr), YT>(h, r, Y, ldY, T, ldT, 0, J); });
+    return finish_ingest(h, r, X, ldX, true, h->dColPart, COLSUM_PARTS);
   }
   // stream-ordered allocations: cudaFree of large blocks is a device-wide synchronisation (measured up to 0.9 s for GB-sized blocks)
   char* stage = nullptr;
@@ -826,27 +858,40 @@ static int ingest(erirt_handle* h, const YT* Y, int64_t ldY, const double* T, in
     const int nc = std::min(cc, J - c0);
     CUX(cudaMemcpy2DAsync(sY, n * sizeof(YT), Y + ldY * c0, ldY * sizeof(YT), n * sizeof(YT), nc, cudaMemcpyHostToDevice, h->stream));
     if (has_rt) CUX(cudaMemcpy2DAsync(sT, n * sizeof(double), T + ldT * c0, ldT * sizeof(double), n * sizeof(double), nc, cudaMemcpyHostToDevice, h->stream));
-    with_real(h, [&](auto r) { pack_columns<decltype(r), YT>(h, sY, n, sT, n, c0, nc); });
+    with_real(h, [&](auto rr) { pack_columns<decltype(rr), YT>(h, r, sY, n, sT, n, c0, nc); });
   }
   cleanup();
-  return finish_ingest(h, X, ldX, false, h->dColPart, COLSUM_PARTS);
+  return finish_ingest(h, r, X, ldX, false, h->dColPart, COLSUM_PARTS);
+}
+
+// Ingest of every replica: the matrices have n_batch * n_subj rows, replica r's in rows [r n_subj, (r+1) n_subj).  The constants of a
+// replica come from its rows alone, by the code of a standalone ingest, so they carry the same bits.
+template <typename YT>
+static int ingest(erirt_handle* h, const YT* Y, int64_t ldY, const double* T, int64_t ldT, const double* X, int64_t ldX, bool on_device) {
+  if (!h || !Y) return fail(ERIRT_E_ARG, "null argument");
+  const bool has_rt = h->cfg.model != ERIRT_MLIRT;
+  if (has_rt && !T) return fail(ERIRT_E_ARG, "logT is required for this model");
+  if (h->cfg.n_feat > 0 && !X) return fail(ERIRT_E_ARG, "X is required when n_feat > 0");
+  CU(cudaSetDevice(h->cfg.device));
+  const int64_t n = h->cfg.n_subj * h->nb;
+  if (ldY < n || (has_rt && ldT < n) || (h->cfg.n_feat > 0 && ldX < n))
+    return fail(ERIRT_E_ARG, h->nb > 1 ? "leading dimension smaller than n_batch * n_subj" : "leading dimension smaller than n_subj");
+  if (!has_rt) T = nullptr;
+  if (int rc = clear_data(h)) return rc;
+  for (int r = 0; r < h->nb; ++r)
+    if (int rc = ingest_replica(h, r, Y, ldY, T, ldT, X, ldX, on_device)) return rc;
+  return 0;
 }
 
 // ---- data generated on the device (SURVEY 8f-1) ----
-extern "C" int erirt_generate_data(erirt_handle* h, const double* theta, const double* zeta, const double* a, const double* b,
-                                   const double* lambda, const double* sigma2, const double* rho, const double* X, int64_t ldX,
-                                   int32_t error_type, uint64_t seed) {
-  if (!h || !theta || !a || !b) return fail(ERIRT_E_ARG, "null argument");
+// Replica r: the person vectors and X start at its first row, the item vectors at its first item; data seed `seed`
+static int generate_replica(erirt_handle* h, int r, const double* theta, const double* zeta, const double* a, const double* b,
+                            const double* lambda, const double* sigma2, const double* rho, const double* X, int64_t ldX,
+                            int32_t error_type, uint64_t seed) {
   const bool has_rt = h->cfg.model != ERIRT_MLIRT;
-  if (has_rt && (!zeta || !lambda)) return fail(ERIRT_E_ARG, "zeta and lambda are required for a response-time model");
-  if (error_type < 0 || error_type > 4) return fail(ERIRT_E_ARG, "error_type must be 0 (truncated normal), 1 (unit normal), 2 (norm), 3 (tail) or 4 (skew)");
-  if (has_rt && error_type == 0 && !sigma2) return fail(ERIRT_E_ARG, "sigma2 is required for error_type 0");
   const int64_t n = h->cfg.n_subj;
-  const int J = h->cfg.n_item, Jp = h->L.Jp, F = h->cfg.n_feat;
-  if (F > 0 && (!X || ldX < n)) return fail(ERIRT_E_ARG, "X (leading dimension >= n_subj) is required when n_feat > 0");
-  CU(cudaSetDevice(h->cfg.device));
+  const int J = h->cfg.n_item, Jp = h->L.Jp;
   HostTimer tm;
-  if (int rc = clear_data(h)) return rc;
   // device copy of the small inputs: [theta n][zeta n][a Jp][b Jp][lambda Jp][sd Jp][rho Jp]; the person vectors go straight from
   // the caller's buffers, the item vectors through a small host block
   std::vector<double> hit((size_t)5 * Jp, 0.0);
@@ -866,7 +911,8 @@ extern "C" int erirt_generate_data(erirt_handle* h, const double* theta, const d
   CUX(cudaMemcpyAsync(dbuf + 2 * n, hit.data(), hit.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
   tm.mark("generate: host staging, H2D");
   GenArgs A{};
-  A.Y = h->dY; A.logT = h->dLogT;
+  A.Y = h->dY + r * h->z.cells;
+  A.logT = has_rt ? (char*)h->dLogT + r * h->z.cells * h->rsz : nullptr;
   A.theta = dbuf; A.zeta = has_rt ? dbuf + n : nullptr;
   A.a = dbuf + 2 * n; A.b = A.a + Jp; A.lam = A.a + 2 * Jp; A.sd = A.a + 3 * Jp; A.rho = A.a + 4 * Jp;
   A.n = n; A.J = J; A.Jp = Jp; A.err = error_type; A.has_rt = has_rt ? 1 : 0;
@@ -876,12 +922,37 @@ extern "C" int erirt_generate_data(erirt_handle* h, const double* theta, const d
   CUX(cudaMallocAsync((void**)&dpart, (size_t)3 * Jp * TILE_COLSUM_PARTS * sizeof(double), h->stream));
   with_real(h, [&](auto r) {
     using R = decltype(r);
-    tile_colsum_part_kernel<R><<<TILE_COLSUM_PARTS, Jp, 0, h->stream>>>(h->dY, has_rt ? (const R*)h->dLogT : nullptr, n, Jp, dpart);
+    tile_colsum_part_kernel<R><<<TILE_COLSUM_PARTS, Jp, 0, h->stream>>>(A.Y, (const R*)A.logT, n, Jp, dpart);
   });
-  const int rc = finish_ingest(h, X, ldX, false, dpart, TILE_COLSUM_PARTS);
+  const int rc = finish_ingest(h, r, X, ldX, false, dpart, TILE_COLSUM_PARTS);
   cleanup();
   tm.mark("generate: launches, device work");
   return rc;
+}
+
+// A batch generates replica r from rows [r n_subj, (r+1) n_subj) of theta, zeta and X, items [r n_item, (r+1) n_item) of the item
+// vectors, and data seed seed + r: the data set a standalone handle generates from the same inputs with that seed.
+extern "C" int erirt_generate_data(erirt_handle* h, const double* theta, const double* zeta, const double* a, const double* b,
+                                   const double* lambda, const double* sigma2, const double* rho, const double* X, int64_t ldX,
+                                   int32_t error_type, uint64_t seed) {
+  if (!h || !theta || !a || !b) return fail(ERIRT_E_ARG, "null argument");
+  const bool has_rt = h->cfg.model != ERIRT_MLIRT;
+  if (has_rt && (!zeta || !lambda)) return fail(ERIRT_E_ARG, "zeta and lambda are required for a response-time model");
+  if (error_type < 0 || error_type > 4) return fail(ERIRT_E_ARG, "error_type must be 0 (truncated normal), 1 (unit normal), 2 (norm), 3 (tail) or 4 (skew)");
+  if (has_rt && error_type == 0 && !sigma2) return fail(ERIRT_E_ARG, "sigma2 is required for error_type 0");
+  const int64_t n = h->cfg.n_subj;
+  const int J = h->cfg.n_item;
+  if (h->cfg.n_feat > 0 && (!X || ldX < n * h->nb))
+    return fail(ERIRT_E_ARG, h->nb > 1 ? "X (leading dimension >= n_batch * n_subj) is required when n_feat > 0"
+                                       : "X (leading dimension >= n_subj) is required when n_feat > 0");
+  CU(cudaSetDevice(h->cfg.device));
+  if (int rc = clear_data(h)) return rc;
+  auto at = [](const double* p, int64_t off) { return p ? p + off : nullptr; };
+  for (int r = 0; r < h->nb; ++r)
+    if (int rc = generate_replica(h, r, theta + r * n, at(zeta, r * n), a + (int64_t)r * J, b + (int64_t)r * J, at(lambda, (int64_t)r * J),
+                                  at(sigma2, (int64_t)r * J), at(rho, (int64_t)r * J), at(X, r * n), ldX, error_type, seed + (uint64_t)r))
+      return rc;
+  return 0;
 }
 
 // The data set held by the handle (ingested or generated), back in Julia's column-major Float64 (logT as stored: f32-rounded in f32 mode)
@@ -890,23 +961,27 @@ extern "C" int erirt_get_data(erirt_handle* h, double* Y, int64_t ldY, double* l
   if (!h->data_set) return fail(ERIRT_E_STATE, "no data set: call erirt_set_data or erirt_generate_data first");
   const int64_t n = h->cfg.n_subj;
   const int J = h->cfg.n_item, Jp = h->L.Jp;
-  if ((Y && ldY < n) || (logT && ldT < n)) return fail(ERIRT_E_ARG, "leading dimension smaller than n_subj");
+  if ((Y && ldY < n * h->nb) || (logT && ldT < n * h->nb))
+    return fail(ERIRT_E_ARG, h->nb > 1 ? "leading dimension smaller than n_batch * n_subj" : "leading dimension smaller than n_subj");
   if (logT && h->cfg.model == ERIRT_MLIRT) return fail(ERIRT_E_ARG, "GibbsMlIrt has no response times");
   CU(cudaSetDevice(h->cfg.device));
   double* tmp = nullptr;
   CU(cudaMallocAsync((void**)&tmp, (size_t)n * J * sizeof(double), h->stream));
   cudaError_t e = cudaSuccess;
-  if (Y) {
-    tile_to_colmajor_kernel<uint8_t><<<1024, 256, 0, h->stream>>>(h->dY, n, J, Jp, tmp);
-    e = cudaMemcpy2DAsync(Y, ldY * sizeof(double), tmp, n * sizeof(double), n * sizeof(double), J, cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-  }
-  if (logT && e == cudaSuccess) {
-    with_real(h, [&](auto r) {
-      using R = decltype(r);
-      tile_to_colmajor_kernel<R><<<1024, 256, 0, h->stream>>>((const R*)h->dLogT, n, J, Jp, tmp);
-    });
-    e = cudaMemcpy2DAsync(logT, ldT * sizeof(double), tmp, n * sizeof(double), n * sizeof(double), J, cudaMemcpyDeviceToHost, h->stream);
+  for (int r = 0; r < h->nb && e == cudaSuccess; ++r) {  // replica r: rows [r n, (r+1) n)
+    if (Y) {
+      tile_to_colmajor_kernel<uint8_t><<<1024, 256, 0, h->stream>>>(h->dY + r * h->z.cells, n, J, Jp, tmp);
+      e = cudaMemcpy2DAsync(Y + r * n, ldY * sizeof(double), tmp, n * sizeof(double), n * sizeof(double), J, cudaMemcpyDeviceToHost, h->stream);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    }
+    if (logT && e == cudaSuccess) {
+      with_real(h, [&](auto rr) {
+        using R = decltype(rr);
+        tile_to_colmajor_kernel<R><<<1024, 256, 0, h->stream>>>((const R*)h->dLogT + r * h->z.cells, n, J, Jp, tmp);
+      });
+      e = cudaMemcpy2DAsync(logT + r * n, ldT * sizeof(double), tmp, n * sizeof(double), n * sizeof(double), J, cudaMemcpyDeviceToHost, h->stream);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);  // tmp is reused by the next replica
+    }
   }
   cudaFreeAsync(tmp, h->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
@@ -928,7 +1003,7 @@ extern "C" int erirt_set_data_y8(erirt_handle* h, const uint8_t* Y, int64_t ldY,
 // all-reduce the ingest constants over shards once, derive mean/std of logT
 static int finalize_constants(erirt_handle* h) {
   if (h->consts_final) return 0;
-  CU(cudaMemcpyAsync(h->dConsts, h->dConstsLocal, h->c_count * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
+  CU(cudaMemcpyAsync(h->dConsts, h->dConstsLocal, (size_t)h->z.consts * h->nb * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
   if (h->world > 1) {
     if (h->peer_ready) {
       peer_allreduce_kernel<<<1, 512, 0, h->stream>>>(h->dPeerBufs, h->dXseq, h->world, h->rank, h->xstride, h->dConsts, h->c_count, h->dStatus);
@@ -939,18 +1014,23 @@ static int finalize_constants(erirt_handle* h) {
       return fail(ERIRT_E_STATE, "sharded chain without a communicator: call erirt_peer_attach (or erirt_comm_init with an NCCL id) first");
     }
   }
-  std::vector<double> c(h->c_count);
-  CU(cudaMemcpyAsync(c.data(), h->dConsts, h->c_count * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  std::vector<double> c((size_t)h->z.consts * h->nb);
+  CU(cudaMemcpyAsync(c.data(), h->dConsts, c.size() * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
-  double s1 = 0, s2 = 0;
-  for (int j = 0; j < h->cfg.n_item; ++j) { s1 += c[h->c_T1 + j]; s2 += c[h->c_T2 + j]; }
-  const double n = (double)h->cfg.n_subj_total * h->cfg.n_item;
-  double d[4] = {0, 1, 0, 0};
-  if (h->cfg.model != ERIRT_MLIRT) {
-    d[0] = s1 / n;                                   // mean(Data.logT)   Draw.pl.jl:215
-    d[1] = std::sqrt((s2 - s1 * s1 / n) / (n - 1.0));  // std(Data.logT)
+  std::vector<double> derived;  // 4 per replica
+  for (int r = 0; r < h->nb; ++r) {
+    const double* cr = c.data() + r * h->z.consts;
+    double s1 = 0, s2 = 0;
+    for (int j = 0; j < h->cfg.n_item; ++j) { s1 += cr[h->c_T1 + j]; s2 += cr[h->c_T2 + j]; }
+    const double n = (double)h->cfg.n_subj_total * h->cfg.n_item;
+    double d[4] = {0, 1, 0, 0};
+    if (h->cfg.model != ERIRT_MLIRT) {
+      d[0] = s1 / n;                                   // mean(Data.logT)   Draw.pl.jl:215
+      d[1] = std::sqrt((s2 - s1 * s1 / n) / (n - 1.0));  // std(Data.logT)
+    }
+    derived.insert(derived.end(), d, d + 4);
   }
-  CU(cudaMemcpyAsync(h->dDerived, d, sizeof(d), cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMemcpyAsync(h->dDerived, derived.data(), derived.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   h->consts_final = true;
   return 0;
@@ -988,29 +1068,37 @@ static int param_slot(erirt_handle* h, int field, int* off, int* len) {
   return -1;
 }
 
+// A batch stacks replicas: a person field has n_batch * n_subj rows (column-major, replica r in rows [r n_subj, (r+1) n_subj)), a
+// parameter n_batch consecutive blocks of its standalone length.
 extern "C" int erirt_set_state(erirt_handle* h, int32_t field, const double* v, int64_t n) {
   if (!h || !v) return fail(ERIRT_E_ARG, "null argument");
   CU(cudaSetDevice(h->cfg.device));
   PersonField pf;
   int off, len;
+  const int64_t ns = h->cfg.n_subj;
   if (person_field(h, field, &pf)) {
-    const int64_t want = h->cfg.n_subj * pf.J;
+    const int64_t want = ns * pf.J * h->nb;
     if (n != want) return fail(ERIRT_E_ARG, "field %d expects %lld values, got %lld", field, (long long)want, (long long)n);
+    const int64_t stride = pf.J == 1 ? h->z.vec : h->z.cells;  // one replica's copy of the device field
     double* tmp;
-    CU(cudaMallocAsync((void**)&tmp, n * sizeof(double), h->stream));
-    cudaMemcpyAsync(tmp, v, n * sizeof(double), cudaMemcpyHostToDevice, h->stream);
-    with_real(h, [&](auto r) {
-      using R = decltype(r);
-      colmajor_to_tile_kernel<R><<<1024, 256, 0, h->stream>>>(tmp, h->cfg.n_subj, pf.J, pf.Jp, (R*)pf.p);
-    });
+    CU(cudaMallocAsync((void**)&tmp, ns * pf.J * sizeof(double), h->stream));
+    for (int r = 0; r < h->nb; ++r) {
+      cudaMemcpy2DAsync(tmp, ns * sizeof(double), v + r * ns, ns * h->nb * sizeof(double), ns * sizeof(double), pf.J, cudaMemcpyHostToDevice,
+                        h->stream);
+      with_real(h, [&](auto rr) {
+        using R = decltype(rr);
+        colmajor_to_tile_kernel<R><<<1024, 256, 0, h->stream>>>(tmp, ns, pf.J, pf.Jp, (R*)pf.p + r * stride);
+      });
+    }
     cudaFreeAsync(tmp, h->stream);
     cudaError_t e = cudaStreamSynchronize(h->stream);
     if (e != cudaSuccess) return fail(ERIRT_E_CUDA, "set_state: %s", cudaGetErrorString(e));
     return 0;
   }
   if (param_slot(h, field, &off, &len) == 0) {
-    if (n != len) return fail(ERIRT_E_ARG, "field %d expects %d values, got %lld", field, len, (long long)n);
-    if (len > 0) CU(cudaMemcpy(h->dParams + off, v, len * sizeof(double), cudaMemcpyHostToDevice));
+    if (n != (int64_t)len * h->nb) return fail(ERIRT_E_ARG, "field %d expects %lld values, got %lld", field, (long long)len * h->nb, (long long)n);
+    for (int r = 0; r < h->nb && len > 0; ++r)
+      CU(cudaMemcpy(h->dParams + r * h->z.params + off, v + (int64_t)r * len, len * sizeof(double), cudaMemcpyHostToDevice));
     return 0;
   }
   return fail(ERIRT_E_ARG, "unknown field %d", field);
@@ -1021,25 +1109,31 @@ extern "C" int erirt_get_state(erirt_handle* h, int32_t field, double* out, int6
   CU(cudaSetDevice(h->cfg.device));
   PersonField pf;
   int off, len;
+  const int64_t ns = h->cfg.n_subj;
   if (person_field(h, field, &pf)) {
-    const int64_t want = h->cfg.n_subj * pf.J;
+    const int64_t want = ns * pf.J * h->nb;
     if (n != want) return fail(ERIRT_E_ARG, "field %d expects %lld values, got %lld", field, (long long)want, (long long)n);
+    const int64_t stride = pf.J == 1 ? h->z.vec : h->z.cells;
     double* tmp;
-    CU(cudaMallocAsync((void**)&tmp, n * sizeof(double), h->stream));
-    with_real(h, [&](auto r) {
-      using R = decltype(r);
-      tile_to_colmajor_kernel<R><<<1024, 256, 0, h->stream>>>((const R*)pf.p, h->cfg.n_subj, pf.J, pf.Jp, tmp);
-    });
-    cudaMemcpyAsync(out, tmp, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
+    CU(cudaMallocAsync((void**)&tmp, ns * pf.J * sizeof(double), h->stream));
+    for (int r = 0; r < h->nb; ++r) {
+      with_real(h, [&](auto rr) {
+        using R = decltype(rr);
+        tile_to_colmajor_kernel<R><<<1024, 256, 0, h->stream>>>((const R*)pf.p + r * stride, ns, pf.J, pf.Jp, tmp);
+      });
+      cudaMemcpy2DAsync(out + r * ns, ns * h->nb * sizeof(double), tmp, ns * sizeof(double), ns * sizeof(double), pf.J, cudaMemcpyDeviceToHost,
+                        h->stream);
+    }
     cudaFreeAsync(tmp, h->stream);
     cudaError_t e = cudaStreamSynchronize(h->stream);
     if (e != cudaSuccess) return fail(ERIRT_E_CUDA, "get_state: %s", cudaGetErrorString(e));
     return 0;
   }
   if (param_slot(h, field, &off, &len) == 0) {
-    if (n != len) return fail(ERIRT_E_ARG, "field %d expects %d values, got %lld", field, len, (long long)n);
+    if (n != (int64_t)len * h->nb) return fail(ERIRT_E_ARG, "field %d expects %lld values, got %lld", field, (long long)len * h->nb, (long long)n);
     CU(cudaStreamSynchronize(h->stream));
-    if (len > 0) CU(cudaMemcpy(out, h->dParams + off, len * sizeof(double), cudaMemcpyDeviceToHost));
+    for (int r = 0; r < h->nb && len > 0; ++r)
+      CU(cudaMemcpy(out + (int64_t)r * len, h->dParams + r * h->z.params + off, len * sizeof(double), cudaMemcpyDeviceToHost));
     return 0;
   }
   return fail(ERIRT_E_ARG, "unknown field %d", field);
@@ -1095,8 +1189,9 @@ static GlobalArgs make_global_args(erirt_handle* h, int stage) {
     // have flushed the instruction caches: more than one tile per CTA.  Behind a one-round launch (the small problems) it would only
     // delay the real pass.
     const bool fast = runs_fast_kernel(h, stage);
+    // A replica batch does not rehearse (its CTAs would fetch the same code in parallel).
     const int64_t tiles = h->n_pad / (fast ? h->S.P : h->S_gen.P);
-    A.rehearse = tiles > (fast ? h->grid : h->grid_gen) ? 1 : 0;
+    A.rehearse = h->nb == 1 && tiles > (fast ? h->grid : h->grid_gen) ? 1 : 0;
   }
   A.tile_ctr = h->dTileCtr;
   A.sweep_ctr = h->dSweep;
@@ -1149,12 +1244,15 @@ static cudaError_t launch_chain_kernel(const void* kfn, dim3 grid, dim3 block, v
   return cudaLaunchKernelExC(&lc, kfn, args);
 }
 
+// A replica batch launches the BATCH instantiations of the kernels (layout.cuh BatchArgs): the person grid gains a replica dimension,
+// the global kernel one CTA per replica.
 static int launch_person(erirt_handle* h, int stage) {
   const void* kfn = person_kernel_for(h, stage);
   return with_real(h, [&](auto r) -> int {
     PersonArgs<decltype(r)> A = make_person_args<decltype(r)>(h, stage);
-    void* args[] = {&A};
-    CU(launch_chain_kernel(kfn, dim3(stage == 0 ? h->grid : h->grid_gen), dim3(CTA_THREADS), args, A.S.total, h->stream));
+    BatchArgs<PersonArgs<decltype(r)>> B{A, h->z, h->cfg.seed, h->cfg.chain};  // A: replica 0
+    void* args[] = {h->nb > 1 ? (void*)&B : (void*)&A};
+    CU(launch_chain_kernel(kfn, dim3(stage == 0 ? h->grid : h->grid_gen, h->nb), dim3(CTA_THREADS), args, A.S.total, h->stream));
     return 0;
   });
 }
@@ -1164,9 +1262,10 @@ static int launch_global(erirt_handle* h, int stage) {
   if (h->comm && !h->peer_ready)  // fallback: the exchange is otherwise fused into the kernel below
     NC(nccl::all_reduce(h->dStats, h->dStats, (size_t)h->L.s_count, nccl::kFloat64, nccl::kSum, h->comm, h->stream));
   GlobalArgs G = make_global_args(h, stage);
+  BatchArgs<GlobalArgs> B{G, h->z, h->cfg.seed, h->cfg.chain};
   const size_t gsm = (size_t)(h->L.s_count + 2 + (h->L.F + 1) * (h->L.F + 1) + 5 * h->L.Jp) * sizeof(double);  // staged statistics, X'X, raw variates
-  void* args[] = {&G};
-  CU(launch_chain_kernel((const void*)global_draw_kernel, dim3(1), dim3(G_THREADS), args, gsm, h->stream));
+  void* args[] = {h->nb > 1 ? (void*)&B : (void*)&G};
+  CU(launch_chain_kernel(global_kernel_for(h), dim3(h->nb), dim3(G_THREADS), args, gsm, h->stream));
   return 0;
 }
 
@@ -1200,8 +1299,8 @@ extern "C" int erirt_sample(erirt_handle* h, int64_t n_sweeps) {
   int rc = finalize_constants(h);
   if (rc) return rc;
   if (!h->prologue_done) {
-    CU(cudaMemsetAsync(h->dSweep, 0, sizeof(uint32_t), h->stream));
-    CU(cudaMemsetAsync(h->dStats, 0, (h->L.s_count + 2) * sizeof(double), h->stream));
+    CU(cudaMemsetAsync(h->dSweep, 0, h->nb * sizeof(uint32_t), h->stream));
+    CU(cudaMemsetAsync(h->dStats, 0, h->z.stats * h->nb * sizeof(double), h->stream));
     rc = enqueue_step(h, true);  // P(0), G(1)
     if (rc) return rc;
     h->prologue_done = true;
@@ -1264,10 +1363,14 @@ extern "C" int erirt_sample(erirt_handle* h, int64_t n_sweeps) {
     h->person_ms = tot / (double)(h->kev_used / 2);
   }
   h->sweeps_done += n_sweeps;
-  int status = 0;
-  CU(cudaMemcpy(&status, h->dStatus, sizeof(int), cudaMemcpyDeviceToHost));
-  if (status <= -1000) return fail(ERIRT_E_NCCL, "peer exchange timed out waiting for rank %d (a GPU of the sharded chain is gone); the chain is unusable", -1000 - status);
-  if (status != 0) return fail(ERIRT_E_NUMERIC, "a posterior covariance was not positive definite at sweep %d (PosDefException in the reference)", status);
+  std::vector<int> status(h->nb);  // sticky, one per replica
+  CU(cudaMemcpy(status.data(), h->dStatus, h->nb * sizeof(int), cudaMemcpyDeviceToHost));
+  if (status[0] <= -1000) return fail(ERIRT_E_NCCL, "peer exchange timed out waiting for rank %d (a GPU of the sharded chain is gone); the chain is unusable", -1000 - status[0]);
+  for (int r = 0; r < h->nb; ++r) {
+    if (status[r] == 0) continue;
+    if (h->nb == 1) return fail(ERIRT_E_NUMERIC, "a posterior covariance was not positive definite at sweep %d (PosDefException in the reference)", status[r]);
+    return fail(ERIRT_E_NUMERIC, "replica %d: a posterior covariance was not positive definite at sweep %d (PosDefException in the reference)", r, status[r]);
+  }
   return 0;
 }
 
@@ -1310,6 +1413,7 @@ __global__ void trace_gather_kernel(double* __restrict__ dst, int64_t n_iter, in
 struct TraceSource {
   const double* small;
   int64_t small0, small_w;
+  int64_t small_stride;  // replica batch: length of one replica's copy of `small`
   int pfield;
   int64_t pcol0, pn;
   bool person_cols;  // [first_col, first_col + n_cols) includes person columns
@@ -1323,25 +1427,26 @@ static int trace_source(const erirt_handle* h, int which, int64_t first_col, int
   if (first_col < 0 || n_cols < 0 || first_col + n_cols > W) return fail(ERIRT_E_ARG, "columns [%lld,%lld) outside [0,%lld)", (long long)first_col, (long long)(first_col + n_cols), (long long)W);
   const int64_t N = h->cfg.n_subj, J = h->cfg.n_item;
   // column ranges: person block [0,N) for ra/rt, trailing nu block for LatentQr qr
-  TraceSource s{nullptr, 0, 0, 0, -1, 0, false};
-  if (which == ERIRT_TRACE_RA) { s.small = h->dTrRa; s.small0 = N; s.small_w = 2 * J; s.pfield = 0; s.pcol0 = 0; s.pn = N; }
-  else if (which == ERIRT_TRACE_RT) { s.small = h->dTrRt; s.small0 = N; s.small_w = 2 * J; s.pfield = 1; s.pcol0 = 0; s.pn = N; }
+  TraceSource s{nullptr, 0, 0, 0, 0, -1, 0, false};
+  if (which == ERIRT_TRACE_RA) { s.small = h->dTrRa; s.small0 = N; s.small_w = 2 * J; s.small_stride = h->z.tr_items; s.pfield = 0; s.pcol0 = 0; s.pn = N; }
+  else if (which == ERIRT_TRACE_RT) { s.small = h->dTrRt; s.small0 = N; s.small_w = 2 * J; s.small_stride = h->z.tr_items; s.pfield = 1; s.pcol0 = 0; s.pn = N; }
   else if (which == ERIRT_TRACE_QR) {
-    s.small = h->dTrQr; s.small_w = h->qw;
+    s.small = h->dTrQr; s.small_w = h->qw; s.small_stride = h->z.tr_qr;
     if (h->cfg.model == ERIRT_RTIRT_LATENTQR) { s.pfield = 2; s.pcol0 = h->qw; s.pn = N; }
-  } else { s.small = h->dTrLl; s.small_w = 1; }
+  } else { s.small = h->dTrLl; s.small_w = 1; s.small_stride = h->z.tr_ll; }
   s.person_cols = first_col < s.pcol0 + s.pn && first_col + n_cols > s.pcol0;
   *src = s;
   return 0;
 }
 
-// Columns [col0, col0 + nc) of chain l into dst [nc][n_iter] (trace_gather_kernel)
-static void gather_trace(erirt_handle* h, const TraceSource& s, double* dst, int64_t col0, int64_t nc, int64_t l) {
+// Columns [col0, col0 + nc) of chain l of replica rep into dst [nc][n_iter] (trace_gather_kernel)
+static void gather_trace(erirt_handle* h, const TraceSource& s, int rep, double* dst, int64_t col0, int64_t nc, int64_t l) {
   const int64_t nIter = h->cfg.n_iter;
   const int grid = (int)std::min<int64_t>((nIter * nc + 255) / 256, (int64_t)h->sm_count * 16);
+  const double* small = s.small + rep * s.small_stride;
   with_real(h, [&](auto r) {
     using R = decltype(r);
-    trace_gather_kernel<R><<<grid, 256, 0, h->stream>>>(dst, nIter, nc, col0, l, h->cfg.n_chain, h->sweeps_done, s.small, s.small0, s.small_w,
+    trace_gather_kernel<R><<<grid, 256, 0, h->stream>>>(dst, nIter, nc, col0, l, h->cfg.n_chain, h->sweeps_done, small, s.small0, s.small_w,
                                                          (const R*)h->dPtrace, s.pfield, s.pcol0, s.pn, h->n_pad);
   });
 }
@@ -1360,13 +1465,16 @@ extern "C" int erirt_get_trace(erirt_handle* h, int32_t which, int64_t first_col
   double* tmp = nullptr;
   CU(cudaMallocAsync((void**)&tmp, (size_t)nIter * chunk_cols * sizeof(double), h->stream));
   cudaError_t e = cudaSuccess;
-  for (int64_t l = 0; l < nChain && e == cudaSuccess; ++l)
-    for (int64_t c0 = 0; c0 < n_cols && e == cudaSuccess; c0 += chunk_cols) {
-      const int64_t nc = std::min(chunk_cols, n_cols - c0);
-      gather_trace(h, src, tmp, first_col + c0, nc, l);
-      e = cudaMemcpyAsync(out + nIter * (c0 + n_cols * l), tmp, (size_t)nIter * nc * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);  // tmp is reused by the next chunk
-    }
+  // a batch appends the replica as the last axis: out[m + n_iter * (c + n_cols * (l + n_chain * r))]
+  for (int r = 0; r < h->nb && e == cudaSuccess; ++r)
+    for (int64_t l = 0; l < nChain && e == cudaSuccess; ++l)
+      for (int64_t c0 = 0; c0 < n_cols && e == cudaSuccess; c0 += chunk_cols) {
+        const int64_t nc = std::min(chunk_cols, n_cols - c0);
+        gather_trace(h, src, r, tmp, first_col + c0, nc, l);
+        e = cudaMemcpyAsync(out + nIter * (c0 + n_cols * (l + nChain * r)), tmp, (size_t)nIter * nc * sizeof(double), cudaMemcpyDeviceToHost,
+                            h->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);  // tmp is reused by the next chunk
+      }
   cudaFreeAsync(tmp, h->stream);
   if (e != cudaSuccess) return fail(ERIRT_E_CUDA, "get_trace: %s", cudaGetErrorString(e));
   return 0;
@@ -1445,11 +1553,13 @@ extern "C" int erirt_trace_ess_rhat(erirt_handle* h, int32_t which, int64_t firs
   double* tmp = nullptr;
   CU(cudaMallocAsync((void**)&tmp, (size_t)nIter * chunk_cols * nChain * sizeof(double), h->stream));
   int rc = 0;
-  for (int64_t c0 = 0; c0 < n_cols && rc == 0; c0 += chunk_cols) {
-    const int64_t nc = std::min(chunk_cols, n_cols - c0);
-    for (int64_t l = 0; l < nChain; ++l) gather_trace(h, src, tmp + nIter * nc * l, first_col + c0, nc, l);
-    rc = run_ess_rhat(tmp, nIter, nc, nChain, skip, done_iter - skip, h->stream, ess + c0, rhat + c0);
-  }
+  // a batch returns n_batch * n_cols results, replica-major
+  for (int r = 0; r < h->nb && rc == 0; ++r)
+    for (int64_t c0 = 0; c0 < n_cols && rc == 0; c0 += chunk_cols) {
+      const int64_t nc = std::min(chunk_cols, n_cols - c0);
+      for (int64_t l = 0; l < nChain; ++l) gather_trace(h, src, r, tmp + nIter * nc * l, first_col + c0, nc, l);
+      rc = run_ess_rhat(tmp, nIter, nc, nChain, skip, done_iter - skip, h->stream, ess + r * n_cols + c0, rhat + r * n_cols + c0);
+    }
   cudaFreeAsync(tmp, h->stream);
   cudaStreamSynchronize(h->stream);
   return rc;
@@ -1463,18 +1573,22 @@ extern "C" int erirt_get_moments(erirt_handle* h, int32_t field, double* mean, d
   if (nu_cell && !h->dNuMom) return fail(ERIRT_E_STATE, "the running moments of the N x J weights of CrossQr need erirt_config.nu_cell_moments = 1");
   PersonField pf;
   person_field(h, field, &pf);
-  if (n != h->cfg.n_subj * pf.J) return fail(ERIRT_E_ARG, nu_cell ? "expects n_subj * n_item values" : "expects n_subj values");
+  if (n != h->cfg.n_subj * pf.J * h->nb)
+    return fail(ERIRT_E_ARG, nu_cell ? "expects n_subj * n_item values" : (h->nb > 1 ? "expects n_batch * n_subj values" : "expects n_subj values"));
   CU(cudaSetDevice(h->cfg.device));
   CU(cudaStreamSynchronize(h->stream));
   const int64_t nChain = h->cfg.n_chain;
   const int64_t first = (int64_t)h->cfg.n_burnin * nChain;  // sweeps with m > n_burnin
   const int64_t cnt = h->sweeps_done > first ? h->sweeps_done - first : 0;
-  // running sum and sum of squares of the field, laid out like it: [2][n_pad][Jp]
-  const double* s1 = nu_cell ? h->dNuMom : h->dMom + (size_t)(2 * slot) * h->n_pad;
   // mean and SD are finished on the device and copied straight into the caller's buffers (pinned buffers make this a plain DMA)
   double* tmp = nullptr;
   CU(cudaMallocAsync((void**)&tmp, (size_t)2 * n * sizeof(double), h->stream));
-  tile_moments_kernel<<<1024, 256, 0, h->stream>>>(s1, s1 + (size_t)h->n_pad * pf.Jp, h->cfg.n_subj, pf.J, pf.Jp, (double)cnt, tmp, tmp + n);
+  const int64_t nr = n / h->nb;  // values of one replica
+  for (int r = 0; r < h->nb; ++r) {
+    // running sum and sum of squares of the field, laid out like it: [2][n_pad][Jp]
+    const double* s1 = nu_cell ? h->dNuMom : h->dMom + r * h->z.mom + (size_t)(2 * slot) * h->n_pad;
+    tile_moments_kernel<<<1024, 256, 0, h->stream>>>(s1, s1 + (size_t)h->n_pad * pf.Jp, h->cfg.n_subj, pf.J, pf.Jp, (double)cnt, tmp + r * nr, tmp + n + r * nr);
+  }
   cudaError_t e = cudaMemcpyAsync(mean, tmp, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
   if (e == cudaSuccess && sd) e = cudaMemcpyAsync(sd, tmp + n, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
   cudaFreeAsync(tmp, h->stream);
@@ -1489,10 +1603,10 @@ extern "C" int erirt_loglik_current(erirt_handle* h, double* out) {
   CU(cudaSetDevice(h->cfg.device));
   int rc = finalize_constants(h);
   if (rc) return rc;
-  if (!h->prologue_done) CU(cudaMemsetAsync(h->dStats, 0, (h->L.s_count + 2) * sizeof(double), h->stream));
+  if (!h->prologue_done) CU(cudaMemsetAsync(h->dStats, 0, h->z.stats * h->nb * sizeof(double), h->stream));
   if ((rc = launch_person(h, 3))) return rc;
   if ((rc = launch_global(h, 3))) return rc;
-  CU(cudaMemcpyAsync(out, h->dLlOut, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaMemcpyAsync(out, h->dLlOut, h->nb * sizeof(double), cudaMemcpyDeviceToHost, h->stream));  // one per replica
   CU(cudaStreamSynchronize(h->stream));
   return 0;
 }
@@ -1528,10 +1642,15 @@ extern "C" int erirt_get_stats(erirt_handle* h, erirt_stats* out) {
   if (h->cfg.model == ERIRT_RTIRT_CROSSQR) per_cell = (1 + 3 * r) + (1 + 4 * r);  // K_a: Y, logT, omega, nu; K_b: Y, logT, nu r/w, omega w
   int nv = has_rt ? 2 : 1;
   if (h->cfg.model == ERIRT_RTIRT_LATENTQR) nv = 3;
-  out->bytes_per_sweep = N * J * per_cell + N * r * (2 * nv + F);
+  out->bytes_per_sweep = (N * J * per_cell + N * r * (2 * nv + F)) * h->nb;  // a batch reports totals over its replicas
   double d[2] = {0, 0};
   CU(cudaStreamSynchronize(h->stream));
-  CU(cudaMemcpy(d, h->dStats + h->L.s_count, sizeof(d), cudaMemcpyDeviceToHost));
+  for (int b = 0; b < h->nb; ++b) {
+    double db[2];
+    CU(cudaMemcpy(db, h->dStats + b * h->z.stats + h->L.s_count, sizeof(db), cudaMemcpyDeviceToHost));
+    d[0] += db[0];
+    d[1] += db[1];
+  }
   out->pg_deferred_frac = d[1] > 0 ? d[0] / d[1] : 0.0;
   return 0;
 }
@@ -1585,12 +1704,18 @@ static CkHeader ck_header(erirt_handle* h) {
   for (const CkSeg& sg : ck_segments(h)) H.payload_bytes += (int64_t)sg.bytes;
   return H;
 }
+// checkpoints, sharding and the peer exchange are per chain: a replica batch refuses them
+static int refuse_batch(const erirt_handle* h, const char* what) {
+  return fail(ERIRT_E_UNSUPPORTED, "%s is not supported on a replica batch (n_batch = %d)", what, h->nb);
+}
 extern "C" int64_t erirt_checkpoint_size(erirt_handle* h) {
   if (!h) { fail(ERIRT_E_ARG, "null handle"); return -1; }
+  if (h->nb > 1) return refuse_batch(h, "erirt_checkpoint_size");
   return (int64_t)sizeof(CkHeader) + ck_header(h).payload_bytes;
 }
 extern "C" int erirt_checkpoint_save(erirt_handle* h, void* buf, int64_t size) {
   if (!h || !buf) return fail(ERIRT_E_ARG, "null argument");
+  if (h->nb > 1) return refuse_batch(h, "erirt_checkpoint_save");
   const CkHeader H = ck_header(h);
   const int64_t need = (int64_t)sizeof(CkHeader) + H.payload_bytes;
   if (size < need) return fail(ERIRT_E_ARG, "checkpoint buffer of %lld bytes, %lld needed", (long long)size, (long long)need);
@@ -1607,6 +1732,7 @@ extern "C" int erirt_checkpoint_save(erirt_handle* h, void* buf, int64_t size) {
 }
 extern "C" int erirt_checkpoint_load(erirt_handle* h, const void* buf, int64_t size) {
   if (!h || !buf) return fail(ERIRT_E_ARG, "null argument");
+  if (h->nb > 1) return refuse_batch(h, "erirt_checkpoint_load");
   if (size < (int64_t)sizeof(CkHeader)) return fail(ERIRT_E_ARG, "checkpoint shorter than its header");
   CkHeader H;
   memcpy(&H, buf, sizeof(H));
@@ -1648,6 +1774,7 @@ extern "C" int erirt_nccl_unique_id(void* id128) {
 }
 extern "C" int erirt_comm_init(erirt_handle* h, int32_t rank, int32_t world, const void* id128) {
   if (!h) return fail(ERIRT_E_ARG, "null argument");
+  if (h->nb > 1) return refuse_batch(h, "erirt_comm_init");
   if (world < 1 || rank < 0 || rank >= world) return fail(ERIRT_E_ARG, "bad rank/world");
   if (h->prologue_done) return fail(ERIRT_E_STATE, "erirt_comm_init must precede erirt_sample");
   CU(cudaSetDevice(h->cfg.device));
@@ -1666,6 +1793,7 @@ extern "C" int erirt_comm_init(erirt_handle* h, int32_t rank, int32_t world, con
 
 extern "C" int erirt_peer_export(erirt_handle* h, void* ipc_handle64) {
   if (!h || !ipc_handle64) return fail(ERIRT_E_ARG, "null argument");
+  if (h->nb > 1) return refuse_batch(h, "erirt_peer_export");
   if (h->world < 2) return fail(ERIRT_E_STATE, "erirt_peer_export needs erirt_comm_init with world >= 2 first");
   if (h->prologue_done) return fail(ERIRT_E_STATE, "erirt_peer_export must precede erirt_sample");
   static_assert(sizeof(cudaIpcMemHandle_t) == 64, "CUDA IPC handle size");
@@ -1715,6 +1843,7 @@ extern "C" int erirt_peer_export(erirt_handle* h, void* ipc_handle64) {
 }
 extern "C" int erirt_peer_attach(erirt_handle* h, const void* ipc_handles) {
   if (!h || !ipc_handles) return fail(ERIRT_E_ARG, "null argument");
+  if (h->nb > 1) return refuse_batch(h, "erirt_peer_attach");
   if (!h->xbuf) return fail(ERIRT_E_STATE, "erirt_peer_export has not been called");
   if (h->prologue_done) return fail(ERIRT_E_STATE, "erirt_peer_attach must precede erirt_sample");
   CU(cudaSetDevice(h->cfg.device));
@@ -1757,6 +1886,7 @@ extern "C" int erirt_peer_attach(erirt_handle* h, const void* ipc_handles) {
 
 extern "C" int erirt_peer_detach(erirt_handle* h) {
   if (!h) return fail(ERIRT_E_ARG, "null handle");
+  if (h->nb > 1) return refuse_batch(h, "erirt_peer_detach");
   CU(cudaSetDevice(h->cfg.device));
   CU(cudaStreamSynchronize(h->stream));  // (the peer mappings stay open with the cached exchange buffer, for the next handle)
   // Later sweeps go through ncclAllReduce when the chain has an NCCL communicator; a chain created with

@@ -425,7 +425,10 @@ __device__ inline void global_raw_variates(const GlobalArgs& A, uint32_t s, doub
   }
 }
 
-__global__ void __maxnreg__(80) global_draw_kernel(const GlobalArgs A) {
+// BATCH: the replica-batch instantiation (layout.cuh BatchArgs), one CTA per replica
+template <bool BATCH = false>
+__global__ void __maxnreg__(80) global_draw_kernel(KernelArgs<GlobalArgs, BATCH> A) {
+  if constexpr (BATCH) to_replica(A, blockIdx.x);
 #ifdef ERIRT_TICKS
   const long long _g0 = clock64();
   if (threadIdx.x == 0) g_g0 = _g0;

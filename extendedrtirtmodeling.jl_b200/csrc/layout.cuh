@@ -1,6 +1,7 @@
 // layout.cuh -- device data layout shared by the kernels and the host orchestration (DESIGN.md "Data layout in HBM").
 #pragma once
 #include <cstdint>
+#include <type_traits>
 #include "rng.cuh"
 
 namespace erirt {
@@ -176,5 +177,98 @@ struct GlobalArgs {
   uint32_t* xseq;            // exchanges completed so far (identical on every GPU)
   int world, rank, xstride;
 };
+
+// consts vector of a handle (f64): T1[Jp] T2[Jp] K0[Jp] XtX[MAXD*MAXD/4 >= (F+1)^2] sums[2]
+inline int consts_count(const Layout& L) { return 3 * L.Jp + MAXD * MAXD / 4 + 2; }
+
+// ---- replica batches (DESIGN.md 6.6) ----
+// A batched handle holds n_batch independent problems of one configuration.  Each of its device buffers is n_batch copies of the
+// standalone buffer, back to back; these are the lengths of one copy (elements of the buffer's type; Y: bytes).  The sweep,
+// tile and status counters are one element per replica.
+struct ReplicaSizes {
+  int64_t cells;     // Y, logT, omega: n_pad * Jp
+  int64_t vec;       // theta, zeta, nu: n_pad
+  int64_t x;         // X [max(F,1)][n_pad]
+  int64_t mom;       // running moments [6][n_pad]
+  int64_t params;    // p_count
+  int64_t stats;     // s_count + 2 (statistics and the last sweep's PG diagnostics); stats_prev alike
+  int64_t consts;    // consts_count
+  int64_t derived;   // mean and sd of logT (4)
+  int64_t tr_items;  // [cap][2J], trace of a, b and of lambda, sigma2
+  int64_t tr_qr;     // [cap][qw]
+  int64_t tr_ll;     // [cap]
+};
+inline ReplicaSizes replica_sizes(int64_t n_pad, const Layout& L, int cap, int qw) {
+  ReplicaSizes z;
+  z.cells = n_pad * L.Jp;
+  z.vec = n_pad;
+  z.x = n_pad * (L.F > 0 ? L.F : 1);
+  z.mom = 6 * n_pad;
+  z.params = L.p_count;
+  z.stats = L.s_count + 2;
+  z.consts = consts_count(L);
+  z.derived = 4;
+  z.tr_items = (int64_t)cap * 2 * L.J;
+  z.tr_qr = (int64_t)cap * qw;
+  z.tr_ll = cap;
+  return z;
+}
+
+// Kernel parameters of a replica-batch launch: the arguments of replica 0's standalone launch (its key excepted), the replica sizes,
+// and seed and chain, from which replica r derives its key make_key(seed + r, chain).  The person launch is a (gx, n_batch) grid and
+// the global launch n_batch CTAs.
+template <typename Args>
+struct BatchArgs : Args {
+  ReplicaSizes z;
+  uint64_t seed;
+  uint32_t chain;
+};
+// The parameter of a sweep kernel: the standalone arguments, or those of a batch (the BATCH instantiation)
+template <typename Args, bool BATCH>
+using KernelArgs = typename std::conditional<BATCH, BatchArgs<Args>, const Args>::type;
+
+// Replica r's standalone arguments, in place, once at kernel entry: every pointer moves by r copies, and every index inside the kernels
+// stays as it is.  The Cross-family buffers (nu_cell, nu_mom) and the person trace are not part of a batch and stay null.  The key
+// schedule of replica r is built here, in registers: the constant bank cannot be indexed by the replica without serialising the hot
+// Philox rounds.
+template <typename R>
+__device__ __forceinline__ void to_replica(BatchArgs<PersonArgs<R>>& A, uint32_t r) {
+  const ReplicaSizes& z = A.z;
+  A.Y += r * z.cells;
+  A.logT += r * z.cells;
+  A.omega += r * z.cells;
+  A.theta += r * z.vec;
+  A.zeta += r * z.vec;
+  A.nu += r * z.vec;
+  A.X += r * z.x;
+  A.mom += r * z.mom;
+  A.params += r * z.params;
+  A.stats += r * z.stats;
+  A.sweep_ctr += r;
+  A.tile_ctr += r;
+  A.status += r;
+  A.key = make_key(A.seed + r, A.chain);
+  A.sched = make_sched(A.key);
+}
+__device__ __forceinline__ void to_replica(BatchArgs<GlobalArgs>& A, uint32_t r) {
+  const ReplicaSizes& z = A.z;
+  A.params += r * z.params;
+  A.stats += r * z.stats;
+  if (A.stats_prev) A.stats_prev += r * z.stats;
+  A.tile_ctr += r;
+  A.sweep_ctr += r;
+  A.T1 += r * z.consts;
+  A.T2 += r * z.consts;
+  A.K0 += r * z.consts;
+  A.XtX += r * z.consts;
+  A.consts += r * z.derived;
+  A.tr_items_ra += r * z.tr_items;
+  A.tr_items_rt += r * z.tr_items;
+  A.tr_qr += r * z.tr_qr;
+  A.tr_ll += r * z.tr_ll;
+  A.status += r;
+  A.ll_out += r;
+  A.key = make_key(A.seed + r, A.chain);
+}
 
 }  // namespace erirt

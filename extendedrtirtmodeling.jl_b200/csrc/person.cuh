@@ -270,8 +270,10 @@ __device__ __forceinline__ void flush_to_stats(const PersonArgs<R>& A, int J, in
 
 // FAM = 0: the one-launch-per-sweep models (MlIrt, RtIrt, RtIrtNull, Latent, LatentQr) -- the hot configuration, with the
 // Cross-family / evaluation code compiled out; FAM = 1: everything (Cross, CrossQr stages 1/2, stage 3 evaluation).
-template <typename R, int TPP, int FAM>
-__global__ void __launch_bounds__(CTA_THREADS, (sizeof(R) == 8 ? min_ctas_f64<TPP>() : min_ctas_per_sm<TPP>())) person_sweep_kernel(const PersonArgs<R> A) {
+// BATCH: the replica-batch instantiation (layout.cuh BatchArgs), grid (gx, n_batch) with the replica in blockIdx.y
+template <typename R, int TPP, int FAM, bool BATCH = false>
+__global__ void __launch_bounds__(CTA_THREADS, (sizeof(R) == 8 ? min_ctas_f64<TPP>() : min_ctas_per_sm<TPP>())) person_sweep_kernel(KernelArgs<PersonArgs<R>, BATCH> A) {
+  if constexpr (BATCH) to_replica(A, blockIdx.y);
   extern __shared__ __align__(128) unsigned char smem[];
   constexpr int P = CTA_THREADS / TPP;
   constexpr bool F32 = sizeof(R) == 4;

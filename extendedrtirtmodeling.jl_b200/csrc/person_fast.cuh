@@ -39,8 +39,10 @@ __device__ unsigned long long g_ticks[PF_NTICK];
 __device__ __forceinline__ uint32_t y_nibble(uint32_t yw) { return (yw * 0x01020408u) >> 24; }  // bytes 0/1 -> 4-bit index
 
 // MODEL is a template parameter: each instantiation carries the code of one model only (less code to fetch, no model branches)
-template <int TPP, int MODEL>
-__global__ void __launch_bounds__(CTA_THREADS, min_ctas_per_sm<TPP>()) person_sweep_fast_kernel(const PersonArgs<float> A) {
+// BATCH: the replica-batch instantiation (layout.cuh BatchArgs), grid (gx, n_batch) with the replica in blockIdx.y
+template <int TPP, int MODEL, bool BATCH = false>
+__global__ void __launch_bounds__(CTA_THREADS, min_ctas_per_sm<TPP>()) person_sweep_fast_kernel(KernelArgs<PersonArgs<float>, BATCH> A) {
+  if constexpr (BATCH) to_replica(A, blockIdx.y);
   extern __shared__ __align__(128) unsigned char smem[];
   constexpr int P = CTA_THREADS / TPP;
   typedef float R;

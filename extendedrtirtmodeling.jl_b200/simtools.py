@@ -43,10 +43,22 @@ def _field(P, name):
 
 
 def runSimulation(Cond, truePara, Para=("a", "b", "λ", "σ²t"), funcData=simulate.setDataRtIrt, funcGibbs=api.GibbsRtIrt,
-                  typeName="norm", rank=None, world=None, seed=1234, device=None, **sample_kwargs):
+                  typeName="norm", rank=None, world=None, seed=1234, device=None, batch=None, **sample_kwargs):
     """src/SimTools.jl:457-495.  Returns {"True": {p: vector}, 1: {p: posterior mean, "Dic": [DIC], "Diag": {...}}, ..., nRep: {...}}.
     Replication r (1-based) runs on rank (r-1) mod world; with torch.distributed initialised the per-rank results are
-    all-gathered so every rank returns the full Dict.  `sample_kwargs` go to api.sample (dtype, person_trace, ...)."""
+    all-gathered so every rank returns the full Dict.  `sample_kwargs` go to api.sample (dtype, person_trace, ...).
+    batch=k: each rank runs its replications as replica batches of at most k (api.sampleBatch, one GPU launch sequence per
+    batch; not for the Cross family).  A batch keeps no person trace, and the person trace changes the Dict (checkConvergence
+    counts the traced theta / zeta columns, and Post.mean.theta feeds D-hat), so batch=k requires person_trace=False and raises
+    ValueError otherwise, before any GPU work.  Replication `run` keeps its seeds (sampler seed + run, data seed + run, initial
+    values seed + 7919 run), so the Dict is the one batch=None returns with person_trace=False; a batch needs consecutive sampler
+    seeds, so with batch the replications are dealt to the ranks in contiguous blocks instead of round robin."""
+    if batch is not None:
+        if sample_kwargs.get("person_trace", None) is not False:
+            raise ValueError("runSimulation(batch=k) keeps no person trace: pass person_trace=False (the sequential run with "
+                             "person_trace=False returns the same Dict; its default traces theta / zeta and counts them in Diag)")
+        if int(batch) < 1:
+            raise ValueError("batch must be a positive number of replications")
     dist = None
     if rank is None or world is None:
         try:
@@ -68,22 +80,42 @@ def runSimulation(Cond, truePara, Para=("a", "b", "λ", "σ²t"), funcData=simul
             pass
     Run = {"True": {p: _field(truePara, p).ravel().copy() for p in Para}}
     mine = {}
-    for run in range(1, Cond.nRep + 1):
-        if (run - 1) % world != rank:
-            continue
+
+    def setup(run):
         try:
             Data = funcData(Cond, truePara, type=typeName, rng=seed + run)
         except TypeError:  # generators without error types (setDataRtIrt, setDataRtIrtNull, setDataMlIrt)
             Data = funcData(Cond, truePara, rng=seed + run)
-        MCMC = funcGibbs(Cond, Data=Data, truePara=truePara, rng=seed + 7919 * run)
-        api.sample(MCMC, seed=seed + run, device=device, **sample_kwargs)
+        return funcGibbs(Cond, Data=Data, truePara=truePara, rng=seed + 7919 * run)
+
+    def summary(MCMC, dic):
         Post = {p: _field(MCMC.Post.mean, p).copy() for p in Para}
-        try:
-            Post["Dic"] = [api.getDic(MCMC, dtype=sample_kwargs.get("dtype", "f64"), device=device).DIC]
-        except Exception:  # CrossQr has no D-hat (nu_ij is not traced)
-            Post["Dic"] = [float("nan")]
+        Post["Dic"] = [dic]
         Post["Diag"] = checkConvergence(MCMC, device=device)  # ESS / R-hat by the CUDA kernel on the GPU that sampled
-        mine[run] = Post
+        return Post
+
+    dtype = sample_kwargs.get("dtype", "f64")
+    if batch is None:
+        for run in range(1, Cond.nRep + 1):
+            if (run - 1) % world != rank:
+                continue
+            MCMC = setup(run)
+            api.sample(MCMC, seed=seed + run, device=device, **sample_kwargs)
+            try:
+                dic = api.getDic(MCMC, dtype=dtype, device=device).DIC
+            except Exception:  # CrossQr has no D-hat (nu_ij is not traced)
+                dic = float("nan")
+            mine[run] = summary(MCMC, dic)
+    else:
+        per = -(-Cond.nRep // world)
+        runs = list(range(1 + rank * per, 1 + min(Cond.nRep, (rank + 1) * per)))
+        for i in range(0, len(runs), int(batch)):
+            group = runs[i:i + int(batch)]
+            MCMCs = [setup(run) for run in group]
+            api.sampleBatch(MCMCs, seed=seed + group[0], device=device, **sample_kwargs)
+            dics = api.getDicBatch(MCMCs, dtype=dtype, device=device)
+            for run, MCMC, dic in zip(group, MCMCs, dics):
+                mine[run] = summary(MCMC, dic.DIC)
     if dist is not None and world > 1:
         gathered = [None] * world
         dist.all_gather_object(gathered, mine)

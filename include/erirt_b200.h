@@ -89,6 +89,25 @@ int erirt_version(void);
 const char* erirt_last_error(void);
 
 int erirt_create(const erirt_config* cfg, erirt_handle** out);
+/* Replica batch (DESIGN.md 6.6): one handle holding n_batch (1..65535, else ERIRT_E_ARG) independent problems of the SAME
+ * configuration -- model, dimensions, dtype, n_iter, n_chain, n_burnin, q_rt and keyword options -- each with its own data, initial
+ * state, parameters, statistics, running moments and traces.  erirt_sample advances all of them with one person launch and one global
+ * launch per sweep.  Replica r is the chain of a standalone handle created from *cfg with seed = cfg->seed + r (Philox key
+ * make_key(cfg->seed + r, cfg->chain)) and given replica r's data and initial state: same draws, traces, state and moments, up to the
+ * summation order of the f64 statistics atomics.  erirt_create(cfg, out) is erirt_create_batch(cfg, 1, out).
+ * The other entry points keep their signatures and stack the replicas:
+ *   person-indexed arrays (Y, logT, X, theta, zeta, nu, omega, moments) have n_batch * n_subj rows, replica r in rows
+ *   [r n_subj, (r+1) n_subj) (leading dimensions >= n_batch * n_subj); every other array (a, b, lambda, sigma2, rho, beta, Sigma_p,
+ *   the item vectors of erirt_generate_data) is n_batch consecutive blocks of its standalone length;
+ *   erirt_generate_data uses data seed `seed + r` for replica r; the ingest constants are computed per replica;
+ *   erirt_get_trace: out[m + n_iter*(c + n_cols*(l + n_chain*r))], Julia's [nIter, P, nChain, nBatch];
+ *   erirt_trace_width: the width of one replica;  erirt_trace_ess_rhat: n_batch * n_cols results, replica-major;
+ *   erirt_loglik_current: n_batch values;  erirt_get_stats: totals over the batch;
+ *   erirt_sample: ERIRT_E_NUMERIC when any replica met a non-positive-definite covariance (the message names the first; each
+ *   replica's status is sticky).
+ * With n_batch > 1, ERIRT_E_UNSUPPORTED (before any CUDA call) for RtIrtCross / RtIrtCrossQr and person_trace = 1 at create, and
+ * from erirt_checkpoint_*, erirt_comm_init and erirt_peer_*. */
+int erirt_create_batch(const erirt_config* cfg, int32_t n_batch, erirt_handle** out);
 int erirt_destroy(erirt_handle* h);
 /* The full-size device buffers of a handle and the ingest staging come from the device's stream-ordered memory pool, which keeps up to
  * ERIRT_POOL_KEEP_MB (environment, default 4096) of freed memory for the next handle of the process.  erirt_trim_pool returns all of
@@ -171,7 +190,8 @@ int erirt_loglik_current(erirt_handle* h, double* out);
 int erirt_get_stats(erirt_handle* h, erirt_stats* out);
 /* Debugging aid (compute-sanitizer is not available everywhere): a handle created with ERIRT_GUARDS=1 in the environment places a
  * 256-byte guard zone after every device buffer; this returns how many guard bytes have been overwritten since (0 = clean), or -1
- * when the handle has no guard zones.  No counterpart in the reference. */
+ * when the handle has no guard zones.  A buffer of a replica batch holds the copies of all replicas, so its guard zone catches
+ * writes past the last replica, not writes between two replicas.  No counterpart in the reference. */
 int64_t erirt_debug_check_guards(erirt_handle* h);
 
 /* ---- checkpoint / resume (SURVEY 8f-4): state, auxiliaries, Philox sweep counter, running moments and traces of the chain ----

@@ -12,7 +12,7 @@ using ExtendedRtIrtModeling
 import ExtendedRtIrtModeling: sample!, InputPara, GibbsMlIrt, GibbsRtIrt, GibbsRtIrtNull, GibbsRtIrtCross, GibbsRtIrtCrossQr,
                                GibbsRtIrtLatent, GibbsRtIrtLatentQr
 
-export GibbsRtIrtQuantile, lean, LeanGibbs, LeanPost, Shard, sample_sharded!, ess_rhat_gpu, checkConvergence_gpu
+export GibbsRtIrtQuantile, lean, LeanGibbs, LeanPost, Shard, sample_sharded!, sample_batch!, ess_rhat_gpu, checkConvergence_gpu
 
 const LIB = get(ENV, "ERIRT_B200_LIB", joinpath(@__DIR__, "..", "extendedrtirtmodeling.jl_b200", "liberirt_b200.so"))
 
@@ -299,6 +299,81 @@ shard.offset + MCMC.Cond.nSubj` of Y, logT, X (its `Data`) and their initial θ,
 with the SAME `seed`.  Item / structural traces are identical on every rank; Post.mean.θ / ζ / ν are this rank's persons.
 """
 sample_sharded!(MCMC::LeanGibbs, shard::Shard; kw...) = sample!(MCMC; shard=shard, kw...)
+
+# ---- replica batches (erirt_create_batch, DESIGN.md 6.6): B replications of one model, e.g. the nRep data sets of runSimulation
+#      (src/SimTools.jl:457-495), sampled by ONE handle with one person launch and one global launch per sweep ----
+function _trace4!(h, which, out::Array{Float64,4}, first_col)   # [nIter, ncols, nChain, B]
+    GC.@preserve out check(ccall((:erirt_get_trace, LIB), Cint, (Ptr{Cvoid}, Int32, Int64, Int64, Ptr{Float64}),
+                                 h, which, first_col, size(out, 2), out))
+end
+
+"""
+    sample_batch!(MCMCs::AbstractVector; intercept=false, itemtype="2pl", cov2one, dtype=1, seed=rand(UInt64), device=0)
+
+`sample!(MCMCs[r]; seed=seed + r - 1, person_trace=false)` for every r, as one replica batch on one GPU.  The model objects are of one
+of the five one-launch types (GibbsMlIrt, GibbsRtIrt, GibbsRtIrtNull, GibbsRtIrtLatent, GibbsRtIrtLatentQr) with equal Cond; each has
+its own Data and initial Para.  Replica r's chain is the one its own `sample!` with that seed would draw (same Philox stream), so
+Post (item / structural traces, logLike) and Post.mean (θ, ζ, ν from the running moments) are filled as that call fills them.
+"""
+function sample_batch!(MCMCs::AbstractVector; intercept=false, itemtype::Union{String}="2pl", cov2one=nothing, dtype=1,
+                       seed=rand(UInt64), device=0)
+    T, B = typeof(MCMCs[1]), length(MCMCs)
+    Cond = MCMCs[1].Cond
+    all(M -> typeof(M) === T && M.Cond == Cond, MCMCs) || error("sample_batch!: the model objects must share one type and one Cond")
+    (T === GibbsRtIrtCross || T === GibbsRtIrtCrossQr) && error("sample_batch!: the Cross family is not batched")
+    itemtype in ["1pl", "2pl"] || error("Invalid input: the item type must be '1pl' or '2pl'.")
+    cov2one === nothing && (cov2one = !(T === GibbsRtIrtLatent || T === GibbsRtIrtLatentQr))
+    N, J, F, nb = Cond.nSubj, Cond.nItem, Cond.nFeat, Cond.nBurnin
+    has_rt, lqr = !(T === GibbsMlIrt), T === GibbsRtIrtLatentQr
+    cfg = ErirtConfig(1, MODEL_ID[T], N, N, 0, J, F, Cond.nIter, Cond.nChain, nb, Cond.qRt, intercept, itemtype == "1pl", cov2one,
+                      dtype, seed, 0, 0, 0, device, 1, 0, 0, ntuple(_ -> Int32(0), 6))
+    href = Ref{Ptr{Cvoid}}(C_NULL)
+    check(ccall((:erirt_create_batch, LIB), Cint, (Ref{ErirtConfig}, Int32, Ref{Ptr{Cvoid}}), cfg, Int32(B), href))
+    h = href[]
+    try
+        # person-indexed matrices stack the replicas along the rows; every other field is B consecutive blocks
+        Y = reduce(vcat, [Matrix{Float64}(M.Data.Y) for M in MCMCs])
+        logT = has_rt ? reduce(vcat, [Matrix{Float64}(M.Data.logT) for M in MCMCs]) : zeros(0, 0)
+        X = F > 0 ? reduce(vcat, [Matrix{Float64}(M.Data.X) for M in MCMCs]) : zeros(0, 0)
+        GC.@preserve Y logT X check(ccall((:erirt_set_data, LIB), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Int64),
+            h, Y, B * N, has_rt ? pointer(logT) : C_NULL, B * N, F > 0 ? pointer(X) : C_NULL, B * N))
+        stacked(f) = reduce(vcat, [vec(Matrix{Float64}(reshape(f(M.Para), :, 1))) for M in MCMCs])
+        _set_state(h, F_THETA, stacked(p -> p.θ)); _set_state(h, F_A, stacked(p -> p.a)); _set_state(h, F_B, stacked(p -> p.b))
+        if has_rt
+            _set_state(h, F_ZETA, stacked(p -> p.ζ)); _set_state(h, F_LAMBDA, stacked(p -> p.λ)); _set_state(h, F_SIGMA2, stacked(p -> p.σ²t))
+            _set_state(h, F_SIGMA_P, stacked(p -> p.Σp))
+        end
+        _set_state(h, F_BETA, stacked(p -> p.β))
+        check(ccall((:erirt_sample, LIB), Cint, (Ptr{Cvoid}, Int64), h, Cond.nIter * Cond.nChain))
+        qw = Int(ccall((:erirt_trace_width, LIB), Int64, (Ptr{Cvoid}, Int32), h, T_QR)) - (lqr ? N : 0)
+        shape(w) = Array{Float64}(undef, Cond.nIter, w, Cond.nChain, B)
+        ra, rt, qr, ll = shape(2J), shape(has_rt ? 2J : 0), shape(qw), shape(1)
+        _trace4!(h, T_RA, ra, N); has_rt && _trace4!(h, T_RT, rt, N); _trace4!(h, T_QR, qr, 0); _trace4!(h, T_LL, ll, 0)
+        θ, θsd = _moments(h, F_THETA, B * N)
+        ζ, ζsd = has_rt ? _moments(h, F_ZETA, B * N) : (nothing, nothing)
+        ν, νsd = lqr ? _moments(h, F_NU, B * N) : (nothing, nothing)
+        for (r, M) in enumerate(MCMCs)
+            P, rows = M.Post, ((r - 1) * N + 1):(r * N)
+            c0 = size(P.ra, 2) - 2J
+            P.ra[:, (c0 + 1):(c0 + 2J), :] .= ra[:, :, :, r]
+            has_rt && (P.rt[:, (c0 + 1):(c0 + 2J), :] .= rt[:, :, :, r])
+            P.qr[:, 1:qw, :] .= qr[:, :, :, r]
+            P.logLike .= ll[:, :, :, r]
+            sel(v) = v === nothing ? nothing : v[rows]
+            res = (person=(θ=sel(θ), θsd=sel(θsd), ζ=sel(ζ), ζsd=sel(ζsd), ν=sel(ν), νsd=sel(νsd)), νcell=Float64[])
+            if T === GibbsMlIrt
+                P.mean = InputPara(θ=res.person.θ, a=_pm(P.ra, (c0 + 1):(c0 + J), nb), b=_pm(P.ra, (c0 + J + 1):(c0 + 2J), nb),
+                                   β=_pm(P.qr, 1:(F + 1), nb))
+            else
+                _rt_mean!(M, (T === GibbsRtIrt || T === GibbsRtIrtNull) ? 2 * (F + 1) : F + 2, res; with_ν=lqr)
+            end
+        end
+    finally
+        ccall((:erirt_destroy, LIB), Cint, (Ptr{Cvoid},), h)
+    end
+    return MCMCs
+end
 
 # ---- simulated data generated on the device (erirt_generate_data): the N x J part of setData* (src/SimTools.jl:117-368) never exists on
 #      the host.  `truePara` holds the person-level draws θ (and ζ) made by the caller as in setData*, X the covariates (or nothing);
